@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # product arm (CUDA kernels, C ABI)
     python bench.py --impl reference --steps K --warmup W    # reference arm: CPU oracle port, all host threads
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one pass of the hot path over one batch: kz_step over 65,536 device-resident games per GPU
 (apply the action, generate the successor's legal moves, termination, auto-reset, write the 13,527-byte
@@ -417,6 +418,9 @@ def run_product(args):
     kernel_ms = sum(a.elapsed_time(b) for a, b in kev) / args.steps
     ply1 = float(env.export()[2][:, 1].float().mean())
     errs = int((env.errors() != 0).sum())
+    if args.dump_outputs and rank == 0:
+        last = it[0] - 1  # the last timed step wrote these slots and the next actions it chose
+        dump_step_outputs(args.dump_outputs, env, obs_buf[last % SLOTS], mask_buf[last % SLOTS][:, :13527], act[it[0] & 1])
 
     # ---- end-to-end through the public API with HOST buffers: per step the actions come from pinned host
     # memory (H2D) and the step's results + the next legal actions are read back to pinned host memory (D2H).
@@ -582,6 +586,37 @@ def run_product(args):
         emit(line)
     finish_process_group(world)
     return 0
+
+
+DUMP_OBS_ROWS = 512  # games whose observation + legal-mask rows --dump-outputs writes: 512 x 69 KB = 35 MB as float32
+DUMP_GAME_ROWS = 1 << 19  # games whose per-game results it writes: at most 7 x 2 MB
+
+
+def _dump_rows(n: int, k: int):
+    """All n games, or a fixed seeded sample of k of them in ascending order."""
+    import numpy as np
+    return np.arange(n) if n <= k else np.sort(np.random.default_rng(SEED).choice(n, k, replace=False))
+
+
+def dump_step_outputs(out_dir: str, env, obs, mask, next_actions):
+    """--dump-outputs: what one VecShogiEnv.step returned to its caller, as float32 .npy files under out_dir (every
+    value is a small integer or an fp32 number, so float32 holds it exactly).  obs / legal_mask hold the rows of
+    obs_rows (a seeded sample when there are more than DUMP_OBS_ROWS games); the per-game results those of game_rows."""
+    import numpy as np
+    import torch
+    n = env.n
+    obs_rows, game_rows = _dump_rows(n, DUMP_OBS_ROWS), _dump_rows(n, DUMP_GAME_ROWS)
+    oi, gi = torch.from_numpy(obs_rows).to(obs.device), torch.from_numpy(game_rows).to(obs.device)
+    arrays = {"obs": obs.index_select(0, oi), "legal_mask": mask.index_select(0, oi),
+              "next_action": next_actions[:n], "reward": env.reward, "done": env.done, "reason": env.reason,
+              "winner": env.winner, "ep_len": env.ep_len, "legal_count": env.legal_count}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if name not in ("obs", "legal_mask"):
+            t = t.index_select(0, gi)
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "obs_rows.npy"), obs_rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "game_rows.npy"), game_rows.astype(np.float64))
 
 
 def cfg5_positions(n: int):
@@ -951,7 +986,12 @@ def main():
     ap.add_argument("--no-graph-rollout", action="store_true", help="run the rollout loop eagerly (one warm-up epoch suffices then)")
     ap.add_argument("--ppo-steps", type=int, default=2, help="timed PPO epochs of the `ppo` record")
     ap.add_argument("--ppo-warmup", type=int, default=2, help="untimed PPO epochs (the first captures the update graph, the second the rollout graph)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (observations, legal masks, rewards, done "
+                         "flags, next actions, ...) as float32 DIR/<name>.npy, at most 64 MB (default env workload only)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "product" or args.workload != "env"):
+        ap.error("--dump-outputs applies to the default workload (--impl product --workload env)")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference_ppo(args) if args.workload == "ppo" else run_reference(args)

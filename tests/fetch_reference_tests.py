@@ -1,8 +1,8 @@
 """Copy the reference's own hot-path test files into baseline/_ref_tests/ (git-ignored, like baseline/_ref) so that they
 travel to the GPU box with the tree, where tests/test_gpu_reference_suite.py runs them unmodified against this repository's
-classes through the keisei -> shogidrl_b200 alias package (tests/ref_alias).  Run in a container that has the checkout:
+classes through the keisei -> shogidrl_b200 alias package (tests/ref_alias).  Run where a checkout of the reference is at hand:
 
-    python tests/fetch_reference_tests.py [/root/reference]
+    python tests/fetch_reference_tests.py [reference checkout, default $SHOGIDRL_REFERENCE]
 
 The mock-driven tests of the two training-side callers of the path (tests/training/test_step_manager.py and
 test_env_manager.py, with the reference's conftest.py for their fixtures) and two CPU-only files of tests/shogi
@@ -26,7 +26,9 @@ HOST_FILES = [("", "conftest.py"), ("training", "test_step_manager.py"), ("train
 
 
 def main() -> int:
-    ref = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
+    ref = sys.argv[1] if len(sys.argv) > 1 else os.environ.get("SHOGIDRL_REFERENCE")
+    if not ref:
+        sys.exit("usage: python tests/fetch_reference_tests.py <reference checkout> (or set SHOGIDRL_REFERENCE)")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     dst = os.path.join(root, "baseline", "_ref_tests")
     os.makedirs(dst, exist_ok=True)

@@ -1,7 +1,7 @@
-"""Live differential checks against the Python reference, for the container that has it (skipped where
-/root/reference is absent, e.g. on the GPU box -- there the committed golden fixtures stand in).  Fresh seeds every
-round trip through the same comparisons as the golden tests: oracle vs reference self-play, the mapper's whole table,
-SFEN text, ExperienceBuffer host semantics."""
+"""Live differential checks against the Python reference (tachyon-beep/shogidrl), where a checkout of it is at hand:
+SHOGIDRL_REFERENCE names its root.  Skipped without it -- the committed golden fixtures, written by the reference,
+stand in.  Fresh seeds every round trip through the same comparisons as the golden tests: oracle vs reference
+self-play, the mapper's whole table, SFEN text, ExperienceBuffer host semantics."""
 import os
 import random
 import sys
@@ -10,8 +10,9 @@ import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "keisei")), reason="reference checkout not present")
+REF = os.environ.get("SHOGIDRL_REFERENCE", "")
+pytestmark = pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "keisei")),
+                                reason="reference checkout not present (set SHOGIDRL_REFERENCE)")
 
 
 @pytest.fixture(scope="module")
