@@ -203,6 +203,20 @@ int kz_sample_bitmap(const void* logits, int logits_bf16, int64_t ld, const uint
                      int n, uint64_t seed, uint64_t offset, const uint64_t* offset_dev, void* actions,
                      int actions_i64, float* logp, float* entropy, int deterministic, void* stream);
 
+/* The scripted opponent SimpleHeuristicOpponent.select_move (keisei/utils/opponents.py) for the CURRENT position of each
+ * of the n games: the legal moves are split into tiers -- 0 capture (destination holds a piece of the other colour),
+ * 1 non-promoting move of the mover's unpromoted pawn, 2 everything else, every drop included -- and the pick is the k-th
+ * member of the first non-empty tier in ascending action order, k = mulhi(rand32(seed, env_offset+env, rng_step), tier
+ * size): kz_refresh's next_actions convention.  The legal set is read from exactly one of
+ *   mask   [n][mask_stride] bytes (non-zero = legal; kz_step / kz_refresh rows), or
+ *   bitmap [n][bitmap_stride_words] uint32 (kz_step_rollout / kz_legal_bitmap rows; 4-byte aligned);
+ * both forms give identical results.  actions: int64 if actions_i64 else int32, -1 when there is no legal move.
+ * Optional: tier (u8: 0 capture, 1 pawn, 2 other, 255 none) and tier_count (int32: size of the chosen tier).
+ * Needs no tables. */
+int kz_heuristic_actions(const void* state, int n, int hist_cap, const uint8_t* mask, int64_t mask_stride,
+                         const uint32_t* bitmap, int64_t bitmap_stride_words, void* actions, int actions_i64, uint8_t* tier,
+                         int32_t* tier_count, uint64_t seed, uint32_t rng_step, uint32_t env_offset, void* stream);
+
 /* ExperienceBuffer.compute_advantages_and_returns (experience_buffer.py:99-145) over a [T][N]
  * layout, one reverse scan per env column (N = 1 is the reference's flat buffer):
  *   delta = (r + (gamma * nv) * m) - V ;  gae = delta + (gamma_lambda * m) * gae   (no FMA)

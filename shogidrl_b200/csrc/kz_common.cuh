@@ -73,6 +73,16 @@ __device__ __forceinline__ uint32_t spread16(uint32_t x) {  // bit i -> bit 2i
   return x;
 }
 
+// Counter-based per-game random stream: kz_step's next_actions and kz_heuristic_actions draw from it.  The formula is
+// part of the interface: a CPU restatement of it replays those draws bit for bit.
+__device__ __forceinline__ uint32_t rand32(unsigned long long seed, unsigned long long env, unsigned long long step) {
+  unsigned long long x = seed ^ (env * 0x9E3779B97F4A7C15ull) ^ (step * 0xBF58476D1CE4E5B9ull);
+  x ^= x >> 30; x *= 0xBF58476D1CE4E5B9ull;
+  x ^= x >> 27; x *= 0x94D049BB133111EBull;
+  x ^= x >> 31;
+  return (uint32_t)(x >> 32);
+}
+
 __device__ __forceinline__ int sq_row(int s) { return (s * 57) >> 9; }  // floor(s / 9) for s < 96
 __device__ __forceinline__ int sq_col(int s) { return s - 9 * sq_row(s); }
 

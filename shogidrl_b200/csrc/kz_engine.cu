@@ -595,14 +595,6 @@ struct StepParams {
   uint32_t* cobs_out;  // optional compact observation [n][KZ_COBS_WORDS] (kz_step_rollout / kz_legal_bitmap)
 };
 
-__device__ __forceinline__ uint32_t rand32(unsigned long long seed, unsigned long long env, unsigned long long step) {
-  unsigned long long x = seed ^ (env * 0x9E3779B97F4A7C15ull) ^ (step * 0xBF58476D1CE4E5B9ull);
-  x ^= x >> 30; x *= 0xBF58476D1CE4E5B9ull;
-  x ^= x >> 27; x *= 0x94D049BB133111EBull;
-  x ^= x >> 31;
-  return (uint32_t)(x >> 32);
-}
-
 __device__ __forceinline__ uint16_t ld_u16(const uint8_t* p) { return (uint16_t)(p[0] | (p[1] << 8)); }
 __device__ __forceinline__ void st_u16(uint8_t* p, int v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); }
 

@@ -2,14 +2,14 @@
 //   kz_sample_masked : masked softmax -> Categorical sample / argmax -> log_prob (+ entropy)
 //                      (keisei/core/base_actor_critic.py:64-116; torch.distributions.Categorical(probs=...))
 //   kz_gae           : reverse-time GAE over a [T][N] rollout (keisei/core/experience_buffer.py:99-145)
+//   kz_heuristic_actions : the scripted SimpleHeuristicOpponent's move for every game (keisei/utils/opponents.py)
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <float.h>
 #include <stdint.h>
 #include <stdio.h>
 #include "../../include/keisei_b200.h"
-
-#define FULL 0xffffffffu
+#include "kz_common.cuh"
 
 int kz_cuda_fail(cudaError_t e);  // kz_engine.cu: records the message for kz_last_cuda_error
 
@@ -257,6 +257,120 @@ __global__ void __launch_bounds__(256, 4) kz_sample_kernel(const void* logits, i
     else reinterpret_cast<int*>(actions)[row] = (int)act;
     if (logp) logp[row] = lp;
     if (entropy) entropy[row] = ent;
+  }
+}
+
+// ---- SimpleHeuristicOpponent.select_move (keisei/utils/opponents.py) for n games, one warp per game ----
+// The legal moves fall into three tiers: 0 capture (the destination holds a piece of the other colour; legal moves never
+// land on own pieces, so "occupied" suffices), 1 non-promoting move of the mover's unpromoted pawn, 2 everything else,
+// every drop included.  The pick is uniform over the first non-empty tier: its k-th member in ascending action order,
+// k = mulhi(rand32(seed, env, step), tier size) -- kz_step's next_actions convention, so a CPU replay can follow it.
+// A board move's index is from*160 + 2*to' + promote, so the 16 actions [16A, 16A + 16) of window A < 810 share the
+// source square A / 10 and cover the destinations to' = 8*(A % 10) .. +7 (to = to' + (to' >= from)); windows 810.. are
+// drops.  A window's tiers are then its legality bits ANDed with 8 bits of the enemy-occupancy bitboard (spread to bit
+// pairs) and, when the source holds an own pawn, with the non-promoting (even) bits.
+#define HEUR_WINDOWS ((KZ_NUM_ACTIONS + 15) / 16)  // 846
+#define HEUR_ROUNDS ((HEUR_WINDOWS + 31) / 32)      // 27: window A = 32 * round + lane
+
+// legality bits of actions [16A, 16A + 16); MaskWindows' windows follow the row's own 16-byte phase, so two are merged
+__device__ __forceinline__ uint32_t legal16(const MaskWindows& W, int A) {
+  const uint32_t lo = MaskWindows::bits16(W.load(A));
+  if (!W.shift) return lo;
+  return ((lo >> W.shift) | (MaskWindows::bits16(W.load(A + 1)) << (16 - W.shift))) & 0xFFFFu;
+}
+__device__ __forceinline__ uint32_t legal16(const BitmapWindows& W, int A) { return W.load(A); }
+
+// capture (t0) and pawn (t1) bits of window A's legality bits v; the rest of v is tier 2
+__device__ __forceinline__ void heur_classify(uint32_t v, int A, const BB& enemy, const BB& pawns, uint32_t& t0, uint32_t& t1) {
+  t0 = t1 = 0u;
+  if (A >= 810 || !v) return;
+  const int from = A / 10, lo = 8 * (A - 10 * from);
+  const int wd = lo >> 5;
+  const uint32_t a = wd == 0 ? enemy.w0 : (wd == 1 ? enemy.w1 : enemy.w2);
+  const uint32_t b = wd == 0 ? enemy.w1 : (wd == 1 ? enemy.w2 : 0u);
+  const uint32_t x = __funnelshift_r(a, b, lo & 31) & 0x1FFu;  // enemy bits of squares lo .. lo + 8
+  const uint32_t below = lowmask32(from - lo) & 0xFFu;         // to' < from: to = to'; above: to = to' + 1
+  const uint32_t e8 = ((x & below) | ((x >> 1) & ~below)) & 0xFFu;
+  t0 = v & (spread16(e8) * 3u);
+  if (bb_test(pawns, from)) t1 = v & ~t0 & 0x5555u;
+}
+
+template <class WIN>  // MaskWindows: byte mask rows; BitmapWindows: 448-word legal bitmap rows.  ldm in bytes.
+__global__ void __launch_bounds__(256) kz_heuristic_kernel(const uint8_t* __restrict__ boards, const uint8_t* __restrict__ meta,
+                                                           int n, const void* legal, long long ldm, void* actions,
+                                                           int actions_i64, uint8_t* tier_out, int32_t* count_out,
+                                                           unsigned long long seed, uint32_t rng_step, uint32_t env_offset) {
+  __shared__ uint16_t s_bits[8][HEUR_ROUNDS * 32];  // the row's legality bits, window by window, for the selection pass
+  const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
+  const int g = blockIdx.x * 8 + wi;
+  if (g >= n) return;
+  const uint8_t* b = boards + (size_t)g * 96;
+  const int side = meta[(size_t)g * 32 + 14];
+  uint32_t e[3], p[3];
+#pragma unroll
+  for (int j = 0; j < 3; j++) {
+    const int s = lane + 32 * j;
+    const int c = s < 81 ? b[s] : 0;
+    e[j] = __ballot_sync(FULL, c != 0 && code_color(c) != side);
+    p[j] = __ballot_sync(FULL, c == 1 + 14 * side);
+  }
+  const BB enemy{e[0], e[1], e[2]}, pawns{p[0], p[1], p[2]};
+  const WIN W(reinterpret_cast<const char*>(legal) + (size_t)g * ldm);
+  uint16_t* bits = s_bits[wi];
+
+  // pass 1: tier sizes (each lane writes and later reads only its own windows: no warp barrier needed)
+  int c0 = 0, c1 = 0, c2 = 0;
+#pragma unroll 9
+  for (int r = 0; r < HEUR_ROUNDS; r++) {
+    const int A = 32 * r + lane;
+    uint32_t v = A < HEUR_WINDOWS ? legal16(W, A) : 0u;
+    if (A == HEUR_WINDOWS - 1) v &= (1u << (KZ_NUM_ACTIONS - 16 * (HEUR_WINDOWS - 1))) - 1u;  // bitmap pad bits
+    uint32_t t0, t1;
+    heur_classify(v, A, enemy, pawns, t0, t1);
+    c0 += __popc(t0); c1 += __popc(t1); c2 += __popc(v & ~(t0 | t1));
+    bits[A] = (uint16_t)v;
+  }
+  const int n0 = (int)__reduce_add_sync(FULL, (unsigned)c0), n1 = (int)__reduce_add_sync(FULL, (unsigned)c1),
+            n2 = (int)__reduce_add_sync(FULL, (unsigned)c2);
+  const int tier = n0 ? 0 : (n1 ? 1 : (n2 ? 2 : 255));
+  const int cnt = n0 ? n0 : (n1 ? n1 : n2);
+
+  // pass 2: the k-th member of the tier, rounds in ascending action order (lane order inside a round)
+  long long pick = -1;
+  if (cnt > 0) {
+    const int k = (int)(((unsigned long long)rand32(seed, (unsigned long long)env_offset + (unsigned long long)g, rng_step) *
+                         (unsigned long long)cnt) >> 32);
+    int base = 0;
+    for (int r = 0; r < HEUR_ROUNDS; r++) {
+      const int A = 32 * r + lane;
+      const uint32_t v = bits[A];
+      uint32_t t0, t1;
+      heur_classify(v, A, enemy, pawns, t0, t1);
+      uint32_t m = tier == 0 ? t0 : (tier == 1 ? t1 : (v & ~(t0 | t1)));
+      const int c = __popc(m);
+      const int tot = (int)__reduce_add_sync(FULL, (unsigned)c);
+      if (k < base + tot) {  // warp-uniform
+        int incl = c;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += t; }
+        int rem = k - base - (incl - c);
+        int found = -1;
+        if (rem >= 0 && rem < c) {
+          while (rem--) m &= m - 1;
+          found = 16 * A + __ffs(m) - 1;
+        }
+        const uint32_t own = __ballot_sync(FULL, found >= 0);
+        pick = __shfl_sync(FULL, found, __ffs(own) - 1);
+        break;
+      }
+      base += tot;
+    }
+  }
+  if (lane == 0) {
+    if (actions_i64) reinterpret_cast<long long*>(actions)[g] = pick;
+    else reinterpret_cast<int*>(actions)[g] = (int)pick;
+    if (tier_out) tier_out[g] = (uint8_t)tier;
+    if (count_out) count_out[g] = cnt;
   }
 }
 
@@ -540,6 +654,29 @@ int kz_sample_bitmap(const void* logits, int logits_bf16, int64_t ld, const uint
     return KZ_E_ARG;
   return sample_impl(logits, logits_bf16, ld, bitmap, ldb_words * 4, 1, n, seed, offset, offset_dev, actions, actions_i64, logp,
                      entropy, deterministic, stream);
+}
+
+int kz_heuristic_actions(const void* state, int n, int hist_cap, const uint8_t* mask, int64_t mask_stride,
+                         const uint32_t* bitmap, int64_t bitmap_stride_words, void* actions, int actions_i64, uint8_t* tier,
+                         int32_t* tier_count, uint64_t seed, uint32_t rng_step, uint32_t env_offset, void* stream) {
+  int64_t offs[3], total = 0;
+  if (!state || !actions || (mask == nullptr) == (bitmap == nullptr) || kz_state_layout(n, hist_cap, offs, &total) != KZ_OK)
+    return KZ_E_ARG;
+  if (mask && mask_stride < KZ_NUM_ACTIONS) return KZ_E_ARG;
+  if (bitmap && (bitmap_stride_words < KZ_BITMAP_WORDS_MIN || ((uintptr_t)bitmap & 3))) return KZ_E_ARG;
+  if (((uintptr_t)actions & (actions_i64 ? 7 : 3)) || ((uintptr_t)tier_count & 3)) return KZ_E_ARG;
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
+  if (bitmap)
+    kz_heuristic_kernel<BitmapWindows><<<(n + 7) / 8, 256, 0, st>>>(base + offs[0], base + offs[1], n, bitmap,
+                                                                     bitmap_stride_words * 4, actions, actions_i64, tier,
+                                                                     tier_count, seed, rng_step, env_offset);
+  else
+    kz_heuristic_kernel<MaskWindows><<<(n + 7) / 8, 256, 0, st>>>(base + offs[0], base + offs[1], n, mask, mask_stride,
+                                                                   actions, actions_i64, tier, tier_count, seed, rng_step,
+                                                                   env_offset);
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? KZ_OK : fail(e);
 }
 
 int kz_gae(const float* rewards, const float* values, const uint8_t* dones, const float* last_value, int T, int N,

@@ -2,9 +2,11 @@
 
 The reference's evaluation strategies each run a scalar ``get_legal_moves -> get_legal_mask -> select_action ->
 make_move`` loop per game (keisei/evaluation/strategies/single_opponent.py:162-221).  Here N games are played at
-once on a VecShogiEnv: the agent moves for one colour, the opponent (uniform-random legal, the engine's fused
-policy, or a second agent) for the other; games that finish are reset and keep counting until ``num_games`` have
-been completed."""
+once on a VecShogiEnv: one player moves for one colour, the other for the other; games that finish are reset and keep
+counting until ``num_games`` have been completed.  A player is an agent-like object (``select_actions(obs, mask)``) or
+one of the reference's scripted opponents (keisei/utils/opponents.py), played on the device: ``"random"`` /
+``SimpleRandomOpponent`` (the engine's fused uniform-random legal action) or ``"heuristic"`` /
+``SimpleHeuristicOpponent`` (``VecShogiEnv.heuristic_actions``, one launch per step)."""
 from __future__ import annotations
 
 import json
@@ -14,6 +16,7 @@ from typing import Any, Dict, List, Mapping, Optional, Tuple
 
 import torch
 
+from .utils.opponents import BaseOpponent, SimpleHeuristicOpponent, SimpleRandomOpponent
 from .vec_env import VecShogiEnv
 
 OUTCOMES = ("draw", "agent_win", "opponent_win")  # the reference's result strings (elo_registry.py:86)
@@ -33,16 +36,31 @@ class EvaluationResult:
         return self.agent_wins / max(1, self.games)
 
 
+def _player_kind(player) -> str:
+    """"random", "heuristic" or "agent" for a player of evaluate_vs_opponent (None = the uniform-random player)."""
+    if player is None or isinstance(player, SimpleRandomOpponent) or (isinstance(player, str) and player == "random"):
+        return "random"
+    if isinstance(player, SimpleHeuristicOpponent) or (isinstance(player, str) and player == "heuristic"):
+        return "heuristic"
+    if isinstance(player, (str, BaseOpponent)):
+        raise ValueError(f"unknown scripted player {player!r}: expected 'random', 'heuristic', SimpleRandomOpponent, "
+                         "SimpleHeuristicOpponent or an agent with select_actions(obs, mask)")
+    return "agent"
+
+
 def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int = 1024, max_moves_per_game: int = 500,
                          device="cuda", seed: int = 0, deterministic: bool = True,
                          max_steps: Optional[int] = None) -> EvaluationResult:
-    """Play ``num_games`` games of ``agent`` against ``opponent`` (None = uniform-random legal moves).  The agent
-    plays Black in even-numbered envs and White in odd-numbered ones.  Every env has a fixed QUOTA of games
-    (``num_games`` spread evenly over the envs): the first ``quota`` games an env finishes are counted and later ones
+    """Play ``num_games`` games of ``agent`` against ``opponent`` (None = uniform-random legal moves).  Either side may
+    be an agent-like object, ``"random"``, ``"heuristic"`` or an instance of the two scripted opponent classes; results
+    are counted from ``agent``'s side.  The agent plays Black in even-numbered envs and White in odd-numbered ones.
+    Every env has a fixed QUOTA of games (``num_games`` spread evenly over the envs): the first ``quota`` games an env finishes are counted and later ones
     are ignored, so the sample is ``num_games`` independent games exactly as the reference's sequential loop plays them
     -- counting "the first num_games completions of the batch" would over-sample short (decisive) games, because a
     fast env restarts and finishes again while the long draws are still running.  Every tensor stays on the device;
     the host reads four counters per step."""
+    kinds = (_player_kind(agent), _player_kind(opponent))
+    random_actions = "random" in kinds
     n = min(num_envs, max(2, num_games))
     env = VecShogiEnv(n, max_moves_per_game=max_moves_per_game, device=device, seed=seed, auto_reset=True)
     dev = env.device
@@ -51,6 +69,15 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
     quota[: num_games % n] += 1
     completed = torch.zeros(n, dtype=torch.int64, device=dev)
     env.refresh(random_actions=True)
+    heuristic = env.heuristic_actions() if "heuristic" in kinds else None
+
+    def actions_of(player, kind):
+        if kind == "random":
+            return env.next_actions
+        if kind == "heuristic":
+            return heuristic
+        return player.select_actions(env.obs, env.mask, is_training=not deterministic)[0]
+
     # side to move per env: read from plane 42 of the observation (1.0 = Black to move)
     done_games = agent_w = opp_w = draws = 0
     length_sum = 0
@@ -60,13 +87,12 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
     while done_games < num_games and steps < limit:
         black_to_move = env.obs[:, 42, 0, 0] > 0.5
         agent_turn = black_to_move == agent_is_black
-        a_agent, _, _ = agent.select_actions(env.obs, env.mask, is_training=not deterministic)
-        if opponent is None:
-            a_opp = env.next_actions
-        else:
-            a_opp, _, _ = opponent.select_actions(env.obs, env.mask, is_training=not deterministic)
+        a_agent = actions_of(agent, kinds[0])
+        a_opp = actions_of(opponent, kinds[1])
         actions = torch.where(agent_turn, a_agent, a_opp).contiguous()
-        out = env.step(actions, random_actions=opponent is None)
+        out = env.step(actions, random_actions=random_actions)
+        if heuristic is not None:
+            env.heuristic_actions(out=heuristic)  # for the returned state (auto-reset applied)
         steps += 1
         d = (out["done"] != 0) & (completed < quota)  # finished games that still count towards their env's quota
         completed += d
@@ -191,8 +217,9 @@ def tournament_standings(results: Mapping[str, EvaluationResult]) -> Dict[str, A
 
 def evaluate_tournament(agent, opponents: Mapping[str, Any], num_games_per_opponent: int,
                         **kwargs) -> Tuple[Dict[str, Any], Dict[str, EvaluationResult]]:
-    """Round of matches against every opponent of the pool (name -> agent-like object, or None for the uniform-random
-    player), colours balanced inside each match; returns (standings, per-opponent results)."""
+    """Round of matches against every opponent of the pool (name -> a player of evaluate_vs_opponent: an agent-like
+    object, "random" / None, "heuristic" or a scripted opponent instance), colours balanced inside each match; returns
+    (standings, per-opponent results)."""
     results = {name: evaluate_vs_opponent(agent, num_games_per_opponent, opponent=opp, **kwargs)
                for name, opp in opponents.items()}
     return tournament_standings(results), results
@@ -215,8 +242,9 @@ def benchmark_performance(results: Mapping[str, EvaluationResult]) -> Dict[str, 
 def evaluate_benchmark(agent, suite: Mapping[str, Any], num_games_per_case: int,
                        **kwargs) -> Tuple[Dict[str, Any], Dict[str, EvaluationResult]]:
     """The benchmark strategy (benchmark.py:330-426, 556-637) on the vectorised engine: ``num_games_per_case`` games against
-    every case of the suite (name -> opponent agent, or None for the uniform-random baseline the reference's default suite
-    starts with), colours balanced; returns (the reference's performance dictionary, per-case results)."""
+    every case of the suite (name -> a player of evaluate_vs_opponent; the reference's default suite is
+    {"benchmark_random": None, "benchmark_heuristic": "heuristic"}), colours balanced; returns (the reference's performance
+    dictionary, per-case results)."""
     results = {name: evaluate_vs_opponent(agent, num_games_per_case, opponent=opp, **kwargs) for name, opp in suite.items()}
     return benchmark_performance(results), results
 
@@ -234,7 +262,8 @@ def evaluate_ladder(agent, agent_id: str, pool: Mapping[str, Any], tracker: Opti
                     num_games_per_match: int = 2, num_opponents_to_select: int = 5,
                     **kwargs) -> Tuple[Dict[str, float], Dict[str, EvaluationResult]]:
     """One ladder pass (ladder.py:490-558): select opponents near the agent's rating, play a colour-balanced match
-    against each, update the ratings game by game; returns (rating snapshot, per-opponent results)."""
+    against each (pool: name -> a player of evaluate_vs_opponent), update the ratings game by game; returns (rating
+    snapshot, per-opponent results)."""
     tracker = tracker if tracker is not None else EloTracker()
     ratings = {name: tracker.get_agent_rating(name) for name in pool}
     chosen = select_ladder_opponents(tracker.get_agent_rating(agent_id), ratings, num_opponents_to_select)

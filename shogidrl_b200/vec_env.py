@@ -221,6 +221,40 @@ class VecShogiEnv:
                                          self.legal_count.data_ptr(), self._sp()), "kz_legal_bitmap")
         return obs, bitmap
 
+    # The heuristic opponent draws from the env's random stream keyed by seed ^ HEURISTIC_SALT, so its pick is independent
+    # of the fused uniform-random action (next_actions, keyed by the seed itself) drawn for the same step and env.
+    HEURISTIC_SALT = 0x48657572697374  # "Heurist"
+
+    def heuristic_actions(self, out: Optional[torch.Tensor] = None, mask: Optional[torch.Tensor] = None,
+                          bitmap: Optional[torch.Tensor] = None, tier: Optional[torch.Tensor] = None,
+                          tier_count: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The scripted SimpleHeuristicOpponent's move (keisei/utils/opponents.py) for every env's CURRENT position
+        (kz_heuristic_actions): a uniform pick among the captures if there are any, else among the non-promoting moves of
+        an unpromoted pawn, else among all other legal moves; -1 where there is no legal move.  The legal set is read from
+        ``mask`` (default ``self.mask``) or from ``bitmap`` rows (int32 [n, 448], as ``step_rollout`` writes them), not
+        both.  ``out`` int64 / int32 [n] (default: a new int64 tensor); ``tier`` (uint8 [n]: 0 capture, 1 pawn, 2 other,
+        255 none) and ``tier_count`` (int32 [n]: size of the chosen tier) are optional.  Draws with ``step_index``."""
+        if mask is not None and bitmap is not None:
+            raise ValueError("heuristic_actions: give the legal set as mask or as bitmap, not both")
+        mp, ms, bp, bs = None, 0, None, 0
+        if bitmap is not None:
+            bp, bs = self._bitmap_args(bitmap)
+        else:
+            mp, ms = self._mask_args(self.mask if mask is None else mask)
+        if out is None:
+            out = torch.empty(self.n, dtype=torch.int64, device=self.device)
+        for t, dts, what in ((out, (torch.int64, torch.int32), "out"), (tier, (torch.uint8,), "tier"),
+                             (tier_count, (torch.int32,), "tier_count")):
+            if t is not None and (t.device != self.device or t.dtype not in dts or not t.is_contiguous()
+                                  or t.numel() < self.n):
+                raise ValueError(f"{what}: expected a contiguous {dts[0]} [{self.n}] tensor on {self.device}, got "
+                                 f"{tuple(t.shape)} {t.dtype} on {t.device}")
+        nv.check(self._L.kz_heuristic_actions(self.state.data_ptr(), self.n, self.hist_cap, mp, ms, bp, bs, out.data_ptr(),
+                                              int(out.dtype == torch.int64), nv.ptr(tier), nv.ptr(tier_count),
+                                              (self.seed ^ self.HEURISTIC_SALT) & 0xFFFFFFFFFFFFFFFF, self.step_index,
+                                              self.env_offset, self._sp()), "kz_heuristic_actions")
+        return out
+
     def _cobs_arg(self, cobs: Optional[torch.Tensor]):
         if cobs is None:
             return None
