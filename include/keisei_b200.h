@@ -31,6 +31,8 @@ extern "C" {
 #define KZ_MASK_PAD_STRIDE 13536 /* 16-byte multiple >= 13527: fast-path row stride */
 #define KZ_BITMAP_WORDS 448     /* row of a legal BITMAP: bit i = action i legal; 423 words used, zero-padded to 14 per lane */
 #define KZ_BITMAP_WORDS_MIN 423 /* smallest row stride (in 32-bit words) the bitmap readers accept */
+#define KZ_POOL_RECORD_WORDS 512  /* one start-position record (kz_pool_records): 2 KB, layout below */
+#define KZ_POOL_BITMAP_OFFSET 64  /* word of a record where its 448-word legal bitmap begins */
 #define KZ_COBS_WORDS 40        /* compact observation: 84 bytes of plane indices + 18 fp32 constant-plane values + pad = 160 B */
 
 /* termination reason codes (shogi_core_definitions.py:135-147) */
@@ -135,6 +137,41 @@ int kz_step_range(void* state, int n, int hist_cap, int first, int count, int co
                   int64_t bitmap_stride_words, uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner,
                   int32_t* ep_len, int32_t* legal_count, void* next_actions, uint64_t seed, uint32_t rng_step,
                   uint32_t env_offset, int auto_reset, void* stream);
+
+/* ---- start-position pools: finished games restart from a table of precomputed positions instead of the start position.
+ * A RECORD (KZ_POOL_RECORD_WORDS uint32, 16-byte aligned) holds everything the auto-reset writes:
+ *   words 0..23   the 96-byte board row (81 piece codes; bytes 84..95 = words x, y, z of the 124-bit position key),
+ *   words 24..31  the 32-byte meta row: hands (bytes 0..13), side to move (14), move_count (18..19, u16), word w of the
+ *                 key (28..31); status 0, winner none, error bits / plies since reset / max_moves / episodes 0,
+ *   word 32       legal-move count, word 33 in-check flag (0 / 1), words 34..63 zero,
+ *   words 64..511 the legal bitmap (KZ_BITMAP_WORDS words, kz_legal_bitmap's row).
+ * kz_pool_records packs one record per game of a batch that kz_load_positions + kz_refresh (in_check) + kz_legal_bitmap
+ * have just prepared: state = that batch (n games, hist_cap), bitmap / legal_count / in_check = those calls' outputs.
+ * The positions must be non-terminal (kz_refresh(eval_termination=1) status 0, at least one legal move) and must not let
+ * the side to move capture the opponent's king; kz_pool_records does not check this. */
+int kz_pool_records(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words,
+                    const int32_t* legal_count, const uint8_t* in_check, uint32_t* records, void* stream);
+/* kz_step_range with auto-reset, where a game that finishes in this launch restarts from pool record k:
+ *   k = pick[g] when pick (int32 [n], indexed by the game's position in the batch) is given, otherwise
+ *   k = mulhi(rand32(pool_seed, env_offset + g, E), pool_size) with E the game's finished-episode counter after this
+ *       episode has been counted (export meta8[7]) -- so a replayed CUDA graph, whose rng_step values repeat, still draws
+ *       fresh starts; values of pick outside [0, pool_size) are taken modulo pool_size.
+ * The game keeps its own max_moves; move_count continues from the record's (so the ep_len a game reports counts the
+ * record's move_count too); the repetition table is emptied and the plies
+ * since reset set to 0.  start_ids (optional int32 [n]) receives k for every game that restarts.  Every output of the
+ * returned state (obs, mask or bitmap, cobs, legal_count, next_actions) comes from the record exactly as kz_step's
+ * outputs come from the start position. */
+int kz_step_pool(void* state, int n, int hist_cap, int first, int count, int counter_slot, const void* actions,
+                 int actions_i64, float* obs, int64_t obs_stride, uint8_t* mask, int64_t mask_stride, uint32_t* bitmap,
+                 int64_t bitmap_stride_words, uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner,
+                 int32_t* ep_len, int32_t* legal_count, void* next_actions, uint64_t seed, uint32_t rng_step,
+                 uint32_t env_offset, const uint32_t* pool, int pool_size, const int32_t* pick, uint64_t pool_seed,
+                 int32_t* start_ids, void* stream);
+/* kz_reset from the pool: the envs whose env_mask byte is non-zero (all if NULL) restart from record k, chosen as in
+ * kz_step_pool with E = the current finished-episode counter (not advanced); start_ids optional as there.  As after
+ * kz_reset, the rows of the new positions come from kz_refresh / kz_legal_bitmap. */
+int kz_reset_pool(void* state, int n, int hist_cap, const uint8_t* env_mask, int max_moves, const uint32_t* pool, int pool_size,
+                  const int32_t* pick, uint64_t pool_seed, uint32_t env_offset, int32_t* start_ids, void* stream);
 
 /* Split pipeline (experimental; same results as kz_step, bit for bit): kz_step_compact is kz_step without the two row
  * outputs -- it leaves the successor's 13,527-bit legal bitmap in bitmap [n][448] uint32 (bit i of the row = action i;

@@ -26,9 +26,10 @@ EXPORTS = [
     "kz_obs_conv_wgrad", "kz_ppo_loss", "kz_eval_masked_bwd_bias", "kz_adam_clip_workspace", "kz_adam_clip_step",
     "kz_step_compact", "kz_expand", "kz_step_rollout", "kz_legal_bitmap", "kz_bitmap_expand", "kz_sample_bitmap",
     "kz_eval_bitmap_fwd", "kz_eval_bitmap_bwd", "kz_step_range", "kz_cobs_conv_fwd", "kz_cobs_conv_wgrad_ctas",
-    "kz_cobs_conv_wgrad", "kz_heuristic_actions",
+    "kz_cobs_conv_wgrad", "kz_heuristic_actions", "kz_pool_records", "kz_step_pool", "kz_reset_pool",
 ]
 COBS_WORDS = 40
+POOL_RECORD_WORDS = 512
 ABI_VERSION = 2
 
 
@@ -75,6 +76,10 @@ def lib() -> C.CDLL:
     L.kz_eval_bitmap_fwd.argtypes = [vp, i32, i64, vp, i64, vp, vp, i32, vp, vp, vp, vp]
     L.kz_eval_bitmap_bwd.argtypes = [vp, i32, i64, vp, i64, vp, vp, i32, vp, vp, vp, vp, i64, vp, vp]
     L.kz_heuristic_actions.argtypes = [vp, i32, i32, vp, i64, vp, i64, vp, i32, vp, vp, u64, u32, u32, vp]
+    L.kz_pool_records.argtypes = [vp, i32, i32, vp, i64, vp, vp, vp, vp]
+    L.kz_step_pool.argtypes = [vp, i32, i32, i32, i32, i32, vp, i32, vp, i64, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp,
+                               u64, u32, u32, vp, i32, vp, u64, vp, vp]
+    L.kz_reset_pool.argtypes = [vp, i32, i32, vp, i32, vp, i32, vp, u64, u32, vp, vp]
     L.kz_legal_mask.argtypes = [vp, i32, i32, vp, i64, vp, vp]
     L.kz_observe.argtypes = [vp, i32, i32, vp, i64, vp]
     L.kz_errors.argtypes = [vp, i32, i32, vp, i32, vp]

@@ -593,6 +593,12 @@ struct StepParams {
   uint32_t* bitmap_out;  // the legal bitmap [n][bitmap_stride] (modes 0-2; mode 2 writes it instead of the mask row)
   long long bitmap_stride;  // words per bitmap row (>= BITMAP_WORDS, a multiple of 4)
   uint32_t* cobs_out;  // optional compact observation [n][KZ_COBS_WORDS] (kz_step_rollout / kz_legal_bitmap)
+  // start-position pool (kz_step_pool; read by the POOL instantiations only)
+  const uint32_t* pool;          // [pool_size][KZ_POOL_RECORD_WORDS] records (kz_pool_records)
+  int pool_size;
+  const int32_t* pool_pick;      // optional: record of each game that restarts in this launch
+  unsigned long long pool_seed;  // otherwise drawn from rand32(pool_seed, env_offset + g, finished episodes)
+  int32_t* start_ids;            // optional: receives the record index of each game that restarts
 };
 
 __device__ __forceinline__ uint16_t ld_u16(const uint8_t* p) { return (uint16_t)(p[0] | (p[1] << 8)); }
@@ -602,7 +608,9 @@ __device__ __forceinline__ void st_u16(uint8_t* p, int v) { p[0] = (uint8_t)v; p
 // 13,527-bit legal bitmap is written out instead.
 // MODE 1 = step (the hot kernel: only the fast paths are compiled in, the generator is inlined), MODE 0 = refresh
 // (loaded positions: nested-generation uchifuzume, full key, optional termination evaluation).
-template <int MODE>
+// POOL (modes 1 and 2, kz_step_pool): a finished game restarts from a record of the start-position pool instead of the
+// start position; nothing else differs.
+template <int MODE, bool POOL = false>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_kernel(const StepParams P) {
   for (int i = threadIdx.x; i < 81 * 8 * 3; i += blockDim.x) s_ray[i] = g_ray[i];
   for (int i = threadIdx.x; i < NCLS * 81 * 3; i += blockDim.x) s_step[i] = g_step[i];
@@ -1042,21 +1050,47 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
 
     if (MODE != 0 && status != 0 && P.auto_reset) {
       // StepManager.handle_episode_end -> game.reset() (step_manager.py:437-440; shogi_game.py:113-130)
-      __syncwarp();
-      if (lane < 24) reinterpret_cast<uint32_t*>(ws.board)[lane] = reinterpret_cast<const uint32_t*>(c_init_board)[lane];
-      if (lane < 14) ws.meta[lane] = 0;
-      side = 0; status = 0; winner = -1; move_count = 0; hist_len = 0;
-      episodes += 1;
-      key = make_uint4(reinterpret_cast<const uint32_t*>(c_init_board)[21], reinterpret_cast<const uint32_t*>(c_init_board)[22],
-                       reinterpret_cast<const uint32_t*>(c_init_board)[23], c_init_key_w);
-      {
-        uint4* tb = P.hist + (size_t)g * P.rep_slots;
-        for (int i = lane; i < P.rep_slots; i += 32) tb[i] = make_uint4(0, 0, 0, 0);
+      if constexpr (POOL) {
+        // the same reset from record k of the start-position pool: state rows, position key, legal bitmap, count and
+        // in-check flag as kz_pool_records packed them from kz_refresh / kz_legal_bitmap (DESIGN.md section 4.9)
+        episodes += 1;
+        uint32_t k = P.pool_pick ? (uint32_t)P.pool_pick[g]
+                                 : (uint32_t)(((unsigned long long)rand32(P.pool_seed, (unsigned long long)P.env_offset + g,
+                                                                          episodes) * (unsigned long long)P.pool_size) >> 32);
+        if (k >= (uint32_t)P.pool_size) k %= (uint32_t)P.pool_size;
+        const uint32_t* rec = P.pool + (size_t)k * KZ_POOL_RECORD_WORDS;
+        const uint8_t* rmeta = reinterpret_cast<const uint8_t*>(rec + 24);
+        __syncwarp();
+        if (lane < 24) reinterpret_cast<uint32_t*>(ws.board)[lane] = rec[lane];
+        if (lane < 14) ws.meta[lane] = rmeta[lane];
+        side = rmeta[14]; status = 0; winner = -1; move_count = ld_u16(rmeta + 18); hist_len = 0;
+        key = make_uint4(rec[21], rec[22], rec[23], rec[31]);
+        {
+          uint4* tb = P.hist + (size_t)g * P.rep_slots;
+          for (int i = lane; i < P.rep_slots; i += 32) tb[i] = make_uint4(0, 0, 0, 0);
+        }
+        for (int i = lane; i < BITMAP_WORDS; i += 32) ws.bitmap[i] = rec[KZ_POOL_BITMAP_OFFSET + i];
+        gr.count = (int)rec[32];
+        gr.in_check = rec[33] != 0;
+        if (lane == 0 && P.start_ids) P.start_ids[g] = (int32_t)k;
+        __syncwarp();
+      } else {
+        __syncwarp();
+        if (lane < 24) reinterpret_cast<uint32_t*>(ws.board)[lane] = reinterpret_cast<const uint32_t*>(c_init_board)[lane];
+        if (lane < 14) ws.meta[lane] = 0;
+        side = 0; status = 0; winner = -1; move_count = 0; hist_len = 0;
+        episodes += 1;
+        key = make_uint4(reinterpret_cast<const uint32_t*>(c_init_board)[21], reinterpret_cast<const uint32_t*>(c_init_board)[22],
+                         reinterpret_cast<const uint32_t*>(c_init_board)[23], c_init_key_w);
+        {
+          uint4* tb = P.hist + (size_t)g * P.rep_slots;
+          for (int i = lane; i < P.rep_slots; i += 32) tb[i] = make_uint4(0, 0, 0, 0);
+        }
+        for (int i = lane; i < BITMAP_WORDS; i += 32) ws.bitmap[i] = g_init_bitmap[i];
+        gr.count = 30;
+        gr.in_check = false;
+        __syncwarp();
       }
-      for (int i = lane; i < BITMAP_WORDS; i += 32) ws.bitmap[i] = g_init_bitmap[i];
-      gr.count = 30;
-      gr.in_check = false;
-      __syncwarp();
     }
 
     // ---- outputs
@@ -1467,6 +1501,60 @@ __global__ void kz_reset_kernel(uint8_t* boards, uint8_t* meta, uint4* rep, int 
   }
 }
 
+// kz_reset_pool: as kz_reset_kernel, from record k of the start-position pool (same selection as kz_step_kernel<.., true>;
+// the finished-episode counter is kept and not advanced)
+__global__ void kz_reset_pool_kernel(uint8_t* boards, uint8_t* meta, uint4* rep, int rep_slots, int n, const uint8_t* env_mask,
+                                     int max_moves, const uint32_t* pool, int pool_size, const int32_t* pick,
+                                     unsigned long long pool_seed, uint32_t env_offset, int32_t* start_ids) {
+  const int g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (g >= n) return;
+  if (env_mask && !env_mask[g]) return;
+  uint32_t* m = reinterpret_cast<uint32_t*>(meta + (size_t)g * 32);
+  const uint32_t episodes = m[6];
+  __syncwarp();
+  uint32_t k = pick ? (uint32_t)pick[g]
+                    : (uint32_t)(((unsigned long long)rand32(pool_seed, (unsigned long long)env_offset + g, episodes) *
+                                  (unsigned long long)pool_size) >> 32);
+  if (k >= (uint32_t)pool_size) k %= (uint32_t)pool_size;
+  const uint32_t* rec = pool + (size_t)k * KZ_POOL_RECORD_WORDS;
+  for (int i = lane; i < rep_slots; i += 32) rep[(size_t)g * rep_slots + i] = make_uint4(0, 0, 0, 0);
+  uint32_t* b = reinterpret_cast<uint32_t*>(boards + (size_t)g * 96);
+  if (lane < 24) b[lane] = rec[lane];
+  else {
+    const int w = lane - 24;
+    uint32_t v = rec[24 + w];                                             // hands, side, status 0, winner none, err 0, move_count
+    if (w == 5) v = ((uint32_t)max_moves & 0xFFFF) << 16;                 // bytes 20..23: hist_len 0, max_moves
+    if (w == 6) v = episodes;                                             // keep the finished-episode counter
+    m[w] = v;                                                             // w == 7: word w of the position key
+  }
+  if (lane == 0 && start_ids) start_ids[g] = (int32_t)k;
+}
+
+// kz_pool_records: one start-position record per game of a refreshed scratch batch (layout: keisei_b200.h)
+__global__ void kz_pool_records_kernel(const uint8_t* boards, const uint8_t* meta, int n, const uint32_t* bitmap,
+                                       long long bitmap_stride, const int32_t* legal_count, const uint8_t* in_check,
+                                       uint32_t* records) {
+  const int g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (g >= n) return;
+  uint32_t* rec = records + (size_t)g * KZ_POOL_RECORD_WORDS;
+  if (lane < 24) rec[lane] = reinterpret_cast<const uint32_t*>(boards + (size_t)g * 96)[lane];
+  else {
+    const int w = lane - 24;
+    uint32_t v = reinterpret_cast<const uint32_t*>(meta + (size_t)g * 32)[w];
+    if (w == 3) v &= 0x00FFFFFFu;  // bytes 12..15: hands, side to move, status 0
+    if (w == 4) v = (v & 0xFFFF0000u) | 0xFFu;  // bytes 16..19: winner none, err 0, move_count
+    if (w == 5 || w == 6) v = 0;  // plies since reset, max_moves (the env's own applies), finished episodes
+    rec[24 + w] = v;
+  }
+  if (lane == 0) rec[32] = (uint32_t)legal_count[g];
+  if (lane == 1) rec[33] = in_check[g];
+  if (lane >= 2) for (int i = 32 + lane; i < KZ_POOL_BITMAP_OFFSET; i += 30) rec[i] = 0;
+  const uint32_t* src = bitmap + (size_t)g * bitmap_stride;
+  for (int i = lane; i < BITMAP_WORDS; i += 32) rec[KZ_POOL_BITMAP_OFFSET + i] = src[i];
+}
+
 __global__ void kz_load_kernel(uint8_t* boards, uint8_t* meta, uint4* rep, int rep_slots, int n, const int8_t* src_b,
                                const uint8_t* src_h, const uint8_t* src_side, const int32_t* src_mc,
                                const int32_t* src_mm) {
@@ -1628,7 +1716,11 @@ int launch_step(void* state, int n, int hist_cap, StepParams P, cudaStream_t st,
     CK(cudaMemsetAsync(P.tile_counter, 0, sizeof(int), st));
   }
 #endif
-  if (P.mode == 1) kz_step_kernel<1><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
+  if (P.pool) {
+    if (P.mode == 1) kz_step_kernel<1, true><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
+    else if (P.mode == 2) kz_step_kernel<2, true><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
+    else return KZ_E_ARG;
+  } else if (P.mode == 1) kz_step_kernel<1><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
   else if (P.mode == 2) kz_step_kernel<2><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
   else kz_step_kernel<0><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
   CK(cudaGetLastError());
@@ -1730,6 +1822,8 @@ int kz_init_tables(void* stream) {
     CK(cudaFuncSetAttribute(kz_step_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
     CK(cudaFuncSetAttribute(kz_step_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
     CK(cudaFuncSetAttribute(kz_step_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
+    CK(cudaFuncSetAttribute(kz_step_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
+    CK(cudaFuncSetAttribute(kz_step_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
   }
   g_ready[dev] = true;
   // legal bitmap of the start position, computed once by the engine itself on a scratch game
@@ -1765,6 +1859,33 @@ int kz_reset(void* state, int n, int hist_cap, const uint8_t* env_mask, int max_
   uint8_t* base = reinterpret_cast<uint8_t*>(state);
   kz_reset_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
       base + L.off_boards, base + L.off_meta, reinterpret_cast<uint4*>(base + L.off_hist), L.rep_slots, n, env_mask, max_moves);
+  CK(cudaGetLastError());
+  return KZ_OK;
+}
+
+int kz_reset_pool(void* state, int n, int hist_cap, const uint8_t* env_mask, int max_moves, const uint32_t* pool, int pool_size,
+                  const int32_t* pick, uint64_t pool_seed, uint32_t env_offset, int32_t* start_ids, void* stream) {
+  if (!state || n <= 0 || max_moves < 0 || max_moves > 65535 || !pool || pool_size <= 0 || ((uintptr_t)pool & 15))
+    return KZ_E_ARG;
+  if (!host_ready()) return KZ_E_NOT_INIT;
+  const Layout L = layout(n, hist_cap);
+  uint8_t* base = reinterpret_cast<uint8_t*>(state);
+  kz_reset_pool_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      base + L.off_boards, base + L.off_meta, reinterpret_cast<uint4*>(base + L.off_hist), L.rep_slots, n, env_mask, max_moves,
+      pool, pool_size, pick, pool_seed, env_offset, start_ids);
+  CK(cudaGetLastError());
+  return KZ_OK;
+}
+
+int kz_pool_records(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words,
+                    const int32_t* legal_count, const uint8_t* in_check, uint32_t* records, void* stream) {
+  if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535 || !bitmap || bitmap_stride_words < BITMAP_WORDS || !legal_count ||
+      !in_check || !records || ((uintptr_t)records & 15))
+    return KZ_E_ARG;
+  const Layout L = layout(n, hist_cap);
+  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
+  kz_pool_records_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      base + L.off_boards, base + L.off_meta, n, bitmap, bitmap_stride_words, legal_count, in_check, records);
   CK(cudaGetLastError());
   return KZ_OK;
 }
@@ -1852,6 +1973,25 @@ int kz_step_range(void* state, int n, int hist_cap, int first, int count, int co
   P.legal_count = legal_count; P.next_actions = next_actions;
   P.seed = seed; P.rng_step = rng_step; P.env_offset = env_offset;
   P.auto_reset = auto_reset; P.mode = bitmap ? 2 : 1;
+  return launch_step(state, n, hist_cap, P, reinterpret_cast<cudaStream_t>(stream), first, count, counter_slot);
+}
+
+int kz_step_pool(void* state, int n, int hist_cap, int first, int count, int counter_slot, const void* actions,
+                 int actions_i64, float* obs, int64_t obs_stride, uint8_t* mask, int64_t mask_stride, uint32_t* bitmap,
+                 int64_t bitmap_stride_words, uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner,
+                 int32_t* ep_len, int32_t* legal_count, void* next_actions, uint64_t seed, uint32_t rng_step,
+                 uint32_t env_offset, const uint32_t* pool, int pool_size, const int32_t* pick, uint64_t pool_seed,
+                 int32_t* start_ids, void* stream) {
+  if (!actions || (mask && bitmap) || !pool || pool_size <= 0 || ((uintptr_t)pool & 15)) return KZ_E_ARG;
+  StepParams P{};
+  P.actions = actions; P.actions_i64 = actions_i64;
+  P.obs = obs; P.obs_stride = obs_stride; P.mask = mask; P.mask_stride = mask_stride;
+  P.bitmap_out = bitmap; P.bitmap_stride = bitmap_stride_words; P.cobs_out = cobs;
+  P.reward = reward; P.done = done; P.reason = reason; P.winner = winner; P.ep_len = ep_len;
+  P.legal_count = legal_count; P.next_actions = next_actions;
+  P.seed = seed; P.rng_step = rng_step; P.env_offset = env_offset;
+  P.auto_reset = 1; P.mode = bitmap ? 2 : 1;
+  P.pool = pool; P.pool_size = pool_size; P.pool_pick = pick; P.pool_seed = pool_seed; P.start_ids = start_ids;
   return launch_step(state, n, hist_cap, P, reinterpret_cast<cudaStream_t>(stream), first, count, counter_slot);
 }
 

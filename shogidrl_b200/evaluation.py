@@ -12,7 +12,7 @@ from __future__ import annotations
 import json
 from dataclasses import dataclass, field
 from pathlib import Path
-from typing import Any, Dict, List, Mapping, Optional, Tuple
+from typing import Any, Dict, List, Mapping, Optional, Sequence, Tuple
 
 import torch
 
@@ -30,6 +30,7 @@ class EvaluationResult:
     draws: int
     mean_length: float
     outcomes: List[str] = field(default_factory=list)  # one of OUTCOMES per finished game, in completion order
+    start_ids: List[int] = field(default_factory=list)  # with start_positions: the opening of each game of outcomes
 
     @property
     def win_rate(self) -> float:
@@ -48,9 +49,34 @@ def _player_kind(player) -> str:
     return "agent"
 
 
+def paired_openings(games_begun: torch.Tensor, pool_size: int) -> torch.Tensor:
+    """Opening of the next game of every env in a paired evaluation: envs 2i and 2i+1 form pair i, and the j-th game
+    (j = ``games_begun``, counted from 0) of both envs of pair i starts from opening (i + (n/2) * j) mod pool_size, so
+    the pairs walk through the pool side by side and each opening is played once from each side before any repeats.
+    -> int32 [n] on the device of ``games_begun``."""
+    n = games_begun.shape[0]
+    pair = torch.arange(n, device=games_begun.device) // 2
+    return ((pair + (n // 2) * games_begun) % pool_size).to(torch.int32)
+
+
+def _num_envs(num_games: int, num_envs: int, paired: bool) -> int:
+    """Envs of an evaluation batch: at most one per game and at least two; with paired openings an even number (pairs
+    of envs share an opening and a quota), two even when ``num_envs`` is 1."""
+    if num_games < 0 or num_envs < 1:
+        raise ValueError(f"num_games = {num_games}, num_envs = {num_envs}: need num_games >= 0 and num_envs >= 1")
+    n = min(num_envs, max(2, num_games))
+    if paired:
+        if num_games % 2:
+            raise ValueError(f"num_games = {num_games}: with start_positions every opening is played from both sides, so "
+                             "num_games must be even")
+        n = max(2, n - n % 2)
+    return n
+
+
 def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int = 1024, max_moves_per_game: int = 500,
                          device="cuda", seed: int = 0, deterministic: bool = True,
-                         max_steps: Optional[int] = None) -> EvaluationResult:
+                         max_steps: Optional[int] = None, start_positions: Optional[Sequence[str]] = None
+                         ) -> EvaluationResult:
     """Play ``num_games`` games of ``agent`` against ``opponent`` (None = uniform-random legal moves).  Either side may
     be an agent-like object, ``"random"``, ``"heuristic"`` or an instance of the two scripted opponent classes; results
     are counted from ``agent``'s side.  The agent plays Black in even-numbered envs and White in odd-numbered ones.
@@ -58,16 +84,29 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
     are ignored, so the sample is ``num_games`` independent games exactly as the reference's sequential loop plays them
     -- counting "the first num_games completions of the batch" would over-sample short (decisive) games, because a
     fast env restarts and finishes again while the long draws are still running.  Every tensor stays on the device;
-    the host reads four counters per step."""
+    the host reads four counters per step.
+
+    ``start_positions`` (a sequence of SFEN strings): games start from these openings instead of the start position,
+    paired -- both games of a pair of envs start from the same opening, the agent playing Black in one and White in the
+    other (``paired_openings``) -- so that two deterministic players do not repeat the same two games.  ``num_games`` must
+    then be even (and at least two envs run); ``EvaluationResult.start_ids`` gives each counted game's opening.  A game's
+    length (``mean_length``) is its move count at the end, which continues from the opening's move number as the
+    reference's ``ShogiGame.from_sfen`` does: subtract ``move number - 1`` of the opening for the plies played."""
     kinds = (_player_kind(agent), _player_kind(opponent))
     random_actions = "random" in kinds
-    n = min(num_envs, max(2, num_games))
-    env = VecShogiEnv(n, max_moves_per_game=max_moves_per_game, device=device, seed=seed, auto_reset=True)
+    n = _num_envs(num_games, num_envs, start_positions is not None)
+    env = VecShogiEnv(n, max_moves_per_game=max_moves_per_game, device=device, seed=seed, auto_reset=True,
+                      start_positions=start_positions)
     dev = env.device
     agent_is_black = (torch.arange(n, device=dev) % 2) == 0
     quota = torch.full((n,), num_games // n, dtype=torch.int64, device=dev)
     quota[: num_games % n] += 1
     completed = torch.zeros(n, dtype=torch.int64, device=dev)
+    pooled = env.pool is not None
+    if pooled:
+        pool_size = env.pool.shape[0]
+        finished = torch.zeros(n, dtype=torch.int64, device=dev)  # games each env has finished, quota or not
+        env.reset(refresh=False, start_pick=paired_openings(finished, pool_size))
     env.refresh(random_actions=True)
     heuristic = env.heuristic_actions() if "heuristic" in kinds else None
 
@@ -82,6 +121,7 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
     done_games = agent_w = opp_w = draws = 0
     length_sum = 0
     outcomes: List[str] = []
+    start_ids: List[int] = []
     steps = 0
     limit = max_steps if max_steps is not None else (max_moves_per_game + 1) * (1 + num_games // n) + 8
     while done_games < num_games and steps < limit:
@@ -90,7 +130,12 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
         a_agent = actions_of(agent, kinds[0])
         a_opp = actions_of(opponent, kinds[1])
         actions = torch.where(agent_turn, a_agent, a_opp).contiguous()
-        out = env.step(actions, random_actions=random_actions)
+        if pooled:
+            playing = env.start_ids.clone()  # the openings of the games this step may finish
+            out = env.step(actions, random_actions=random_actions, start_pick=paired_openings(finished + 1, pool_size))
+            finished += out["done"] != 0
+        else:
+            out = env.step(actions, random_actions=random_actions)
         if heuristic is not None:
             env.heuristic_actions(out=heuristic)  # for the returned state (auto-reset applied)
         steps += 1
@@ -101,12 +146,15 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
             agent_won = d & (((w == 0) & agent_is_black) | ((w == 1) & ~agent_is_black))
             opp_won = d & (w >= 0) & ~agent_won
             codes = (agent_won.long() + 2 * opp_won.long())[d]  # index into OUTCOMES, env order
-            stats = torch.cat([torch.stack([d.sum(), agent_won.sum(), opp_won.sum(), (out["ep_len"] * d).sum()]),
-                               codes]).tolist()  # one device-to-host read per step that finished a game
+            parts = [torch.stack([d.sum(), agent_won.sum(), opp_won.sum(), (out["ep_len"] * d).sum()]), codes]
+            if pooled:
+                parts.append(playing.long()[d])
+            stats = torch.cat(parts).tolist()  # one device-to-host read per step that finished a game
             done_games += stats[0]; agent_w += stats[1]; opp_w += stats[2]; length_sum += stats[3]
             draws += stats[0] - stats[1] - stats[2]
-            outcomes.extend(OUTCOMES[c] for c in stats[4:])
-    return EvaluationResult(done_games, agent_w, opp_w, draws, length_sum / max(1, done_games), outcomes)
+            outcomes.extend(OUTCOMES[c] for c in stats[4: 4 + stats[0]])
+            start_ids.extend(stats[4 + stats[0]:])
+    return EvaluationResult(done_games, agent_w, opp_w, draws, length_sum / max(1, done_games), outcomes, start_ids)
 
 
 # ---------------------------------------------------------------------------------------------------------------

@@ -6,7 +6,7 @@ owns its own games and only gradients (DDP) and three normalisation scalars cros
 from __future__ import annotations
 
 import time
-from typing import Callable, Dict, Iterable, Optional
+from typing import Callable, Dict, Iterable, Optional, Sequence
 
 import torch
 
@@ -19,13 +19,13 @@ from .step_manager import VecStepManager
 
 class SelfPlayTrainer:
     def __init__(self, model, config, num_envs: int, horizon: int, device="cuda", use_mixed_precision: bool = True,
-                 total_envs: Optional[int] = None):
+                 total_envs: Optional[int] = None, start_positions: Optional[Sequence[str]] = None):
         rank, world = kd.world()
         self.device = torch.device(device)
         offset = kd.shard_envs(total_envs, rank, world)[0] if total_envs else rank * num_envs
         seed = getattr(config.env, "seed", 0) or 0
         self.env = VecShogiEnv(num_envs, max_moves_per_game=config.env.max_moves_per_game, device=self.device,
-                               seed=int(seed), env_offset=offset, auto_reset=True)
+                               seed=int(seed), env_offset=offset, auto_reset=True, start_positions=start_positions)
         self.agent = PPOAgent(model, config, self.device, use_mixed_precision=use_mixed_precision)
         self.agent.model.sample_seed = int(seed) * 7919 + rank
         self.agent.enable_ddp()
@@ -34,6 +34,14 @@ class SelfPlayTrainer:
         self.global_timestep = 0
         self.current_epoch = 0
         self.rank, self.world = rank, world
+
+    def set_start_positions(self, sfens: Optional[Sequence[str]]) -> None:
+        """Start the games that finish from now on from this pool of SFEN positions (None: the start position again),
+        e.g. a curriculum that changes between epochs; games in progress continue.  See
+        ``VecShogiEnv.set_start_positions``.  The captured rollout graph names the old pool and is recaptured on the next
+        ``collect``."""
+        self.env.set_start_positions(sfens)
+        self.driver.drop_graph()
 
     def collect(self) -> Dict[str, int]:
         self.driver.collect()

@@ -256,6 +256,7 @@ class VecStepManager:
         tr = getattr(getattr(agent, "config", None), "training", None)
         self.graph_rollout = bool(getattr(tr, "cuda_graph_rollout", True))
         self._graph = None
+        self._graph_pool = None  # the start-position pool (address, size) the captured rollout launches with
         self._eager_runs = 0
         self.model_eval_mode = False  # True: sample from the network in eval() (the reference's worker processes)
 
@@ -281,11 +282,14 @@ class VecStepManager:
             model.cache_inference_weights()  # once per rollout, outside the captured loop (fixed addresses)
         try:
             if self.graph_rollout and self.env.device.type == "cuda":
+                pool = self._pool_key()
+                if self._graph is not None and pool != self._graph_pool:
+                    self.drop_graph()  # its step launches name the replaced (or removed) start-position pool
                 if self._graph is None and self._eager_runs >= 1:
                     graph = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(graph):
                         self._collect_steps()
-                    self._graph = graph
+                    self._graph, self._graph_pool = graph, pool
                 if self._graph is not None:
                     self._graph.replay()
                     return
@@ -294,6 +298,14 @@ class VecStepManager:
         finally:
             if cached:
                 model.cache_inference_weights(live=False)  # the parameters are about to change (PPO update)
+
+    def _pool_key(self):
+        pool = getattr(self.env, "pool", None)
+        return None if pool is None else (pool.data_ptr(), pool.shape[0])
+
+    def drop_graph(self) -> None:
+        """Forget the captured rollout; the next ``collect`` captures a new one."""
+        self._graph, self._graph_pool = None, None
 
     def _collect_steps(self) -> None:
         b, env = self.buffer, self.env

@@ -6,7 +6,7 @@ GPU; observations and masks are written by the kernel straight into caller-provi
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional
+from typing import Dict, Optional, Sequence
 
 import numpy as np
 import torch
@@ -14,10 +14,38 @@ import torch
 from . import _native as nv
 
 
+def parse_start_positions(sfens: Sequence[str], max_moves: int):
+    """Parse a start-position pool on the host: -> (boards int8 [P, 81], hands uint8 [P, 14], sides uint8 [P],
+    move_counts int32 [P]).  Raises ValueError naming the index of the first entry that does not parse or whose move
+    number already reaches ``max_moves``."""
+    from .shogi.sfen import pack_sfen
+    if isinstance(sfens, str):
+        raise ValueError("start positions: expected a sequence of SFEN strings, got one string")
+    packed = []
+    for i, s in enumerate(sfens):
+        try:
+            p = pack_sfen(str(s))
+        except Exception as e:  # the SFEN parser raises ValueError, KeyError or IndexError on malformed text
+            raise ValueError(f"start position {i} ({s!r}) does not parse: {e}") from e
+        if p[3] >= max_moves:
+            raise ValueError(f"start position {i} ({s!r}) is terminal at load: move count {p[3]} >= max_moves {max_moves}")
+        packed.append(p)
+    if not packed:
+        raise ValueError("start positions: the pool is empty (pass None to restart from the start position)")
+    return (np.stack([p[0] for p in packed]), np.stack([p[1] for p in packed]),
+            np.asarray([p[2] for p in packed], np.uint8), np.asarray([p[3] for p in packed], np.int32))
+
+
 class VecShogiEnv:
+    # Pool draws are keyed by seed ^ POOL_SALT (auto-reset inside kz_step_pool) and seed ^ POOL_RESET_SALT (explicit
+    # reset), so that they are independent of the fused random actions and of each other: a reset() right after an
+    # auto-reset (same finished-episode counter) does not redraw the same entry.
+    POOL_SALT = 0x506F6F6C5374  # "PoolSt"
+    POOL_RESET_SALT = 0x506F6F6C5273  # "PoolRs"
+
     def __init__(self, num_envs: int, max_moves_per_game: int = 500, device="cuda", seed: int = 1234,
                  env_offset: int = 0, auto_reset: bool = True, hist_cap: Optional[int] = None,
-                 step_streams: Optional[int] = None):
+                 step_streams: Optional[int] = None, start_positions: Optional[Sequence[str]] = None):
         self.device = nv.require_cuda(device)
         self.n = int(num_envs)
         self.max_moves = int(max_moves_per_game)
@@ -60,6 +88,14 @@ class VecShogiEnv:
         if self.n % (8 * self.step_streams) != 0:
             self.step_streams = 1
         self._side_streams = [torch.cuda.Stream(device=d) for _ in range(self.step_streams)] if self.step_streams > 1 else []
+        # start-position pool (set_start_positions): records on the device, and the pool index of each env's current game
+        # (-1: begun from the start position).  _ids_in_use: some entry may still name a pool entry while no pool is set,
+        # so resets from the start position must write -1 over it.
+        self.pool: Optional[torch.Tensor] = None
+        self.start_ids = torch.full((self.n,), -1, dtype=torch.int32, device=d)
+        self._ids_in_use = False
+        if start_positions is not None:
+            self.set_start_positions(start_positions, reset=False)
         self.reset()
 
     # ------------------------------------------------------------------ helpers
@@ -89,14 +125,104 @@ class VecShogiEnv:
     def _mask_args(self, mask: Optional[torch.Tensor]):
         return self._rows_arg(mask, "mask", (torch.uint8, torch.bool), nv.NUM_ACTIONS)
 
+    def _pick_arg(self, start_pick: Optional[torch.Tensor], in_step: bool = True):
+        if start_pick is None:
+            return None
+        if self.pool is None:
+            raise ValueError("start_pick needs a start-position pool (set_start_positions)")
+        if in_step and not self.auto_reset:
+            raise ValueError("start_pick: this env does not reset finished games (auto_reset=False), so no game would "
+                             "start from it; use reset(start_pick=...)")
+        if (start_pick.device != self.device or start_pick.dtype != torch.int32 or not start_pick.is_contiguous()
+                or start_pick.numel() < self.n):
+            raise ValueError(f"start_pick: expected a contiguous int32 [{self.n}] tensor on {self.device}, got "
+                             f"{tuple(start_pick.shape)} {start_pick.dtype} on {start_pick.device}")
+        return start_pick.data_ptr()
+
     # ------------------------------------------------------------------ API
-    def reset(self, env_mask: Optional[torch.Tensor] = None, refresh: bool = True, random_actions: bool = False):
-        """ShogiGame.reset for all (or the masked) envs; returns (obs, mask) of the new positions."""
+    def set_start_positions(self, sfens: Optional[Sequence[str]], reset: bool = False) -> None:
+        """Restart finished games from a pool of SFEN positions instead of the start position (None: back to the start
+        position).  Every game that finishes from now on -- in ``step`` / ``step_rollout`` or through ``reset()`` --
+        starts from a uniformly drawn entry, or from the entry a step's ``start_pick`` names.  ``start_ids`` (int32 [n])
+        holds, for each env's current game, its entry in the pool that was set when that game started, or -1 if it
+        started from the start position; games in progress continue and keep their ids when the pool changes, and
+        ``reset=True`` restarts every env from the new pool (or the start position) at once.  Each entry is parsed on the host and its record (board, hands, side to move, move number, position key,
+        legal bitmap, legal count, in-check flag) is computed once on the device by the engine's refresh path
+        (kz_pool_records).  Raises ValueError naming the index of an entry that does not parse, is terminal at load
+        (checkmate, stalemate, move number >= max_moves) or lets the side to move capture the opponent's king."""
+        if sfens is None:
+            self.pool = None
+        else:
+            self.pool = self._build_pool(parse_start_positions(sfens, self.max_moves))
+            self._ids_in_use = True
+        if reset:
+            self.reset()
+
+    def _build_pool(self, parsed) -> torch.Tensor:
+        """Pool records (int32 [P, POOL_RECORD_WORDS]) of parsed positions: kz_load_positions + kz_refresh
+        (termination, in-check) + kz_legal_bitmap on a scratch batch of the P positions, then kz_pool_records."""
+        boards, hands, sides, mcs = parsed
+        P, d, sp = len(sides), self.device, self._sp()
+        offs, total = (C.c_int64 * 3)(), C.c_int64()
+        nv.check(self._L.kz_state_layout(P, 0, offs, C.byref(total)), "kz_state_layout")
+        state = torch.zeros(total.value, dtype=torch.uint8, device=d)
+        dev = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt).to(d).contiguous()  # noqa: E731
+        b, h, s, mc = dev(boards, torch.int8), dev(hands, torch.uint8), dev(sides, torch.uint8), dev(mcs, torch.int32)
+        mm = torch.full((P,), self.max_moves, dtype=torch.int32, device=d)
+        nv.check(self._L.kz_load_positions(state.data_ptr(), P, 0, b.data_ptr(), h.data_ptr(), s.data_ptr(), mc.data_ptr(),
+                                           mm.data_ptr(), sp), "kz_load_positions")
+        count = torch.zeros(P, dtype=torch.int32, device=d)
+        check = torch.zeros(P, dtype=torch.uint8, device=d)
+        nv.check(self._L.kz_refresh(state.data_ptr(), P, 0, None, 0, None, 0, count.data_ptr(), None, 1, 0, 0, 0, 1,
+                                    check.data_ptr(), sp), "kz_refresh")
+        bitmap = torch.zeros((P, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
+        nv.check(self._L.kz_legal_bitmap(state.data_ptr(), P, 0, None, 0, bitmap.data_ptr(), nv.BITMAP_WORDS, None,
+                                         count.data_ptr(), sp), "kz_legal_bitmap")
+        meta = torch.empty((P, 8), dtype=torch.int32, device=d)
+        nv.check(self._L.kz_export_positions(state.data_ptr(), P, 0, None, None, meta.data_ptr(), sp), "kz_export_positions")
+        # a legal board move onto the square of the opponent's king (kz_step flags that as KZ_ERR_KING_CAPTURE)
+        side = s.long()
+        ksq = torch.where(b == (8 + 14 * (1 - side))[:, None], torch.arange(81, device=d), 81).amin(1)  # 81: no king
+        frm = torch.arange(81, device=d)[None, :]
+        to = ksq[:, None].clamp(max=80)
+        idx = ((frm * 80 + to - (to > frm).long()) * 2)[:, :, None] + torch.arange(2, device=d)
+        bits = (bitmap.long().gather(1, (idx >> 5).view(P, -1)) >> (idx & 31).view(P, -1)) & 1
+        ok_from = ((frm != to) & (ksq[:, None] < 81))[:, :, None].expand(P, 81, 2).reshape(P, -1)
+        king_capture = ((bits != 0) & ok_from).any(1)
+        status, count_h, kc = meta[:, 3].cpu(), count.cpu(), king_capture.cpu()
+        for i in range(P):
+            if int(status[i]) != 0 or int(count_h[i]) == 0:
+                raise ValueError(f"start position {i} is terminal at load ({nv.REASONS.get(int(status[i])) or 'no legal move'})")
+            if bool(kc[i]):
+                raise ValueError(f"start position {i} lets the side to move capture the opponent's king")
+        records = torch.empty((P, nv.POOL_RECORD_WORDS), dtype=torch.int32, device=d)
+        nv.check(self._L.kz_pool_records(state.data_ptr(), P, 0, bitmap.data_ptr(), nv.BITMAP_WORDS, count.data_ptr(),
+                                         check.data_ptr(), records.data_ptr(), sp), "kz_pool_records")
+        return records
+
+    def reset(self, env_mask: Optional[torch.Tensor] = None, refresh: bool = True, random_actions: bool = False,
+              start_pick: Optional[torch.Tensor] = None):
+        """ShogiGame.reset for all (or the masked) envs; returns (obs, mask) of the new positions.  With a start-position
+        pool the envs restart from pool entries (``start_pick``: int32 [n] entry per env, default a uniform draw)."""
         mp = None
         if env_mask is not None:
             env_mask = env_mask.to(device=self.device, dtype=torch.uint8).contiguous()
             mp = env_mask.data_ptr()
-        nv.check(self._L.kz_reset(self.state.data_ptr(), self.n, self.hist_cap, mp, self.max_moves, self._sp()), "kz_reset")
+        pk = self._pick_arg(start_pick, in_step=False)
+        if self.pool is not None:
+            nv.check(self._L.kz_reset_pool(self.state.data_ptr(), self.n, self.hist_cap, mp, self.max_moves,
+                                           self.pool.data_ptr(), self.pool.shape[0], pk,
+                                           (self.seed ^ self.POOL_RESET_SALT) & 0xFFFFFFFFFFFFFFFF, self.env_offset,
+                                           self.start_ids.data_ptr(), self._sp()), "kz_reset_pool")
+        else:
+            nv.check(self._L.kz_reset(self.state.data_ptr(), self.n, self.hist_cap, mp, self.max_moves, self._sp()),
+                     "kz_reset")
+            if self._ids_in_use:
+                if env_mask is None:
+                    self.start_ids.fill_(-1)
+                    self._ids_in_use = False
+                else:
+                    self.start_ids.masked_fill_(env_mask != 0, -1)
         if env_mask is None:
             self.step_index = 0
         if refresh:
@@ -121,10 +247,11 @@ class VecShogiEnv:
 
     def step(self, actions: torch.Tensor, obs: Optional[torch.Tensor] = None, mask: Optional[torch.Tensor] = None,
              random_actions: bool = False, write_obs: bool = True, write_mask: bool = True,
-             next_out: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+             next_out: Optional[torch.Tensor] = None, start_pick: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         """make_move for every env.  ``obs`` / ``mask`` may point into a rollout buffer (e.g. obs_buf[t+1]).
         With ``random_actions`` the kernel also writes a uniform-random legal action for the returned state
-        into ``next_out`` (default ``self.next_actions``; must not alias ``actions``)."""
+        into ``next_out`` (default ``self.next_actions``; must not alias ``actions``).  With a start-position pool,
+        ``start_pick`` (int32 [n]) names the entry each env restarts from if its game finishes in this step."""
         if (actions.device != self.device or actions.dtype not in (torch.int64, torch.int32)
                 or not actions.is_contiguous() or actions.numel() < self.n):
             raise ValueError(f"actions: expected {self.n} contiguous int64/int32 policy indices on {self.device}, got "
@@ -140,9 +267,13 @@ class VecShogiEnv:
                 nxt = nxt.view(torch.int32)[: self.n]
             if nxt.data_ptr() == actions.data_ptr():
                 raise ValueError("next_out must not alias actions (the kernel reads one while writing the other)")
+        pk = self._pick_arg(start_pick)
         self.step_index += 1  # after validation: a rejected call leaves the RNG counter where it was
         if self.step_streams > 1:
-            self._step_ranges(actions, op, os_, mp, ms, None, 0, self.reward, self.done, nxt)
+            self._step_ranges(actions, op, os_, mp, ms, None, 0, self.reward, self.done, nxt, pick=pk)
+            self._restarted_from_start(self.done)
+        elif self._pooled():
+            self._step_pool(0, self.n, 0, actions, op, os_, mp, ms, None, 0, None, self.reward, self.done, nxt, pk, self._sp())
         else:
             nv.check(self._L.kz_step(self.state.data_ptr(), self.n, self.hist_cap, actions.data_ptr(),
                                      int(actions.dtype == torch.int64), op, os_, mp, ms, self.reward.data_ptr(),
@@ -150,18 +281,20 @@ class VecShogiEnv:
                                      self.ep_len.data_ptr(), self.legal_count.data_ptr(),
                                      nxt.data_ptr() if nxt is not None else None, self.seed, self.step_index,
                                      self.env_offset, int(self.auto_reset), self._sp()), "kz_step")
+        self._restarted_from_start(self.done)
         return {"obs": obs, "mask": mask, "reward": self.reward, "done": self.done, "reason": self.reason,
                 "winner": self.winner, "ep_len": self.ep_len, "legal_count": self.legal_count}
 
     def step_rollout(self, actions: torch.Tensor, obs: Optional[torch.Tensor], bitmap: torch.Tensor,
                      reward: Optional[torch.Tensor] = None, done: Optional[torch.Tensor] = None,
                      random_actions: bool = False, next_out: Optional[torch.Tensor] = None,
-                     cobs: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+                     cobs: Optional[torch.Tensor] = None, start_pick: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         """``step`` in its rollout form (kz_step_rollout): the successor's legal set is written as the 13,527-bit legal
         bitmap (int32 [n, 448] rows, e.g. ``RolloutBuffer.bitmaps[t + 1]``) instead of the byte mask -- 1.8 KB instead
         of 13.5 KB per game here and in every later pass of the sampler / PPO update over it.  ``obs`` as in ``step``
         (None: no observation rows); ``reward`` / ``done`` may point into rollout storage (fp32 / uint8 [n]); ``cobs``
-        (int32 [n, 40]) receives the compact observations the policy network's input layer reads (kz_cobs_conv_*)."""
+        (int32 [n, 40]) receives the compact observations the policy network's input layer reads (kz_cobs_conv_*);
+        ``start_pick`` as in ``step``."""
         if (actions.device != self.device or actions.dtype not in (torch.int64, torch.int32)
                 or not actions.is_contiguous() or actions.numel() < self.n):
             raise ValueError(f"actions: expected {self.n} contiguous int64/int32 policy indices on {self.device}")
@@ -180,9 +313,13 @@ class VecShogiEnv:
                 nxt = nxt.view(torch.int32)[: self.n]
             if nxt.data_ptr() == actions.data_ptr():
                 raise ValueError("next_out must not alias actions (the kernel reads one while writing the other)")
+        pk = self._pick_arg(start_pick)
         self.step_index += 1
         if self.step_streams > 1:
-            self._step_ranges(actions, op, os_, None, 0, bp, bs, reward, done, nxt, cp)
+            self._step_ranges(actions, op, os_, None, 0, bp, bs, reward, done, nxt, cp, pick=pk)
+            self._restarted_from_start(done)
+        elif self._pooled():
+            self._step_pool(0, self.n, 0, actions, op, os_, None, 0, bp, bs, cp, reward, done, nxt, pk, self._sp())
         else:
             nv.check(self._L.kz_step_rollout(self.state.data_ptr(), self.n, self.hist_cap, actions.data_ptr(),
                                              int(actions.dtype == torch.int64), op, os_, bp, bs, cp, reward.data_ptr(),
@@ -190,10 +327,28 @@ class VecShogiEnv:
                                              self.ep_len.data_ptr(), self.legal_count.data_ptr(),
                                              nxt.data_ptr() if nxt is not None else None, self.seed, self.step_index,
                                              self.env_offset, int(self.auto_reset), self._sp()), "kz_step_rollout")
+        self._restarted_from_start(done)
         return {"obs": obs, "bitmap": bitmap, "reward": reward, "done": done, "reason": self.reason,
                 "winner": self.winner, "ep_len": self.ep_len, "legal_count": self.legal_count}
 
-    def _step_ranges(self, actions, op, os_, mp, ms, bp, bs, reward, done, nxt, cp=None) -> None:
+    def _pooled(self) -> bool:
+        return self.pool is not None and self.auto_reset
+
+    def _restarted_from_start(self, done: torch.Tensor) -> None:
+        """After a launch without a pool: games that finished restarted from the start position (start_ids -1)."""
+        if self._ids_in_use and self.pool is None and self.auto_reset:
+            self.start_ids.masked_fill_(done[: self.n] != 0, -1)
+
+    def _step_pool(self, first, count, slot, actions, op, os_, mp, ms, bp, bs, cp, reward, done, nxt, pick, stream) -> None:
+        nv.check(self._L.kz_step_pool(self.state.data_ptr(), self.n, self.hist_cap, first, count, slot, actions.data_ptr(),
+                                      int(actions.dtype == torch.int64), op, os_, mp, ms, bp, bs, cp, reward.data_ptr(),
+                                      done.data_ptr(), self.reason.data_ptr(), self.winner.data_ptr(), self.ep_len.data_ptr(),
+                                      self.legal_count.data_ptr(), nxt.data_ptr() if nxt is not None else None, self.seed,
+                                      self.step_index, self.env_offset, self.pool.data_ptr(), self.pool.shape[0], pick,
+                                      (self.seed ^ self.POOL_SALT) & 0xFFFFFFFFFFFFFFFF, self.start_ids.data_ptr(), stream),
+                 "kz_step_pool")
+
+    def _step_ranges(self, actions, op, os_, mp, ms, bp, bs, reward, done, nxt, cp=None, pick=None) -> None:
         """One step as ``step_streams`` concurrent kz_step_range launches over disjoint ranges of games (each with its own
         work counter), forked from and joined back into the current stream."""
         cur = torch.cuda.current_stream(self.device)
@@ -202,12 +357,15 @@ class VecShogiEnv:
         fork.record(cur)
         for i, st in enumerate(self._side_streams):
             st.wait_event(fork)
-            nv.check(self._L.kz_step_range(self.state.data_ptr(), self.n, self.hist_cap, i * per, per, i, actions.data_ptr(),
-                                           int(actions.dtype == torch.int64), op, os_, mp, ms, bp, bs, cp, reward.data_ptr(),
-                                           done.data_ptr(), self.reason.data_ptr(), self.winner.data_ptr(),
-                                           self.ep_len.data_ptr(), self.legal_count.data_ptr(),
-                                           nxt.data_ptr() if nxt is not None else None, self.seed, self.step_index,
-                                           self.env_offset, int(self.auto_reset), st.cuda_stream), "kz_step_range")
+            if self._pooled():
+                self._step_pool(i * per, per, i, actions, op, os_, mp, ms, bp, bs, cp, reward, done, nxt, pick, st.cuda_stream)
+            else:
+                nv.check(self._L.kz_step_range(self.state.data_ptr(), self.n, self.hist_cap, i * per, per, i,
+                                               actions.data_ptr(), int(actions.dtype == torch.int64), op, os_, mp, ms, bp, bs,
+                                               cp, reward.data_ptr(), done.data_ptr(), self.reason.data_ptr(),
+                                               self.winner.data_ptr(), self.ep_len.data_ptr(), self.legal_count.data_ptr(),
+                                               nxt.data_ptr() if nxt is not None else None, self.seed, self.step_index,
+                                               self.env_offset, int(self.auto_reset), st.cuda_stream), "kz_step_range")
             join = torch.cuda.Event()
             join.record(st)
             cur.wait_event(join)
@@ -274,6 +432,7 @@ class VecShogiEnv:
                      next_out: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         """First half of the split pipeline (kz_step_compact): ``step`` without the mask / observation rows; the
         successor's legal bitmap goes to ``bitmap`` (int32 [n, 448], default ``self.bitmap``) for ``expand``."""
+        self._no_pool("step_compact")
         if (actions.device != self.device or actions.dtype not in (torch.int64, torch.int32)
                 or not actions.is_contiguous() or actions.numel() < self.n):
             raise ValueError(f"actions: expected {self.n} contiguous int64/int32 policy indices on {self.device}")
@@ -296,6 +455,7 @@ class VecShogiEnv:
                                          self.ep_len.data_ptr(), self.legal_count.data_ptr(),
                                          nxt.data_ptr() if nxt is not None else None, self.seed, self.step_index,
                                          self.env_offset, int(self.auto_reset), self._sp()), "kz_step_compact")
+        self._restarted_from_start(self.done)
         return {"bitmap": bitmap, "reward": self.reward, "done": self.done, "reason": self.reason,
                 "winner": self.winner, "ep_len": self.ep_len, "legal_count": self.legal_count}
 
@@ -303,6 +463,7 @@ class VecShogiEnv:
                mask: Optional[torch.Tensor] = None):
         """Second half of the split pipeline (kz_expand): mask and observation rows of the current positions from the
         state and the bitmap ``step_compact`` left."""
+        self._no_pool("expand")
         bitmap = self.bitmap if bitmap is None else bitmap
         self._check_bitmap(bitmap)
         obs = self.obs if obs is None else obs
@@ -312,6 +473,11 @@ class VecShogiEnv:
         nv.check(self._L.kz_expand(self.state.data_ptr(), self.n, self.hist_cap, bitmap.data_ptr(), op, os_, mp, ms,
                                    self._sp()), "kz_expand")
         return obs, mask
+
+    def _no_pool(self, what: str) -> None:
+        if self.pool is not None:
+            raise ValueError(f"{what}: the split pipeline does not restart games from a start-position pool; use step / "
+                             "step_rollout, or set_start_positions(None)")
 
     def _check_bitmap(self, bitmap: torch.Tensor) -> None:
         if (bitmap.device != self.device or bitmap.dtype != torch.int32 or not bitmap.is_contiguous()
