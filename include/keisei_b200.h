@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define KZ_ABI_VERSION 2
+#define KZ_ABI_VERSION 3
 #define KZ_NUM_ACTIONS 13527
 #define KZ_OBS_FLOATS 3726  /* 46 x 9 x 9 */
 #define KZ_MASK_PAD_STRIDE 13536 /* 16-byte multiple >= 13527: fast-path row stride */
@@ -172,19 +172,6 @@ int kz_step_pool(void* state, int n, int hist_cap, int first, int count, int cou
  * kz_reset, the rows of the new positions come from kz_refresh / kz_legal_bitmap. */
 int kz_reset_pool(void* state, int n, int hist_cap, const uint8_t* env_mask, int max_moves, const uint32_t* pool, int pool_size,
                   const int32_t* pick, uint64_t pool_seed, uint32_t env_offset, int32_t* start_ids, void* stream);
-
-/* Split pipeline (experimental; same results as kz_step, bit for bit): kz_step_compact is kz_step without the two row
- * outputs -- it leaves the successor's 13,527-bit legal bitmap in bitmap [n][448] uint32 (bit i of the row = action i;
- * 16-byte aligned) -- and kz_expand writes the mask and observation rows of the CURRENT positions from the state and
- * that bitmap (PolicyOutputMapper.get_legal_mask, utils.py:310-336; generate_neural_network_observation,
- * shogi_game_io.py:434-539).  Meant for two groups of games on two streams: one group's row stores then overlap the
- * other group's move generation instead of stalling it. */
-int kz_step_compact(void* state, int n, int hist_cap, const void* actions, int actions_i64, uint32_t* bitmap,
-                    float* reward, uint8_t* done, uint8_t* reason, int8_t* winner, int32_t* ep_len, int32_t* legal_count,
-                    void* next_actions, uint64_t seed, uint32_t rng_step, uint32_t env_offset, int auto_reset,
-                    void* stream);
-int kz_expand(const void* state, int n, int hist_cap, const uint32_t* bitmap, float* obs, int64_t obs_stride,
-              uint8_t* mask, int64_t mask_stride, void* stream);
 
 /* Rollout form of kz_step (the PPO self-play path, StepManager.execute_step step_manager.py:98-348 over n games): as
  * kz_step, but the successor's legal moves are left as the 13,527-bit legal BITMAP -- bitmap [n][bitmap_stride_words]

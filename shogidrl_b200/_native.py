@@ -24,13 +24,13 @@ EXPORTS = [
     "kz_export_positions", "kz_piece_targets", "kz_refresh", "kz_step", "kz_legal_mask", "kz_observe", "kz_errors", "kz_sample_masked",
     "kz_gae", "kz_gae_exact", "kz_eval_masked_fwd", "kz_eval_masked_bwd", "kz_obs_conv_fwd", "kz_obs_conv_wgrad_ctas",
     "kz_obs_conv_wgrad", "kz_ppo_loss", "kz_eval_masked_bwd_bias", "kz_adam_clip_workspace", "kz_adam_clip_step",
-    "kz_step_compact", "kz_expand", "kz_step_rollout", "kz_legal_bitmap", "kz_bitmap_expand", "kz_sample_bitmap",
+    "kz_step_rollout", "kz_legal_bitmap", "kz_bitmap_expand", "kz_sample_bitmap",
     "kz_eval_bitmap_fwd", "kz_eval_bitmap_bwd", "kz_step_range", "kz_cobs_conv_fwd", "kz_cobs_conv_wgrad_ctas",
     "kz_cobs_conv_wgrad", "kz_heuristic_actions", "kz_pool_records", "kz_step_pool", "kz_reset_pool",
 ]
 COBS_WORDS = 40
 POOL_RECORD_WORDS = 512
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 
 class NativeError(RuntimeError):
@@ -62,8 +62,6 @@ def lib() -> C.CDLL:
     L.kz_export_positions.argtypes = [vp, i32, i32, vp, vp, vp, vp]
     L.kz_refresh.argtypes = [vp, i32, i32, vp, i64, vp, i64, vp, vp, i32, u64, u32, u32, i32, vp, vp]
     L.kz_step.argtypes = [vp, i32, i32, vp, i32, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, u64, u32, u32, i32, vp]
-    L.kz_step_compact.argtypes = [vp, i32, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, u64, u32, u32, i32, vp]
-    L.kz_expand.argtypes = [vp, i32, i32, vp, vp, i64, vp, i64, vp]
     L.kz_step_rollout.argtypes = [vp, i32, i32, vp, i32, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, u64, u32, u32, i32, vp]
     L.kz_step_range.argtypes = [vp, i32, i32, i32, i32, i32, vp, i32, vp, i64, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp,
                                 u64, u32, u32, i32, vp]

@@ -604,8 +604,8 @@ struct StepParams {
 __device__ __forceinline__ uint16_t ld_u16(const uint8_t* p) { return (uint16_t)(p[0] | (p[1] << 8)); }
 __device__ __forceinline__ void st_u16(uint8_t* p, int v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); }
 
-// MODE 2 = step for the split pipeline (kz_step_compact): as MODE 1, but the rows are left to kz_expand_kernel and the
-// 13,527-bit legal bitmap is written out instead.
+// MODE 2 = step in the rollout form (kz_step_rollout): as MODE 1, but the 13,527-bit legal bitmap is written out instead
+// of the mask row.
 // MODE 1 = step (the hot kernel: only the fast paths are compiled in, the generator is inlined), MODE 0 = refresh
 // (loaded positions: nested-generation uchifuzume, full key, optional termination evaluation).
 // POOL (modes 1 and 2, kz_step_pool): a finished game restarts from a record of the start-position pool instead of the
@@ -1330,135 +1330,6 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
 }
 
 // ------------------------------------------------------------------------------------------------
-// Split pipeline, second half: the mask and observation rows of n games from their state rows and legal bitmaps.  Pure
-// streaming work (1.9 KB read, 28.4 KB written per game, no dependent shared-memory chains): it is meant to run on its
-// own stream next to kz_step_kernel<2> of another group of games, so that generating warps never wait behind row stores.
-#ifndef KZ_EXPAND_CTAS_PER_SM
-#define KZ_EXPAND_CTAS_PER_SM 1
-#endif
-#ifndef KZ_EXPAND_PRELOAD
-#define KZ_EXPAND_PRELOAD 0
-#endif
-#ifndef KZ_EXPAND_SPARSE
-#define KZ_EXPAND_SPARSE 0
-#endif
-#ifndef KZ_COMPACT_CTAS_PER_SM
-#define KZ_COMPACT_CTAS_PER_SM 2  // leaves registers for one expander CTA per SM beside the generating CTAs
-#endif
-__global__ void __launch_bounds__(256) kz_expand_kernel(const uint8_t* __restrict__ boards, const uint8_t* __restrict__ meta,
-                                                        const uint32_t* __restrict__ bitmap, int n, float* obs,
-                                                        long long obs_stride, uint8_t* mask, long long mask_stride,
-                                                        int mask_vec) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  auto expand = [](uint32_t b16) {
-    uint4 v;
-    v.x = ((b16 & 0xF) * 0x00204081u) & 0x01010101u;
-    v.y = (((b16 >> 4) & 0xF) * 0x00204081u) & 0x01010101u;
-    v.z = (((b16 >> 8) & 0xF) * 0x00204081u) & 0x01010101u;
-    v.w = (((b16 >> 12) & 0xF) * 0x00204081u) & 0x01010101u;
-    return v;
-  };
-  for (int g = blockIdx.x * 8 + warp; g < n; g += gridDim.x * 8) {
-    const uint32_t* bm = bitmap + (size_t)g * BITMAP_WORDS;
-    if (mask) {
-      uint8_t* mrow = mask + (size_t)g * mask_stride;
-      if (mask_vec) {
-        uint4* m4 = reinterpret_cast<uint4*>(mrow);
-#if KZ_EXPAND_SPARSE
-        // (untested variant for the next round) the fused kernel's recipe: zero-fill the padded row with 256-bit stores,
-        // then expand only the chunks that hold a legal action (about a fifth of them)
-        if (mask_stride >= 13536 && (((uintptr_t)mrow) & 31) == 0) {
-          uint32_t wreg[27];
-#pragma unroll
-          for (int k = 0; k < 27; k++) wreg[k] = lane + 32 * k < 846 ? __ldg(bm + ((lane + 32 * k) >> 1)) : 0u;
-#pragma unroll 1
-          for (int q = lane; q < 423; q += 32) st_zero256(mrow + 32 * q);
-          __syncwarp();  // the overwrites follow the zero fill in program order
-#pragma unroll
-          for (int k = 0; k < 27; k++) {
-            const int q = lane + 32 * k;
-            const uint32_t half = (q & 1) ? (wreg[k] >> 16) : (wreg[k] & 0xFFFF);
-            if (q < 846 && half) m4[q] = expand(half);
-          }
-        } else
-#endif
-        {
-#if KZ_EXPAND_PRELOAD
-        uint32_t wreg[27];  // all of this lane's bitmap words in flight at once (the loop below is then pure ALU + stores)
-#pragma unroll
-        for (int k = 0; k < 27; k++) wreg[k] = lane + 32 * k < 846 ? __ldg(bm + ((lane + 32 * k) >> 1)) : 0u;
-#pragma unroll
-        for (int k = 0; k < 27; k++) {
-          const int q = lane + 32 * k;
-          if (q >= 846) break;
-          const uint32_t w = wreg[k];
-#else
-#pragma unroll 4
-        for (int q = lane; q < 846; q += 32) {  // chunk q = bits [16q, 16q + 16): every chunk is written, no zero fill
-          const uint32_t w = __ldg(bm + (q >> 1));
-#endif
-          const uint4 v = expand((q & 1) ? (w >> 16) : (w & 0xFFFF));
-          if (q < 845 || mask_stride >= 13536) m4[q] = v;
-          else {  // last 7 bytes of an exactly-13,527-byte aligned row
-            const uint32_t parts[2] = {v.x, v.y};
-            for (int b = 0; b < 7; b++) mrow[13520 + b] = (uint8_t)(parts[b >> 2] >> (8 * (b & 3)));
-          }
-        }
-        }
-      } else {
-        for (int i = lane; i < KZ_NUM_ACTIONS; i += 32) mrow[i] = (uint8_t)((__ldg(bm + (i >> 5)) >> (i & 31)) & 1);
-      }
-    }
-    if (obs) {
-      // generate_neural_network_observation (shogi_game_io.py:434-539), as the tail of kz_step_kernel writes it
-      float* orow = obs + (size_t)g * obs_stride;
-      const uint8_t* b = boards + (size_t)g * 96;
-      const uint8_t* m = meta + (size_t)g * 32;
-      const int side = m[14];
-      const int move_count = m[18] | (m[19] << 8), max_moves = m[22] | (m[23] << 8);
-      float pv = 0.f;
-      if (lane < 14) {
-        const int cnt = m[lane < 7 ? side * 7 + lane : (1 - side) * 7 + (lane - 7)];
-        if (cnt > 0) pv = __fdiv_rn((float)cnt, 18.0f);
-      } else if (lane == 14) pv = side == 0 ? 1.f : 0.f;
-      else if (lane == 15) pv = max_moves > 0 ? __fdiv_rn((float)move_count, (float)max_moves) : 0.f;
-      int code3[3];
-#pragma unroll
-      for (int j = 0; j < 3; j++) { const int sq = lane + 32 * j; code3[j] = sq < 81 ? b[sq] : 0; }
-      float2* o2 = reinterpret_cast<float2*>(orow);
-      const int head = (int)(((32u - (unsigned)((uintptr_t)orow & 31)) & 31u) >> 3);
-      const int nb = (KZ_OBS_FLOATS * 4 - head * 8) >> 5;
-      char* body = reinterpret_cast<char*>(orow) + head * 8;
-      if (lane < head) o2[lane] = make_float2(0.f, 0.f);
-#pragma unroll 4
-      for (int q = lane; q < nb; q += 32) st_zero256(body + 32 * q);
-      const int tail0 = head + 4 * nb;
-      if (lane < KZ_OBS_FLOATS / 2 - tail0) o2[tail0 + lane] = make_float2(0.f, 0.f);
-      __syncwarp();  // the overwrites below follow the zero fill in program order
-      uint32_t nzp = __ballot_sync(FULL, pv != 0.f);
-      while (nzp) {
-        const int i = __ffs(nzp) - 1;
-        nzp &= nzp - 1;
-        const float v = __shfl_sync(FULL, pv, i);
-        float* pl = orow + (28 + i) * 81;
-        pl[lane] = v;
-        pl[lane + 32] = v;
-        if (lane < 17) pl[lane + 64] = v;
-      }
-#pragma unroll
-      for (int j = 0; j < 3; j++) {
-        const int sq = lane + 32 * j;
-        const int code = code3[j];
-        if (code) {
-          const int t = code_type(code), mine = code_color(code) == side;
-          const int plane = t < 8 ? (mine ? 0 : 14) + t : (mine ? 8 : 22) + (t - 8);
-          orow[plane * 81 + (side == 0 ? sq : 80 - sq)] = 1.0f;
-        }
-      }
-    }
-  }
-}
-
 // Legal bitmap rows -> byte-mask rows (PolicyOutputMapper.get_legal_mask's layout, utils.py:310-336) for callers of the
 // reference API; any row stride / alignment (4 mask bytes per store when the row is 4-byte aligned).
 __global__ void __launch_bounds__(256) kz_bitmap_expand_kernel(const uint32_t* __restrict__ bitmap, long long ldb,
@@ -1674,6 +1545,17 @@ Layout layout(int n, int hist_cap) {
   return L;
 }
 
+// The kz_step_kernel instantiations, [pool][mode]: refresh (mode 0) has no pool form.  launch_step launches through this
+// table and kz_init_tables sets the dynamic shared-memory limit of every entry.
+using StepKernel = void (*)(const StepParams);
+const StepKernel kStepKernels[2][3] = {{kz_step_kernel<0>, kz_step_kernel<1>, kz_step_kernel<2>},
+                                       {nullptr, kz_step_kernel<1, true>, kz_step_kernel<2, true>}};
+StepKernel step_kernel(int mode, bool pool) { return mode >= 0 && mode < 3 ? kStepKernels[pool][mode] : nullptr; }
+
+#ifndef KZ_COMPACT_CTAS_PER_SM
+#define KZ_COMPACT_CTAS_PER_SM 2
+#endif
+
 int launch_step(void* state, int n, int hist_cap, StepParams P, cudaStream_t st, int first = 0, int count = -1, int slot = 0) {
   if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535) return KZ_E_ARG;
   if (count < 0) count = n - first;
@@ -1703,7 +1585,8 @@ int launch_step(void* state, int n, int hist_cap, StepParams P, cudaStream_t st,
     if (count == 1 && ((uintptr_t)P.mask & 15) == 0) P.mask_vec = 1;
   }
   const int ctas_needed = (count + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
-  // mode 2 without observation rows is the split pipeline's generator (leaves room for kz_expand_kernel beside it)
+  // rollout-form launches without observation rows run KZ_COMPACT_CTAS_PER_SM CTAs per SM: tuned in round 1 next to an
+  // expander kernel (since removed) and not re-measured since
   int grid = sm_count() * ((P.mode == 2 && !P.obs) ? KZ_COMPACT_CTAS_PER_SM : CTAS_PER_SM);
   if (grid > ctas_needed) grid = ctas_needed;
   const size_t dyn = sizeof(WarpScratch) * WARPS_PER_CTA;
@@ -1716,15 +1599,32 @@ int launch_step(void* state, int n, int hist_cap, StepParams P, cudaStream_t st,
     CK(cudaMemsetAsync(P.tile_counter, 0, sizeof(int), st));
   }
 #endif
-  if (P.pool) {
-    if (P.mode == 1) kz_step_kernel<1, true><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
-    else if (P.mode == 2) kz_step_kernel<2, true><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
-    else return KZ_E_ARG;
-  } else if (P.mode == 1) kz_step_kernel<1><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
-  else if (P.mode == 2) kz_step_kernel<2><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
-  else kz_step_kernel<0><<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
+  const StepKernel kernel = step_kernel(P.mode, P.pool != nullptr);
+  if (!kernel) return KZ_E_ARG;
+  kernel<<<grid, WARPS_PER_CTA * 32, dyn, st>>>(P);
   CK(cudaGetLastError());
   return KZ_OK;
+}
+
+// kz_step, kz_step_rollout, kz_step_range and kz_step_pool: games [first, first + count) of the batch, in the mask form
+// (bitmap == NULL) or the rollout form (bitmap != NULL); finished games restart from the pool when pool != NULL.
+int step_games(void* state, int n, int hist_cap, int first, int count, int counter_slot, const void* actions,
+               int actions_i64, float* obs, int64_t obs_stride, uint8_t* mask, int64_t mask_stride, uint32_t* bitmap,
+               int64_t bitmap_stride_words, uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner,
+               int32_t* ep_len, int32_t* legal_count, void* next_actions, uint64_t seed, uint32_t rng_step,
+               uint32_t env_offset, int auto_reset, const uint32_t* pool, int pool_size, const int32_t* pick,
+               uint64_t pool_seed, int32_t* start_ids, void* stream) {
+  if (!actions) return KZ_E_ARG;
+  StepParams P{};
+  P.actions = actions; P.actions_i64 = actions_i64;
+  P.obs = obs; P.obs_stride = obs_stride; P.mask = mask; P.mask_stride = mask_stride;
+  P.bitmap_out = bitmap; P.bitmap_stride = bitmap_stride_words; P.cobs_out = cobs;
+  P.reward = reward; P.done = done; P.reason = reason; P.winner = winner; P.ep_len = ep_len;
+  P.legal_count = legal_count; P.next_actions = next_actions;
+  P.seed = seed; P.rng_step = rng_step; P.env_offset = env_offset;
+  P.auto_reset = auto_reset; P.mode = bitmap ? 2 : 1;
+  P.pool = pool; P.pool_size = pool_size; P.pool_pick = pick; P.pool_seed = pool_seed; P.start_ids = start_ids;
+  return launch_step(state, n, hist_cap, P, reinterpret_cast<cudaStream_t>(stream), first, count, counter_slot);
 }
 
 }  // namespace
@@ -1819,11 +1719,9 @@ int kz_init_tables(void* stream) {
   CK(cudaDeviceGetAttribute(&g_sm_counts[dev], cudaDevAttrMultiProcessorCount, dev));
   {  // per-warp scratch lives in dynamic shared memory (more than 48 KB with tables for CTAs above 8 warps)
     const int dyn = (int)(sizeof(WarpScratch) * WARPS_PER_CTA);
-    CK(cudaFuncSetAttribute(kz_step_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
-    CK(cudaFuncSetAttribute(kz_step_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
-    CK(cudaFuncSetAttribute(kz_step_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
-    CK(cudaFuncSetAttribute(kz_step_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
-    CK(cudaFuncSetAttribute(kz_step_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
+    for (const auto& row : kStepKernels)
+      for (StepKernel kernel : row)
+        if (kernel) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
   }
   g_ready[dev] = true;
   // legal bitmap of the start position, computed once by the engine itself on a scratch game
@@ -1948,15 +1846,9 @@ int kz_step(void* state, int n, int hist_cap, const void* actions, int actions_i
             uint8_t* mask, int64_t mask_stride, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner,
             int32_t* ep_len, int32_t* legal_count, void* next_actions, uint64_t seed, uint32_t rng_step,
             uint32_t env_offset, int auto_reset, void* stream) {
-  if (!actions) return KZ_E_ARG;
-  StepParams P{};
-  P.actions = actions; P.actions_i64 = actions_i64;
-  P.obs = obs; P.obs_stride = obs_stride; P.mask = mask; P.mask_stride = mask_stride;
-  P.reward = reward; P.done = done; P.reason = reason; P.winner = winner; P.ep_len = ep_len;
-  P.legal_count = legal_count; P.next_actions = next_actions;
-  P.seed = seed; P.rng_step = rng_step; P.env_offset = env_offset;
-  P.auto_reset = auto_reset; P.mode = 1;
-  return launch_step(state, n, hist_cap, P, reinterpret_cast<cudaStream_t>(stream));
+  return step_games(state, n, hist_cap, 0, n, 0, actions, actions_i64, obs, obs_stride, mask, mask_stride, nullptr, 0,
+                    nullptr, reward, done, reason, winner, ep_len, legal_count, next_actions, seed, rng_step, env_offset,
+                    auto_reset, nullptr, 0, nullptr, 0, nullptr, stream);
 }
 
 int kz_step_range(void* state, int n, int hist_cap, int first, int count, int counter_slot, const void* actions,
@@ -1964,16 +1856,10 @@ int kz_step_range(void* state, int n, int hist_cap, int first, int count, int co
                   int64_t bitmap_stride_words, uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner,
                   int32_t* ep_len, int32_t* legal_count, void* next_actions, uint64_t seed, uint32_t rng_step,
                   uint32_t env_offset, int auto_reset, void* stream) {
-  if (!actions || (mask && bitmap)) return KZ_E_ARG;
-  StepParams P{};
-  P.actions = actions; P.actions_i64 = actions_i64;
-  P.obs = obs; P.obs_stride = obs_stride; P.mask = mask; P.mask_stride = mask_stride;
-  P.bitmap_out = bitmap; P.bitmap_stride = bitmap_stride_words; P.cobs_out = cobs;
-  P.reward = reward; P.done = done; P.reason = reason; P.winner = winner; P.ep_len = ep_len;
-  P.legal_count = legal_count; P.next_actions = next_actions;
-  P.seed = seed; P.rng_step = rng_step; P.env_offset = env_offset;
-  P.auto_reset = auto_reset; P.mode = bitmap ? 2 : 1;
-  return launch_step(state, n, hist_cap, P, reinterpret_cast<cudaStream_t>(stream), first, count, counter_slot);
+  if (mask && bitmap) return KZ_E_ARG;
+  return step_games(state, n, hist_cap, first, count, counter_slot, actions, actions_i64, obs, obs_stride, mask, mask_stride,
+                    bitmap, bitmap_stride_words, cobs, reward, done, reason, winner, ep_len, legal_count, next_actions, seed,
+                    rng_step, env_offset, auto_reset, nullptr, 0, nullptr, 0, nullptr, stream);
 }
 
 int kz_step_pool(void* state, int n, int hist_cap, int first, int count, int counter_slot, const void* actions,
@@ -1982,69 +1868,20 @@ int kz_step_pool(void* state, int n, int hist_cap, int first, int count, int cou
                  int32_t* ep_len, int32_t* legal_count, void* next_actions, uint64_t seed, uint32_t rng_step,
                  uint32_t env_offset, const uint32_t* pool, int pool_size, const int32_t* pick, uint64_t pool_seed,
                  int32_t* start_ids, void* stream) {
-  if (!actions || (mask && bitmap) || !pool || pool_size <= 0 || ((uintptr_t)pool & 15)) return KZ_E_ARG;
-  StepParams P{};
-  P.actions = actions; P.actions_i64 = actions_i64;
-  P.obs = obs; P.obs_stride = obs_stride; P.mask = mask; P.mask_stride = mask_stride;
-  P.bitmap_out = bitmap; P.bitmap_stride = bitmap_stride_words; P.cobs_out = cobs;
-  P.reward = reward; P.done = done; P.reason = reason; P.winner = winner; P.ep_len = ep_len;
-  P.legal_count = legal_count; P.next_actions = next_actions;
-  P.seed = seed; P.rng_step = rng_step; P.env_offset = env_offset;
-  P.auto_reset = 1; P.mode = bitmap ? 2 : 1;
-  P.pool = pool; P.pool_size = pool_size; P.pool_pick = pick; P.pool_seed = pool_seed; P.start_ids = start_ids;
-  return launch_step(state, n, hist_cap, P, reinterpret_cast<cudaStream_t>(stream), first, count, counter_slot);
-}
-
-int kz_step_compact(void* state, int n, int hist_cap, const void* actions, int actions_i64, uint32_t* bitmap,
-                    float* reward, uint8_t* done, uint8_t* reason, int8_t* winner, int32_t* ep_len, int32_t* legal_count,
-                    void* next_actions, uint64_t seed, uint32_t rng_step, uint32_t env_offset, int auto_reset,
-                    void* stream) {
-  if (!actions || !bitmap || ((uintptr_t)bitmap & 15)) return KZ_E_ARG;
-  StepParams P{};
-  P.actions = actions; P.actions_i64 = actions_i64;
-  P.bitmap_out = bitmap; P.bitmap_stride = BITMAP_WORDS;
-  P.reward = reward; P.done = done; P.reason = reason; P.winner = winner; P.ep_len = ep_len;
-  P.legal_count = legal_count; P.next_actions = next_actions;
-  P.seed = seed; P.rng_step = rng_step; P.env_offset = env_offset;
-  P.auto_reset = auto_reset; P.mode = 2;
-  return launch_step(state, n, hist_cap, P, reinterpret_cast<cudaStream_t>(stream));
-}
-
-int kz_expand(const void* state, int n, int hist_cap, const uint32_t* bitmap, float* obs, int64_t obs_stride,
-              uint8_t* mask, int64_t mask_stride, void* stream) {
-  if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535 || !bitmap || (!obs && !mask)) return KZ_E_ARG;
-  if (!host_ready()) return KZ_E_NOT_INIT;
-  if (obs && ((((uintptr_t)obs) & 15) || (obs_stride & 1) || obs_stride < KZ_OBS_FLOATS)) return KZ_E_ARG;
-  int mask_vec = 0;
-  if (mask) {
-    if (mask_stride < KZ_NUM_ACTIONS) return KZ_E_ARG;
-    mask_vec = ((((uintptr_t)mask) & 15) == 0 && (mask_stride & 15) == 0) ? 1 : 0;
-    if (n == 1 && (((uintptr_t)mask) & 15) == 0) mask_vec = 1;
-  }
-  const Layout L = layout(n, hist_cap);
-  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
-  int grid = sm_count() * KZ_EXPAND_CTAS_PER_SM;
-  if (grid > (n + 7) / 8) grid = (n + 7) / 8;
-  kz_expand_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(base + L.off_boards, base + L.off_meta, bitmap, n,
-                                                                            obs, obs_stride, mask, mask_stride, mask_vec);
-  CK(cudaGetLastError());
-  return KZ_OK;
+  if ((mask && bitmap) || !pool || pool_size <= 0 || ((uintptr_t)pool & 15)) return KZ_E_ARG;
+  return step_games(state, n, hist_cap, first, count, counter_slot, actions, actions_i64, obs, obs_stride, mask, mask_stride,
+                    bitmap, bitmap_stride_words, cobs, reward, done, reason, winner, ep_len, legal_count, next_actions, seed,
+                    rng_step, env_offset, 1, pool, pool_size, pick, pool_seed, start_ids, stream);
 }
 
 int kz_step_rollout(void* state, int n, int hist_cap, const void* actions, int actions_i64, float* obs, int64_t obs_stride,
                     uint32_t* bitmap, int64_t bitmap_stride_words, uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason,
                     int8_t* winner, int32_t* ep_len, int32_t* legal_count, void* next_actions, uint64_t seed,
                     uint32_t rng_step, uint32_t env_offset, int auto_reset, void* stream) {
-  if (!actions || !bitmap) return KZ_E_ARG;
-  StepParams P{};
-  P.actions = actions; P.actions_i64 = actions_i64;
-  P.obs = obs; P.obs_stride = obs_stride;
-  P.bitmap_out = bitmap; P.bitmap_stride = bitmap_stride_words; P.cobs_out = cobs;
-  P.reward = reward; P.done = done; P.reason = reason; P.winner = winner; P.ep_len = ep_len;
-  P.legal_count = legal_count; P.next_actions = next_actions;
-  P.seed = seed; P.rng_step = rng_step; P.env_offset = env_offset;
-  P.auto_reset = auto_reset; P.mode = 2;
-  return launch_step(state, n, hist_cap, P, reinterpret_cast<cudaStream_t>(stream));
+  if (!bitmap) return KZ_E_ARG;
+  return step_games(state, n, hist_cap, 0, n, 0, actions, actions_i64, obs, obs_stride, nullptr, 0, bitmap,
+                    bitmap_stride_words, cobs, reward, done, reason, winner, ep_len, legal_count, next_actions, seed, rng_step,
+                    env_offset, auto_reset, nullptr, 0, nullptr, 0, nullptr, stream);
 }
 
 int kz_legal_bitmap(void* state, int n, int hist_cap, float* obs, int64_t obs_stride, uint32_t* bitmap,

@@ -125,6 +125,15 @@ class VecShogiEnv:
     def _mask_args(self, mask: Optional[torch.Tensor]):
         return self._rows_arg(mask, "mask", (torch.uint8, torch.bool), nv.NUM_ACTIONS)
 
+    def _vec_arg(self, t: Optional[torch.Tensor], what: str, dtypes):
+        """Data pointer of a contiguous [n] vector on the env's device (None stays None)."""
+        if t is None:
+            return None
+        if t.device != self.device or t.dtype not in dtypes or not t.is_contiguous() or t.numel() < self.n:
+            raise ValueError(f"{what}: expected a contiguous {'/'.join(str(d)[6:] for d in dtypes)} [{self.n}] tensor on "
+                             f"{self.device}, got {tuple(t.shape)} {t.dtype} on {t.device}")
+        return t.data_ptr()
+
     def _pick_arg(self, start_pick: Optional[torch.Tensor], in_step: bool = True):
         if start_pick is None:
             return None
@@ -133,11 +142,7 @@ class VecShogiEnv:
         if in_step and not self.auto_reset:
             raise ValueError("start_pick: this env does not reset finished games (auto_reset=False), so no game would "
                              "start from it; use reset(start_pick=...)")
-        if (start_pick.device != self.device or start_pick.dtype != torch.int32 or not start_pick.is_contiguous()
-                or start_pick.numel() < self.n):
-            raise ValueError(f"start_pick: expected a contiguous int32 [{self.n}] tensor on {self.device}, got "
-                             f"{tuple(start_pick.shape)} {start_pick.dtype} on {start_pick.device}")
-        return start_pick.data_ptr()
+        return self._vec_arg(start_pick, "start_pick", (torch.int32,))
 
     # ------------------------------------------------------------------ API
     def set_start_positions(self, sfens: Optional[Sequence[str]], reset: bool = False) -> None:
@@ -252,36 +257,10 @@ class VecShogiEnv:
         With ``random_actions`` the kernel also writes a uniform-random legal action for the returned state
         into ``next_out`` (default ``self.next_actions``; must not alias ``actions``).  With a start-position pool,
         ``start_pick`` (int32 [n]) names the entry each env restarts from if its game finishes in this step."""
-        if (actions.device != self.device or actions.dtype not in (torch.int64, torch.int32)
-                or not actions.is_contiguous() or actions.numel() < self.n):
-            raise ValueError(f"actions: expected {self.n} contiguous int64/int32 policy indices on {self.device}, got "
-                             f"{tuple(actions.shape)} {actions.dtype} on {actions.device}")
         obs = (self.obs if obs is None else obs) if write_obs else None
         mask = (self.mask if mask is None else mask) if write_mask else None
-        op, os_ = self._obs_args(obs)
-        mp, ms = self._mask_args(mask)
-        nxt = None
-        if random_actions:
-            nxt = self.next_actions if next_out is None else next_out
-            if actions.dtype == torch.int32 and nxt.dtype == torch.int64:
-                nxt = nxt.view(torch.int32)[: self.n]
-            if nxt.data_ptr() == actions.data_ptr():
-                raise ValueError("next_out must not alias actions (the kernel reads one while writing the other)")
-        pk = self._pick_arg(start_pick)
-        self.step_index += 1  # after validation: a rejected call leaves the RNG counter where it was
-        if self.step_streams > 1:
-            self._step_ranges(actions, op, os_, mp, ms, None, 0, self.reward, self.done, nxt, pick=pk)
-            self._restarted_from_start(self.done)
-        elif self._pooled():
-            self._step_pool(0, self.n, 0, actions, op, os_, mp, ms, None, 0, None, self.reward, self.done, nxt, pk, self._sp())
-        else:
-            nv.check(self._L.kz_step(self.state.data_ptr(), self.n, self.hist_cap, actions.data_ptr(),
-                                     int(actions.dtype == torch.int64), op, os_, mp, ms, self.reward.data_ptr(),
-                                     self.done.data_ptr(), self.reason.data_ptr(), self.winner.data_ptr(),
-                                     self.ep_len.data_ptr(), self.legal_count.data_ptr(),
-                                     nxt.data_ptr() if nxt is not None else None, self.seed, self.step_index,
-                                     self.env_offset, int(self.auto_reset), self._sp()), "kz_step")
-        self._restarted_from_start(self.done)
+        self._launch(actions, self._obs_args(obs), self._mask_args(mask), (None, 0), None, self.reward, self.done,
+                     random_actions, next_out, start_pick)
         return {"obs": obs, "mask": mask, "reward": self.reward, "done": self.done, "reason": self.reason,
                 "winner": self.winner, "ep_len": self.ep_len, "legal_count": self.legal_count}
 
@@ -295,80 +274,63 @@ class VecShogiEnv:
         (None: no observation rows); ``reward`` / ``done`` may point into rollout storage (fp32 / uint8 [n]); ``cobs``
         (int32 [n, 40]) receives the compact observations the policy network's input layer reads (kz_cobs_conv_*);
         ``start_pick`` as in ``step``."""
-        if (actions.device != self.device or actions.dtype not in (torch.int64, torch.int32)
-                or not actions.is_contiguous() or actions.numel() < self.n):
-            raise ValueError(f"actions: expected {self.n} contiguous int64/int32 policy indices on {self.device}")
-        bp, bs = self._bitmap_args(bitmap)
-        op, os_ = self._obs_args(obs)
-        cp = self._cobs_arg(cobs)
         reward = self.reward if reward is None else reward
         done = self.done if done is None else done
-        for t, dt, what in ((reward, torch.float32, "reward"), (done, torch.uint8, "done")):
-            if t.device != self.device or t.dtype != dt or not t.is_contiguous() or t.numel() < self.n:
-                raise ValueError(f"{what}: expected a contiguous {dt} [{self.n}] tensor on {self.device}")
+        self._vec_arg(reward, "reward", (torch.float32,))
+        self._vec_arg(done, "done", (torch.uint8,))
+        self._launch(actions, self._obs_args(obs), (None, 0), self._bitmap_args(bitmap), self._cobs_arg(cobs), reward, done,
+                     random_actions, next_out, start_pick)
+        return {"obs": obs, "bitmap": bitmap, "reward": reward, "done": done, "reason": self.reason,
+                "winner": self.winner, "ep_len": self.ep_len, "legal_count": self.legal_count}
+
+    def _launch(self, actions: torch.Tensor, obs, mask, bitmap, cobs, reward: torch.Tensor, done: torch.Tensor,
+                random_actions: bool, next_out: Optional[torch.Tensor], start_pick: Optional[torch.Tensor]) -> None:
+        """One step of every env in the mask form (``mask`` rows) or the rollout form (``bitmap`` rows); ``obs`` / ``mask``
+        / ``bitmap`` are validated (pointer, row stride) pairs and ``cobs`` a validated pointer.  Validates the arguments
+        both forms share, then launches kz_step_pool when finished games restart from a pool, kz_step_range otherwise:
+        once on the current stream, or as ``step_streams`` ranges of games (each with its own work counter) forked from
+        and joined back into it."""
+        ap = self._vec_arg(actions, "actions", (torch.int64, torch.int32))
         nxt = None
         if random_actions:
             nxt = self.next_actions if next_out is None else next_out
             if actions.dtype == torch.int32 and nxt.dtype == torch.int64:
                 nxt = nxt.view(torch.int32)[: self.n]
-            if nxt.data_ptr() == actions.data_ptr():
+            if nxt.data_ptr() == ap:
                 raise ValueError("next_out must not alias actions (the kernel reads one while writing the other)")
-        pk = self._pick_arg(start_pick)
-        self.step_index += 1
-        if self.step_streams > 1:
-            self._step_ranges(actions, op, os_, None, 0, bp, bs, reward, done, nxt, cp, pick=pk)
-            self._restarted_from_start(done)
-        elif self._pooled():
-            self._step_pool(0, self.n, 0, actions, op, os_, None, 0, bp, bs, cp, reward, done, nxt, pk, self._sp())
+            nxt = nxt.data_ptr()
+        pick = self._pick_arg(start_pick)
+        self.step_index += 1  # after validation: a rejected call leaves the RNG counter where it was
+        args = (ap, int(actions.dtype == torch.int64), *obs, *mask, *bitmap, cobs, reward.data_ptr(), done.data_ptr(),
+                self.reason.data_ptr(), self.winner.data_ptr(), self.ep_len.data_ptr(), self.legal_count.data_ptr(), nxt,
+                self.seed, self.step_index, self.env_offset)
+        if self.pool is not None and self.auto_reset:
+            fn, name = self._L.kz_step_pool, "kz_step_pool"
+            args += (self.pool.data_ptr(), self.pool.shape[0], pick, (self.seed ^ self.POOL_SALT) & 0xFFFFFFFFFFFFFFFF,
+                     self.start_ids.data_ptr())
         else:
-            nv.check(self._L.kz_step_rollout(self.state.data_ptr(), self.n, self.hist_cap, actions.data_ptr(),
-                                             int(actions.dtype == torch.int64), op, os_, bp, bs, cp, reward.data_ptr(),
-                                             done.data_ptr(), self.reason.data_ptr(), self.winner.data_ptr(),
-                                             self.ep_len.data_ptr(), self.legal_count.data_ptr(),
-                                             nxt.data_ptr() if nxt is not None else None, self.seed, self.step_index,
-                                             self.env_offset, int(self.auto_reset), self._sp()), "kz_step_rollout")
+            fn, name = self._L.kz_step_range, "kz_step_range"
+            args += (int(self.auto_reset),)
+        state = self.state.data_ptr()
+        if self.step_streams == 1:  # no events: rollout steps are captured into a CUDA graph
+            nv.check(fn(state, self.n, self.hist_cap, 0, self.n, 0, *args, self._sp()), name)
+        else:
+            cur = torch.cuda.current_stream(self.device)
+            per = self.n // self.step_streams
+            fork = torch.cuda.Event()
+            fork.record(cur)
+            for i, st in enumerate(self._side_streams):
+                st.wait_event(fork)
+                nv.check(fn(state, self.n, self.hist_cap, i * per, per, i, *args, st.cuda_stream), name)
+                join = torch.cuda.Event()
+                join.record(st)
+                cur.wait_event(join)
         self._restarted_from_start(done)
-        return {"obs": obs, "bitmap": bitmap, "reward": reward, "done": done, "reason": self.reason,
-                "winner": self.winner, "ep_len": self.ep_len, "legal_count": self.legal_count}
-
-    def _pooled(self) -> bool:
-        return self.pool is not None and self.auto_reset
 
     def _restarted_from_start(self, done: torch.Tensor) -> None:
         """After a launch without a pool: games that finished restarted from the start position (start_ids -1)."""
         if self._ids_in_use and self.pool is None and self.auto_reset:
             self.start_ids.masked_fill_(done[: self.n] != 0, -1)
-
-    def _step_pool(self, first, count, slot, actions, op, os_, mp, ms, bp, bs, cp, reward, done, nxt, pick, stream) -> None:
-        nv.check(self._L.kz_step_pool(self.state.data_ptr(), self.n, self.hist_cap, first, count, slot, actions.data_ptr(),
-                                      int(actions.dtype == torch.int64), op, os_, mp, ms, bp, bs, cp, reward.data_ptr(),
-                                      done.data_ptr(), self.reason.data_ptr(), self.winner.data_ptr(), self.ep_len.data_ptr(),
-                                      self.legal_count.data_ptr(), nxt.data_ptr() if nxt is not None else None, self.seed,
-                                      self.step_index, self.env_offset, self.pool.data_ptr(), self.pool.shape[0], pick,
-                                      (self.seed ^ self.POOL_SALT) & 0xFFFFFFFFFFFFFFFF, self.start_ids.data_ptr(), stream),
-                 "kz_step_pool")
-
-    def _step_ranges(self, actions, op, os_, mp, ms, bp, bs, reward, done, nxt, cp=None, pick=None) -> None:
-        """One step as ``step_streams`` concurrent kz_step_range launches over disjoint ranges of games (each with its own
-        work counter), forked from and joined back into the current stream."""
-        cur = torch.cuda.current_stream(self.device)
-        k, per = self.step_streams, self.n // self.step_streams
-        fork = torch.cuda.Event()
-        fork.record(cur)
-        for i, st in enumerate(self._side_streams):
-            st.wait_event(fork)
-            if self._pooled():
-                self._step_pool(i * per, per, i, actions, op, os_, mp, ms, bp, bs, cp, reward, done, nxt, pick, st.cuda_stream)
-            else:
-                nv.check(self._L.kz_step_range(self.state.data_ptr(), self.n, self.hist_cap, i * per, per, i,
-                                               actions.data_ptr(), int(actions.dtype == torch.int64), op, os_, mp, ms, bp, bs,
-                                               cp, reward.data_ptr(), done.data_ptr(), self.reason.data_ptr(),
-                                               self.winner.data_ptr(), self.ep_len.data_ptr(), self.legal_count.data_ptr(),
-                                               nxt.data_ptr() if nxt is not None else None, self.seed, self.step_index,
-                                               self.env_offset, int(self.auto_reset), st.cuda_stream), "kz_step_range")
-            join = torch.cuda.Event()
-            join.record(st)
-            cur.wait_event(join)
 
     def legal_bitmap(self, bitmap: torch.Tensor, obs: Optional[torch.Tensor] = None, cobs: Optional[torch.Tensor] = None):
         """Legal bitmap (and optionally the observation rows / compact observations) of the CURRENT positions
@@ -401,14 +363,10 @@ class VecShogiEnv:
             mp, ms = self._mask_args(self.mask if mask is None else mask)
         if out is None:
             out = torch.empty(self.n, dtype=torch.int64, device=self.device)
-        for t, dts, what in ((out, (torch.int64, torch.int32), "out"), (tier, (torch.uint8,), "tier"),
-                             (tier_count, (torch.int32,), "tier_count")):
-            if t is not None and (t.device != self.device or t.dtype not in dts or not t.is_contiguous()
-                                  or t.numel() < self.n):
-                raise ValueError(f"{what}: expected a contiguous {dts[0]} [{self.n}] tensor on {self.device}, got "
-                                 f"{tuple(t.shape)} {t.dtype} on {t.device}")
-        nv.check(self._L.kz_heuristic_actions(self.state.data_ptr(), self.n, self.hist_cap, mp, ms, bp, bs, out.data_ptr(),
-                                              int(out.dtype == torch.int64), nv.ptr(tier), nv.ptr(tier_count),
+        op = self._vec_arg(out, "out", (torch.int64, torch.int32))
+        tp, cp = self._vec_arg(tier, "tier", (torch.uint8,)), self._vec_arg(tier_count, "tier_count", (torch.int32,))
+        nv.check(self._L.kz_heuristic_actions(self.state.data_ptr(), self.n, self.hist_cap, mp, ms, bp, bs, op,
+                                              int(out.dtype == torch.int64), tp, cp,
                                               (self.seed ^ self.HEURISTIC_SALT) & 0xFFFFFFFFFFFFFFFF, self.step_index,
                                               self.env_offset, self._sp()), "kz_heuristic_actions")
         return out
@@ -427,62 +385,6 @@ class VecShogiEnv:
                 or bitmap.data_ptr() % 16):
             raise ValueError(f"bitmap: expected int32 [{self.n}, {nv.BITMAP_WORDS}] rows (16-byte aligned) on {self.device}")
         return bitmap.data_ptr(), bitmap.stride(0)
-
-    def step_compact(self, actions: torch.Tensor, bitmap: Optional[torch.Tensor] = None, random_actions: bool = False,
-                     next_out: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
-        """First half of the split pipeline (kz_step_compact): ``step`` without the mask / observation rows; the
-        successor's legal bitmap goes to ``bitmap`` (int32 [n, 448], default ``self.bitmap``) for ``expand``."""
-        self._no_pool("step_compact")
-        if (actions.device != self.device or actions.dtype not in (torch.int64, torch.int32)
-                or not actions.is_contiguous() or actions.numel() < self.n):
-            raise ValueError(f"actions: expected {self.n} contiguous int64/int32 policy indices on {self.device}")
-        if bitmap is None:
-            if getattr(self, "bitmap", None) is None:
-                self.bitmap = torch.zeros((self.n, nv.BITMAP_WORDS), dtype=torch.int32, device=self.device)
-            bitmap = self.bitmap
-        self._check_bitmap(bitmap)
-        nxt = None
-        if random_actions:
-            nxt = self.next_actions if next_out is None else next_out
-            if actions.dtype == torch.int32 and nxt.dtype == torch.int64:
-                nxt = nxt.view(torch.int32)[: self.n]
-            if nxt.data_ptr() == actions.data_ptr():
-                raise ValueError("next_out must not alias actions (the kernel reads one while writing the other)")
-        self.step_index += 1
-        nv.check(self._L.kz_step_compact(self.state.data_ptr(), self.n, self.hist_cap, actions.data_ptr(),
-                                         int(actions.dtype == torch.int64), bitmap.data_ptr(), self.reward.data_ptr(),
-                                         self.done.data_ptr(), self.reason.data_ptr(), self.winner.data_ptr(),
-                                         self.ep_len.data_ptr(), self.legal_count.data_ptr(),
-                                         nxt.data_ptr() if nxt is not None else None, self.seed, self.step_index,
-                                         self.env_offset, int(self.auto_reset), self._sp()), "kz_step_compact")
-        self._restarted_from_start(self.done)
-        return {"bitmap": bitmap, "reward": self.reward, "done": self.done, "reason": self.reason,
-                "winner": self.winner, "ep_len": self.ep_len, "legal_count": self.legal_count}
-
-    def expand(self, bitmap: Optional[torch.Tensor] = None, obs: Optional[torch.Tensor] = None,
-               mask: Optional[torch.Tensor] = None):
-        """Second half of the split pipeline (kz_expand): mask and observation rows of the current positions from the
-        state and the bitmap ``step_compact`` left."""
-        self._no_pool("expand")
-        bitmap = self.bitmap if bitmap is None else bitmap
-        self._check_bitmap(bitmap)
-        obs = self.obs if obs is None else obs
-        mask = self.mask if mask is None else mask
-        op, os_ = self._obs_args(obs)
-        mp, ms = self._mask_args(mask)
-        nv.check(self._L.kz_expand(self.state.data_ptr(), self.n, self.hist_cap, bitmap.data_ptr(), op, os_, mp, ms,
-                                   self._sp()), "kz_expand")
-        return obs, mask
-
-    def _no_pool(self, what: str) -> None:
-        if self.pool is not None:
-            raise ValueError(f"{what}: the split pipeline does not restart games from a start-position pool; use step / "
-                             "step_rollout, or set_start_positions(None)")
-
-    def _check_bitmap(self, bitmap: torch.Tensor) -> None:
-        if (bitmap.device != self.device or bitmap.dtype != torch.int32 or not bitmap.is_contiguous()
-                or tuple(bitmap.shape) != (self.n, nv.BITMAP_WORDS)):
-            raise ValueError(f"bitmap: expected a contiguous int32 [{self.n}, {nv.BITMAP_WORDS}] tensor on {self.device}")
 
     def load_positions(self, boards, hands, side, move_count, max_moves=None, eval_termination: bool = True):
         """ShogiGame.from_sfen for every env from already-parsed arrays (numpy or torch)."""

@@ -28,7 +28,7 @@ def test_header_symbols_exported():
 
 def test_abi_version_and_layout():
     L = nv.lib()
-    assert L.kz_abi_version() == 2
+    assert L.kz_abi_version() == 3
     offs = (C.c_int64 * 3)()
     total = C.c_int64()
     assert L.kz_state_layout(65536, 500, offs, C.byref(total)) == 0
@@ -95,8 +95,6 @@ def test_invalid_arguments_are_rejected_before_any_device_work():
     assert L.kz_export_positions(z, 4, 500, z, z, z, z) in bad
     assert L.kz_refresh(z, 4, 500, z, 0, z, 0, z, z, 1, 0, 0, 0, 0, z, z) in bad
     assert L.kz_step(z, 4, 500, z, 1, z, 0, z, 0, z, z, z, z, z, z, z, 0, 0, 0, 1, z) == -1
-    assert L.kz_step_compact(z, 4, 500, z, 1, z, z, z, z, z, z, z, z, 0, 0, 0, 1, z) == -1
-    assert L.kz_expand(z, 4, 500, z, z, 0, z, 0, z) == -1
     assert L.kz_step_rollout(z, 4, 500, z, 1, z, 0, z, 448, z, z, z, z, z, z, z, z, 0, 0, 0, 1, z) == -1
     assert L.kz_legal_bitmap(z, 4, 500, z, 0, z, 448, z, z, z) == -1
     assert L.kz_step_range(z, 4, 500, 0, 2, 0, z, 1, z, 0, z, 0, z, 0, z, z, z, z, z, z, z, z, 0, 0, 0, 1, z) == -1

@@ -574,40 +574,6 @@ def test_storage_and_action_validation_on_a_live_env():
     assert int(out["done"].sum()) == 0 and bool((env.errors() & 1).all())
 
 
-@pytest.mark.parametrize("n,T", [(1000, 50), (4096, 70)])
-def test_split_pipeline_equals_fused_step(n, T):
-    """kz_step_compact + kz_expand (legal bitmap handed over through HBM) against the fused kz_step on twin batches:
-    identical rows and scalars every step, across auto-resets (max_moves 60), in both mask layouts."""
-    from shogidrl_b200 import VecShogiEnv
-
-    dev = torch.device("cuda:0")
-    a = VecShogiEnv(n, max_moves_per_game=60, device=dev, seed=5)
-    b = VecShogiEnv(n, max_moves_per_game=60, device=dev, seed=5)
-    act_a = [torch.zeros(n, dtype=torch.int64, device=dev) for _ in range(2)]
-    act_b = [torch.zeros(n, dtype=torch.int64, device=dev) for _ in range(2)]
-    a.refresh(random_actions=True, next_out=act_a[0])
-    b.refresh(random_actions=True, next_out=act_b[0])
-    contiguous = torch.zeros((n, 13527), dtype=torch.uint8, device=dev)
-    finished = 0
-    for t in range(T):
-        oa = a.step(act_a[t & 1], random_actions=True, next_out=act_a[(t + 1) & 1])
-        ob = b.step_compact(act_b[t & 1], random_actions=True, next_out=act_b[(t + 1) & 1])
-        b.obs.fill_(-1.0)
-        b._mask_store.fill_(7)
-        b.expand()
-        assert torch.equal(a.obs, b.obs) and torch.equal(a.mask, b.mask), t
-        for k in ("reward", "done", "reason", "winner", "ep_len", "legal_count"):
-            assert torch.equal(oa[k], ob[k]), (t, k)
-        assert torch.equal(act_a[(t + 1) & 1], act_b[(t + 1) & 1]), t
-        if t % 16 == 3:
-            contiguous.fill_(9)
-            b.expand(mask=contiguous)
-            assert torch.equal(contiguous, a.mask), t
-        finished += int(oa["done"].sum())
-    assert finished > 0 and all(torch.equal(x, y) for x, y in zip(a.export(), b.export()))
-    assert int(a.errors().abs().sum()) == 0 and int(b.errors().abs().sum()) == 0
-
-
 @pytest.mark.parametrize("n,T", [(4096, 90), (8, 70)])
 def test_row_writer_variants_agree(n, T):
     """kz_step composes 32-byte aligned, padded mask rows once from the legal bitmap, and writes exactly-13,527-byte rows
