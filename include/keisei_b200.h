@@ -195,6 +195,33 @@ int kz_legal_bitmap(void* state, int n, int hist_cap, float* obs, int64_t obs_st
 int kz_bitmap_expand(const uint32_t* bitmap, int64_t bitmap_stride_words, const int64_t* bitmap_rows, int n, uint8_t* mask,
                      int64_t mask_stride, void* stream);
 
+/* ---- move expansion: the outcome of listed moves without moving the games they start from (look-ahead, search, perft).
+ * kz_legal_list turns n legal-bitmap rows (bitmap_stride_words >= KZ_BITMAP_WORDS_MIN, 4-byte aligned) into a list of legal
+ * moves grouped by game: offsets (int64 [n+1], device) is the exclusive prefix sum of the rows' legal counts, and game g's
+ * legal actions go in ascending order to [offsets[g], offsets[g+1]) of actions_out (int64 if actions_i64 else int32), with
+ * parent_out[i] = g (int32, optional).  A row whose offsets disagree with its bitmap writes nothing outside its own range. */
+int kz_legal_list(const uint32_t* bitmap, int64_t bitmap_stride_words, int n, const int64_t* offsets, int32_t* parent_out,
+                  void* actions_out, int actions_i64, void* stream);
+/* kz_expand applies actions[i] (int64 if actions_i64 else int32) to a copy of game parent[i] (int32) of the batch `state`
+ * (n games, hist_cap), for each of the m items.  Every output of item i is what kz_step(auto_reset = 0) would give for that
+ * one move on a clone of the parent with its history: the action checks, err[i] (u8, the parent's error bits with the
+ * move's own), the position key, the repetition count in the parent's table (a match gives the stored count + 1, a miss 1,
+ * so the 4th occurrence is sennichite as in kz_step), termination in the reference's order, reward / done / reason /
+ * winner / ep_len, legal_count, and the rollout-form rows of kz_step_rollout: obs, bitmap, cobs (rows indexed by the item;
+ * every output pointer optional).  The source batch is not written, except for its work counter counter_slot (0..63, as in
+ * kz_step_range).  An item whose parent lies outside [0, n) gets KZ_ERR_BAD_ACTION, reads nothing, and reports what a
+ * rejected action on an empty board reports (reward 0, done 0, legal_count 0).  Items of one parent should be adjacent:
+ * the parent's rows are then read from cache.
+ * child_state (optional, not the source) is a batch of m games laid out by kz_state_layout(m, child_hist_cap): item i
+ * stores its successor there with status and winner as kz_step leaves them, error bits, plies since reset and finished
+ * episodes 0, and an emptied repetition table -- the position as kz_load_positions + kz_refresh would hold it, which can be
+ * listed, expanded or stepped again.  Children do NOT inherit history: a repetition is counted from the child on, as the
+ * reference's ShogiGame.__deepcopy__ forgets the move history (shogi_game.py:165-169).  m == 0 launches nothing. */
+int kz_expand(const void* state, int n, int hist_cap, int counter_slot, const int32_t* parent, const void* actions,
+              int actions_i64, int m, float* obs, int64_t obs_stride, uint32_t* bitmap, int64_t bitmap_stride_words,
+              uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner, int32_t* ep_len,
+              int32_t* legal_count, uint8_t* err, void* child_state, int child_hist_cap, void* stream);
+
 /* Thin conveniences over kz_refresh. */
 int kz_legal_mask(void* state, int n, int hist_cap, uint8_t* mask, int64_t mask_stride,
                   int32_t* legal_count, void* stream);

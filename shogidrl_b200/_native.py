@@ -26,7 +26,8 @@ EXPORTS = [
     "kz_obs_conv_wgrad", "kz_ppo_loss", "kz_eval_masked_bwd_bias", "kz_adam_clip_workspace", "kz_adam_clip_step",
     "kz_step_rollout", "kz_legal_bitmap", "kz_bitmap_expand", "kz_sample_bitmap",
     "kz_eval_bitmap_fwd", "kz_eval_bitmap_bwd", "kz_step_range", "kz_cobs_conv_fwd", "kz_cobs_conv_wgrad_ctas",
-    "kz_cobs_conv_wgrad", "kz_heuristic_actions", "kz_pool_records", "kz_step_pool", "kz_reset_pool",
+    "kz_cobs_conv_wgrad", "kz_heuristic_actions", "kz_pool_records", "kz_step_pool", "kz_reset_pool", "kz_legal_list",
+    "kz_expand",
 ]
 COBS_WORDS = 40
 POOL_RECORD_WORDS = 512
@@ -78,6 +79,8 @@ def lib() -> C.CDLL:
     L.kz_step_pool.argtypes = [vp, i32, i32, i32, i32, i32, vp, i32, vp, i64, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp,
                                u64, u32, u32, vp, i32, vp, u64, vp, vp]
     L.kz_reset_pool.argtypes = [vp, i32, i32, vp, i32, vp, i32, vp, u64, u32, vp, vp]
+    L.kz_legal_list.argtypes = [vp, i64, i32, vp, vp, vp, i32, vp]
+    L.kz_expand.argtypes = [vp, i32, i32, i32, vp, vp, i32, i32, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]
     L.kz_legal_mask.argtypes = [vp, i32, i32, vp, i64, vp, vp]
     L.kz_observe.argtypes = [vp, i32, i32, vp, i64, vp]
     L.kz_errors.argtypes = [vp, i32, i32, vp, i32, vp]

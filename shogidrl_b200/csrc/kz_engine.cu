@@ -599,6 +599,15 @@ struct StepParams {
   const int32_t* pool_pick;      // optional: record of each game that restarts in this launch
   unsigned long long pool_seed;  // otherwise drawn from rand32(pool_seed, env_offset + g, finished episodes)
   int32_t* start_ids;            // optional: receives the record index of each game that restarts
+  // move expansion (kz_expand; read by the MODE 3 instantiation only): item g applies actions[g] to a copy of source game
+  // parent[g]; boards / meta / hist above are the source batch, which is only read
+  const int32_t* parent;  // [n] source game of each item
+  int src_n;              // games in the source batch
+  uint8_t* err_out;       // optional: error bits of each item
+  uint8_t* child_boards;  // optional: child batch of n games (kz_state_layout(n, child_hist_cap)) ...
+  uint8_t* child_meta;
+  uint4* child_hist;      // ... whose repetition tables the kernel empties
+  int child_rep_slots;
 };
 
 __device__ __forceinline__ uint16_t ld_u16(const uint8_t* p) { return (uint16_t)(p[0] | (p[1] << 8)); }
@@ -610,6 +619,10 @@ __device__ __forceinline__ void st_u16(uint8_t* p, int v) { p[0] = (uint8_t)v; p
 // (loaded positions: nested-generation uchifuzume, full key, optional termination evaluation).
 // POOL (modes 1 and 2, kz_step_pool): a finished game restarts from a record of the start-position pool instead of the
 // start position; nothing else differs.
+// MODE 3 = move expansion (kz_expand): as MODE 2 without auto-reset, for items instead of games -- item g reads the state
+// of source game parent[g] (an item whose parent lies outside the batch reads an empty running game and its action is
+// rejected), probes that game's repetition table without inserting, writes its rows and scalars at g, and stores the
+// successor in the child batch (if any) as a game with no history.  Nothing of the source batch is written.
 template <int MODE, bool POOL = false>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_kernel(const StepParams P) {
   for (int i = threadIdx.x; i < 81 * 8 * 3; i += blockDim.x) s_ray[i] = g_ray[i];
@@ -633,11 +646,20 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
   // the round-2 line attribution.)
   auto fetch_state = [&](int g) -> uint32_t {
     if (g >= g_end) return 0u;
-    const uint8_t* src = lane < 24 ? P.boards + (size_t)g * 96 + 4 * lane : P.meta + (size_t)g * 32 + 4 * (lane - 24);
+    int sg = g;  // the game whose state item g starts from
+    if constexpr (MODE == 3) {
+      sg = P.parent[g];
+      if (sg < 0 || sg >= P.src_n) return lane == 28 ? 0xFFu : 0u;  // empty board, status 0, winner none
+    }
+    const uint8_t* src = lane < 24 ? P.boards + (size_t)sg * 96 + 4 * lane : P.meta + (size_t)sg * 32 + 4 * (lane - 24);
     return *reinterpret_cast<const uint32_t*>(src);
   };
   auto fetch_action = [&](int g) -> long long {
     if (g >= g_end || MODE == 0) return 0;
+    if constexpr (MODE == 3) {
+      const int sg = P.parent[g];
+      if (sg < 0 || sg >= P.src_n) return -1;  // rejected: KZ_ERR_BAD_ACTION
+    }
     return P.actions_i64 ? reinterpret_cast<const long long*>(P.actions)[g]
                          : (long long)reinterpret_cast<const int*>(P.actions)[g];
   };
@@ -813,7 +835,8 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
           if (hist_len < P.hist_cap) {
             // issue the probe's loads now; they are consumed after the move generation, which hides the DRAM trip
             probe = true;
-            probe_e = (P.hist + (size_t)g * P.rep_slots)[(key.y + lane) & ((uint32_t)P.rep_slots - 1u)];
+            const int hg = MODE == 3 ? P.parent[g] : g;  // whose repetition table (MODE 3: only a valid parent moves)
+            probe_e = (P.hist + (size_t)hg * P.rep_slots)[(key.y + lane) & ((uint32_t)P.rep_slots - 1u)];
             hist_len += 1;
           } else {
             err |= KZ_ERR_HISTORY_FULL;
@@ -1008,7 +1031,7 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
     }
 
     if (probe) {  // repetition count of the new position: match / insert in the first window, further windows if needed
-      uint4* tb = P.hist + (size_t)g * P.rep_slots;
+      uint4* tb = P.hist + (size_t)(MODE == 3 ? P.parent[g] : g) * P.rep_slots;  // MODE 3: the parent's, read only
       const uint32_t smask = (uint32_t)P.rep_slots - 1u;
       uint32_t start = key.y & smask;
       int count = 0;
@@ -1024,7 +1047,7 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
           const uint32_t oldw = __shfl_sync(FULL, e.w, f);
           const bool was_match = (__ballot_sync(FULL, match) >> f) & 1;
           count = was_match ? min(15, (int)(oldw & 15u) + 1) : 1;
-          if (lane == f) tb[slot] = make_uint4(key.x, key.y, key.z, (key.w & ~15u) | (uint32_t)count);
+          if (MODE != 3 && lane == f) tb[slot] = make_uint4(key.x, key.y, key.z, (key.w & ~15u) | (uint32_t)count);
           break;
         }
         start += 32;
@@ -1048,7 +1071,7 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
       if (winner >= 0) reward = winner == mover ? 1.f : -1.f;
     }
 
-    if (MODE != 0 && status != 0 && P.auto_reset) {
+    if (MODE != 0 && MODE != 3 && status != 0 && P.auto_reset) {
       // StepManager.handle_episode_end -> game.reset() (step_manager.py:437-440; shogi_game.py:113-130)
       if constexpr (POOL) {
         // the same reset from record k of the start-position pool: state rows, position key, legal bitmap, count and
@@ -1102,6 +1125,9 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
       if (P.ep_len) P.ep_len[g] = ep_len_out;
       if (P.legal_count) P.legal_count[g] = gr.count;
       if (P.in_check) P.in_check[g] = (uint8_t)gr.in_check;
+      if constexpr (MODE == 3) {
+        if (P.err_out) P.err_out[g] = (uint8_t)err;
+      }
     }
 
     auto write_mask = [&]() {
@@ -1263,8 +1289,8 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
       uint4* dst = reinterpret_cast<uint4*>(P.bitmap_out + (size_t)g * P.bitmap_stride);
       for (int i = lane; i < BITMAP_WORDS / 4; i += 32) dst[i] = reinterpret_cast<const uint4*>(ws.bitmap)[i];
     }
-    if constexpr (MODE != 2) write_mask();
-    pick_next();
+    if constexpr (MODE != 2 && MODE != 3) write_mask();
+    if constexpr (MODE != 3) pick_next();
     write_obs();
     if (P.cobs_out) {
       // compact observation: what the 46 planes are made of -- per observation square (already rotated for White to move)
@@ -1296,7 +1322,9 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
       __syncwarp();
     }
 
-    // ---- store state
+    // ---- store state (MODE 3: the child, if any, with no history -- error bits, plies since reset and episodes 0, an
+    // emptied repetition table)
+    if constexpr (MODE == 3) { err = 0; hist_len = 0; episodes = 0; }
     __syncwarp();
     if (lane == 0) {
       ws.meta[14] = (uint8_t)side;
@@ -1313,7 +1341,16 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM) kz_step_k
       reinterpret_cast<uint32_t*>(ws.meta)[7] = key.w;
     }
     __syncwarp();
-    {
+    if constexpr (MODE == 3) {
+      if (P.child_boards) {
+        uint32_t* bdst = reinterpret_cast<uint32_t*>(P.child_boards + (size_t)g * 96);
+        uint32_t* mdst = reinterpret_cast<uint32_t*>(P.child_meta + (size_t)g * 32);
+        if (lane < 24) bdst[lane] = reinterpret_cast<uint32_t*>(ws.board)[lane];
+        else mdst[lane - 24] = reinterpret_cast<uint32_t*>(ws.meta)[lane - 24];
+        uint4* tb = P.child_hist + (size_t)g * P.child_rep_slots;
+        for (int i = lane; i < P.child_rep_slots; i += 32) tb[i] = make_uint4(0, 0, 0, 0);
+      }
+    } else {
       uint32_t* bdst = reinterpret_cast<uint32_t*>(P.boards + (size_t)g * 96);
       uint32_t* mdst = reinterpret_cast<uint32_t*>(P.meta + (size_t)g * 32);
       if (lane < 24) bdst[lane] = reinterpret_cast<uint32_t*>(ws.board)[lane];
@@ -1347,6 +1384,42 @@ __global__ void __launch_bounds__(256) kz_bitmap_expand_kernel(const uint32_t* _
     for (int i = (KZ_NUM_ACTIONS / 4) * 4 + lane; i < KZ_NUM_ACTIONS; i += 32) mrow[i] = (uint8_t)((__ldg(bm + (i >> 5)) >> (i & 31)) & 1);
   } else {
     for (int i = lane; i < KZ_NUM_ACTIONS; i += 32) mrow[i] = (uint8_t)((__ldg(bm + (i >> 5)) >> (i & 31)) & 1);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Legal bitmap rows -> a CSR list of legal moves (kz_legal_list), one warp per game: the set bits of row g in ascending
+// order go to [offsets[g], offsets[g+1]).  The warp walks the row 32 words at a time and visits only the non-zero words
+// (ballot); within a word, lane l owns bit l, and its place is the popcount of the bits below it.  Nothing is written
+// outside a row's own range, whatever its offsets say.
+__global__ void __launch_bounds__(256) kz_legal_list_kernel(const uint32_t* __restrict__ bitmap, long long ldb, int n,
+                                                            const long long* __restrict__ offsets, int32_t* parent_out,
+                                                            void* actions_out, int actions_i64) {
+  const int lane = threadIdx.x & 31;
+  const int g = blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (g >= n) return;
+  const long long lo = offsets[g], hi = offsets[g + 1];
+  if (lo < 0) return;
+  const uint32_t* bm = bitmap + (size_t)g * ldb;
+  long long base = lo;
+  for (int w0 = 0; w0 < KZ_BITMAP_WORDS_MIN && base < hi; w0 += 32) {  // warp-uniform
+    const int w = w0 + lane;
+    uint32_t v = w < KZ_BITMAP_WORDS_MIN ? __ldg(bm + w) : 0u;
+    if (w == KZ_BITMAP_WORDS_MIN - 1) v &= (1u << (KZ_NUM_ACTIONS - 32 * (KZ_BITMAP_WORDS_MIN - 1))) - 1u;
+    uint32_t nz = __ballot_sync(FULL, v != 0);
+    while (nz) {
+      const int k = __ffs(nz) - 1;
+      nz &= nz - 1;
+      const uint32_t word = __shfl_sync(FULL, v, k);
+      const long long pos = base + __popc(word & ((1u << lane) - 1u));
+      if (((word >> lane) & 1) && pos < hi) {
+        const int a = (w0 + k) * 32 + lane;
+        if (actions_i64) reinterpret_cast<long long*>(actions_out)[pos] = a;
+        else reinterpret_cast<int32_t*>(actions_out)[pos] = a;
+        if (parent_out) parent_out[pos] = g;
+      }
+      base += __popc(word);
+    }
   }
 }
 
@@ -1545,22 +1618,20 @@ Layout layout(int n, int hist_cap) {
   return L;
 }
 
-// The kz_step_kernel instantiations, [pool][mode]: refresh (mode 0) has no pool form.  launch_step launches through this
-// table and kz_init_tables sets the dynamic shared-memory limit of every entry.
+// The kz_step_kernel instantiations, [pool][mode]: refresh (mode 0) and expansion (mode 3) have no pool form.  launch_step
+// launches through this table and kz_init_tables sets the dynamic shared-memory limit of every entry.
 using StepKernel = void (*)(const StepParams);
-const StepKernel kStepKernels[2][3] = {{kz_step_kernel<0>, kz_step_kernel<1>, kz_step_kernel<2>},
-                                       {nullptr, kz_step_kernel<1, true>, kz_step_kernel<2, true>}};
-StepKernel step_kernel(int mode, bool pool) { return mode >= 0 && mode < 3 ? kStepKernels[pool][mode] : nullptr; }
+const StepKernel kStepKernels[2][4] = {{kz_step_kernel<0>, kz_step_kernel<1>, kz_step_kernel<2>, kz_step_kernel<3>},
+                                       {nullptr, kz_step_kernel<1, true>, kz_step_kernel<2, true>, nullptr}};
+StepKernel step_kernel(int mode, bool pool) { return mode >= 0 && mode < 4 ? kStepKernels[pool][mode] : nullptr; }
 
 #ifndef KZ_COMPACT_CTAS_PER_SM
 #define KZ_COMPACT_CTAS_PER_SM 2
 #endif
 
-int launch_step(void* state, int n, int hist_cap, StepParams P, cudaStream_t st, int first = 0, int count = -1, int slot = 0) {
+// Pointers of the state blob's sections (n games, hist_cap) in P; KZ_E_ARG for a bad blob.
+int bind_state(void* state, int n, int hist_cap, StepParams& P, uint8_t** sched) {
   if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535) return KZ_E_ARG;
-  if (count < 0) count = n - first;
-  if (first < 0 || count <= 0 || first + count > n || slot < 0 || slot >= 64) return KZ_E_ARG;
-  if (!host_ready()) return KZ_E_NOT_INIT;
   if (((uintptr_t)state & 255) != 0) return KZ_E_ARG;
   const Layout L = layout(n, hist_cap);
   uint8_t* base = reinterpret_cast<uint8_t*>(state);
@@ -1569,8 +1640,28 @@ int launch_step(void* state, int n, int hist_cap, StepParams P, cudaStream_t st,
   P.hist = reinterpret_cast<uint4*>(base + L.off_hist);
   P.rep_slots = L.rep_slots;
   P.hist_cap = hist_cap;
+  *sched = base + L.off_sched;
+  return KZ_OK;
+}
+
+int launch_kernel(StepParams P, uint8_t* sched, int slot, cudaStream_t st);
+
+int launch_step(void* state, int n, int hist_cap, StepParams P, cudaStream_t st, int first = 0, int count = -1, int slot = 0) {
+  if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535) return KZ_E_ARG;
+  if (count < 0) count = n - first;
+  if (first < 0 || count <= 0 || first + count > n || slot < 0 || slot >= 64) return KZ_E_ARG;
+  if (!host_ready()) return KZ_E_NOT_INIT;
+  uint8_t* sched = nullptr;
+  if (bind_state(state, n, hist_cap, P, &sched) != KZ_OK) return KZ_E_ARG;
   P.n = count;
   P.g_first = first;
+  return launch_kernel(P, sched, slot, st);
+}
+
+// Row checks, grid, work counter (slot `slot` of the scheduling block `sched`) and the launch of kz_step_kernel<P.mode>
+// over the P.n games (or kz_expand's items) from P.g_first on.
+int launch_kernel(StepParams P, uint8_t* sched, int slot, cudaStream_t st) {
+  const int count = P.n;
   if (P.obs) {
     if (((uintptr_t)P.obs & 15) || (P.obs_stride & 1) || P.obs_stride < KZ_OBS_FLOATS) return KZ_E_ARG;
   }
@@ -1595,7 +1686,7 @@ int launch_step(void* state, int n, int hist_cap, StepParams P, cudaStream_t st,
   if (grid < ctas_needed && count % WARPS_PER_CTA == 0) {
     // launches on one state buffer are ordered by their data dependence, so the counter can live in it (launches over
     // disjoint game ranges that run concurrently, kz_step_range, name different counter slots)
-    P.tile_counter = reinterpret_cast<int*>(base + L.off_sched) + slot;
+    P.tile_counter = reinterpret_cast<int*>(sched) + slot;
     CK(cudaMemsetAsync(P.tile_counter, 0, sizeof(int), st));
   }
 #endif
@@ -1914,6 +2005,49 @@ int kz_legal_mask(void* state, int n, int hist_cap, uint8_t* mask, int64_t mask_
 int kz_observe(void* state, int n, int hist_cap, float* obs, int64_t obs_stride, void* stream) {
   if (!obs) return KZ_E_ARG;
   return kz_refresh(state, n, hist_cap, obs, obs_stride, nullptr, 0, nullptr, nullptr, 0, 0, 0, 0, 0, nullptr, stream);
+}
+
+int kz_legal_list(const uint32_t* bitmap, int64_t bitmap_stride_words, int n, const int64_t* offsets, int32_t* parent_out,
+                  void* actions_out, int actions_i64, void* stream) {
+  if (!bitmap || bitmap_stride_words < KZ_BITMAP_WORDS_MIN || n < 0 || !offsets || !actions_out || ((uintptr_t)bitmap & 3))
+    return KZ_E_ARG;
+  if (n == 0) return KZ_OK;
+  kz_legal_list_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      bitmap, bitmap_stride_words, n, reinterpret_cast<const long long*>(offsets), parent_out, actions_out, actions_i64);
+  CK(cudaGetLastError());
+  return KZ_OK;
+}
+
+int kz_expand(const void* state, int n, int hist_cap, int counter_slot, const int32_t* parent, const void* actions,
+              int actions_i64, int m, float* obs, int64_t obs_stride, uint32_t* bitmap, int64_t bitmap_stride_words,
+              uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner, int32_t* ep_len,
+              int32_t* legal_count, uint8_t* err, void* child_state, int child_hist_cap, void* stream) {
+  if (!state || n <= 0 || !parent || !actions || m < 0 || counter_slot < 0 || counter_slot >= 64) return KZ_E_ARG;
+  if (m == 0) return KZ_OK;
+  if (!host_ready()) return KZ_E_NOT_INIT;
+  StepParams P{};
+  uint8_t* sched = nullptr;
+  // the kernel writes nothing of the source batch but its work counter (MODE 3)
+  if (bind_state(const_cast<void*>(state), n, hist_cap, P, &sched) != KZ_OK) return KZ_E_ARG;
+  P.n = m;
+  P.g_first = 0;
+  P.actions = actions; P.actions_i64 = actions_i64;
+  P.obs = obs; P.obs_stride = obs_stride;
+  P.bitmap_out = bitmap; P.bitmap_stride = bitmap_stride_words; P.cobs_out = cobs;
+  P.reward = reward; P.done = done; P.reason = reason; P.winner = winner; P.ep_len = ep_len;
+  P.legal_count = legal_count;
+  P.mode = 3;
+  P.parent = parent; P.src_n = n; P.err_out = err;
+  if (child_state) {
+    if (child_state == state || child_hist_cap < 0 || child_hist_cap > 65535 || ((uintptr_t)child_state & 255)) return KZ_E_ARG;
+    const Layout C = layout(m, child_hist_cap);
+    uint8_t* cb = reinterpret_cast<uint8_t*>(child_state);
+    P.child_boards = cb + C.off_boards;
+    P.child_meta = cb + C.off_meta;
+    P.child_hist = reinterpret_cast<uint4*>(cb + C.off_hist);
+    P.child_rep_slots = C.rep_slots;
+  }
+  return launch_kernel(P, sched, counter_slot, reinterpret_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

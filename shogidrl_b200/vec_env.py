@@ -102,9 +102,10 @@ class VecShogiEnv:
     def _sp(self):
         return nv.stream_ptr(self.device)
 
-    def _rows_arg(self, t: Optional[torch.Tensor], what: str, dtypes, row_elems: int):
-        """(data pointer, row stride in elements) of caller storage the kernel writes ``n`` rows into; rejects
-        anything the kernel would write out of bounds (the C ABI sees raw pointers only)."""
+    def _rows_arg(self, t: Optional[torch.Tensor], what: str, dtypes, row_elems: int, n: Optional[int] = None):
+        """(data pointer, row stride in elements) of caller storage the kernel writes ``n`` rows into (default: one per
+        env); rejects anything the kernel would write out of bounds (the C ABI sees raw pointers only)."""
+        n = self.n if n is None else n
         if t is None:
             return None, 0
         if t.device != self.device or t.dtype not in dtypes:
@@ -114,23 +115,25 @@ class VecShogiEnv:
             inner = t[0]
         else:
             rows, stride, inner = 1, row_elems, t
-        if rows < self.n or inner.numel() < row_elems or not inner.is_contiguous():
-            raise ValueError(f"{what}: need at least {self.n} rows of {row_elems} contiguous elements, got shape "
+        if rows < n or inner.numel() < row_elems or not inner.is_contiguous():
+            raise ValueError(f"{what}: need at least {n} rows of {row_elems} contiguous elements, got shape "
                              f"{tuple(t.shape)} with strides {tuple(t.stride())}")
         return t.data_ptr(), stride
 
-    def _obs_args(self, obs: Optional[torch.Tensor]):
-        return self._rows_arg(obs, "obs", (torch.float32,), nv.OBS_FLOATS)
+    def _obs_args(self, obs: Optional[torch.Tensor], n: Optional[int] = None):
+        return self._rows_arg(obs, "obs", (torch.float32,), nv.OBS_FLOATS, n)
 
     def _mask_args(self, mask: Optional[torch.Tensor]):
         return self._rows_arg(mask, "mask", (torch.uint8, torch.bool), nv.NUM_ACTIONS)
 
-    def _vec_arg(self, t: Optional[torch.Tensor], what: str, dtypes):
-        """Data pointer of a contiguous [n] vector on the env's device (None stays None)."""
+    def _vec_arg(self, t: Optional[torch.Tensor], what: str, dtypes, n: Optional[int] = None):
+        """Data pointer of a contiguous [n] vector on the env's device (default n: one element per env; None stays
+        None)."""
+        n = self.n if n is None else n
         if t is None:
             return None
-        if t.device != self.device or t.dtype not in dtypes or not t.is_contiguous() or t.numel() < self.n:
-            raise ValueError(f"{what}: expected a contiguous {'/'.join(str(d)[6:] for d in dtypes)} [{self.n}] tensor on "
+        if t.device != self.device or t.dtype not in dtypes or not t.is_contiguous() or t.numel() < n:
+            raise ValueError(f"{what}: expected a contiguous {'/'.join(str(d)[6:] for d in dtypes)} [{n}] tensor on "
                              f"{self.device}, got {tuple(t.shape)} {t.dtype} on {t.device}")
         return t.data_ptr()
 
@@ -341,6 +344,55 @@ class VecShogiEnv:
                                          self.legal_count.data_ptr(), self._sp()), "kz_legal_bitmap")
         return obs, bitmap
 
+    def legal_actions(self):
+        """Every legal move of every env's CURRENT position as a list grouped by env (CSR): -> (offsets int64 [n+1],
+        parent int32 [M], actions int64 [M]); env g's legal actions are actions[offsets[g]:offsets[g+1]] in ascending
+        order, and parent[i] is the env of move i.  kz_legal_bitmap into scratch rows, then kz_legal_list; one host read
+        (of M, to size the list)."""
+        d, sp = self.device, self._sp()
+        bitmap = torch.empty((self.n, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
+        count = torch.empty(self.n, dtype=torch.int32, device=d)
+        nv.check(self._L.kz_legal_bitmap(self.state.data_ptr(), self.n, self.hist_cap, None, 0, bitmap.data_ptr(),
+                                         nv.BITMAP_WORDS, None, count.data_ptr(), sp), "kz_legal_bitmap")
+        offsets = torch.zeros(self.n + 1, dtype=torch.int64, device=d)
+        offsets[1:] = torch.cumsum(count, 0, dtype=torch.int64)
+        m = int(offsets[-1])
+        parent = torch.empty(m, dtype=torch.int32, device=d)
+        actions = torch.empty(m, dtype=torch.int64, device=d)
+        nv.check(self._L.kz_legal_list(bitmap.data_ptr(), nv.BITMAP_WORDS, self.n, offsets.data_ptr(), parent.data_ptr(),
+                                       actions.data_ptr(), 1, sp), "kz_legal_list")
+        return offsets, parent, actions
+
+    def expand(self, parent: torch.Tensor, actions: torch.Tensor, *, obs: Optional[torch.Tensor] = None,
+               bitmap: Optional[torch.Tensor] = None, cobs: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        """What would happen if env ``parent[i]`` played ``actions[i]``, for M items at once, without moving any env
+        (kz_expand): -> dict of per-item tensors reward, done, reason, winner, ep_len, legal_count and err (error bits),
+        each exactly what ``step`` (without auto-reset) would report for that one move on a copy of the env, its
+        repetition history included.  ``parent`` int32 [M] (each in [0, n)), ``actions`` int64 / int32 [M]; ``obs``
+        (fp32 [M, 46, 9, 9]), ``bitmap`` (int32 [M, 448]) and ``cobs`` (int32 [M, 40]) optionally receive the successors'
+        rows as ``step_rollout`` writes them.  Items of one env should be adjacent (as ``legal_actions`` lists them)."""
+        m = int(parent.numel())
+        pp = self._vec_arg(parent, "parent", (torch.int32,), m)
+        ap = self._vec_arg(actions, "actions", (torch.int64, torch.int32), m)
+        nv.require(int(actions.numel()) == m, "parent and actions must have the same length")
+        d = self.device
+        out = {"reward": torch.zeros(m, dtype=torch.float32, device=d), "done": torch.zeros(m, dtype=torch.uint8, device=d),
+               "reason": torch.zeros(m, dtype=torch.uint8, device=d), "winner": torch.zeros(m, dtype=torch.int8, device=d),
+               "ep_len": torch.zeros(m, dtype=torch.int32, device=d),
+               "legal_count": torch.zeros(m, dtype=torch.int32, device=d), "err": torch.zeros(m, dtype=torch.uint8, device=d)}
+        if m == 0:
+            return out
+        if bool(((parent < 0) | (parent >= self.n)).any()):
+            raise ValueError(f"parent: every entry must name an env in [0, {self.n})")
+        op, os_ = self._obs_args(obs, m)
+        bp, bs = (None, 0) if bitmap is None else self._bitmap_args(bitmap, m)
+        nv.check(self._L.kz_expand(self.state.data_ptr(), self.n, self.hist_cap, 0, pp, ap, int(actions.dtype == torch.int64),
+                                   m, op, os_, bp, bs, self._cobs_arg(cobs, m), out["reward"].data_ptr(),
+                                   out["done"].data_ptr(), out["reason"].data_ptr(), out["winner"].data_ptr(),
+                                   out["ep_len"].data_ptr(), out["legal_count"].data_ptr(), out["err"].data_ptr(), None, 0,
+                                   self._sp()), "kz_expand")
+        return out
+
     # The heuristic opponent draws from the env's random stream keyed by seed ^ HEURISTIC_SALT, so its pick is independent
     # of the fused uniform-random action (next_actions, keyed by the seed itself) drawn for the same step and env.
     HEURISTIC_SALT = 0x48657572697374  # "Heurist"
@@ -371,19 +423,21 @@ class VecShogiEnv:
                                               self.env_offset, self._sp()), "kz_heuristic_actions")
         return out
 
-    def _cobs_arg(self, cobs: Optional[torch.Tensor]):
+    def _cobs_arg(self, cobs: Optional[torch.Tensor], n: Optional[int] = None):
+        n = self.n if n is None else n
         if cobs is None:
             return None
-        if (cobs.device != self.device or cobs.dtype != torch.int32 or cobs.dim() != 2 or cobs.shape[0] < self.n
+        if (cobs.device != self.device or cobs.dtype != torch.int32 or cobs.dim() != 2 or cobs.shape[0] < n
                 or cobs.shape[1] != nv.COBS_WORDS or not cobs.is_contiguous()):
-            raise ValueError(f"cobs: expected a contiguous int32 [{self.n}, {nv.COBS_WORDS}] tensor on {self.device}")
+            raise ValueError(f"cobs: expected a contiguous int32 [{n}, {nv.COBS_WORDS}] tensor on {self.device}")
         return cobs.data_ptr()
 
-    def _bitmap_args(self, bitmap: torch.Tensor):
-        if (bitmap.device != self.device or bitmap.dtype != torch.int32 or bitmap.dim() != 2 or bitmap.shape[0] < self.n
+    def _bitmap_args(self, bitmap: torch.Tensor, n: Optional[int] = None):
+        n = self.n if n is None else n
+        if (bitmap.device != self.device or bitmap.dtype != torch.int32 or bitmap.dim() != 2 or bitmap.shape[0] < n
                 or bitmap.shape[1] != nv.BITMAP_WORDS or bitmap.stride(1) != 1 or bitmap.stride(0) % 4
                 or bitmap.data_ptr() % 16):
-            raise ValueError(f"bitmap: expected int32 [{self.n}, {nv.BITMAP_WORDS}] rows (16-byte aligned) on {self.device}")
+            raise ValueError(f"bitmap: expected int32 [{n}, {nv.BITMAP_WORDS}] rows (16-byte aligned) on {self.device}")
         return bitmap.data_ptr(), bitmap.stride(0)
 
     def load_positions(self, boards, hands, side, move_count, max_moves=None, eval_termination: bool = True):
