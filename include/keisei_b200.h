@@ -239,8 +239,9 @@ int kz_errors(void* state, int n, int hist_cap, int32_t* out, int clear, void* s
  * masked softmax over 13,527 logits, Categorical sample (or argmax if deterministic) and
  * log_prob with torch.distributions' probs->logits clamp (eps = FLT_EPSILON).
  *   logits [n][ld] fp32 (logits_bf16 == 0) or bf16; mask [n][ldm] bytes; actions int64/int32;
- *   logp fp32; entropy optional fp32.  Rows whose mask is all zero fall back to the uniform
- *   distribution over all actions (base_actor_critic.py:93-101).  Sampling is inverse-CDF on a
+ *   logp fp32; entropy optional fp32.  A legal logit of -inf has probability 0.  Rows whose softmax is NaN -- mask
+ *   all zero, every legal logit -inf, or a legal logit NaN or +inf -- fall back to the uniform distribution over all
+ *   actions (base_actor_critic.py:93-101): a uniform draw, argmax 0, log_prob log(1/13527).  Sampling is inverse-CDF on a
  *   counter-based uniform keyed (seed, offset + row): statistical, not bitwise, parity with
  *   torch.multinomial.  offset_dev (optional device uint64): added to offset when the kernel runs,
  *   so that a launch captured in a CUDA graph draws fresh numbers on every replay (the caller
@@ -248,8 +249,9 @@ int kz_errors(void* state, int n, int hist_cap, int32_t* out, int clear, void* s
 int kz_sample_masked(const void* logits, int logits_bf16, int64_t ld, const uint8_t* mask, int64_t ldm,
                      int n, uint64_t seed, uint64_t offset, const uint64_t* offset_dev, void* actions,
                      int actions_i64, float* logp, float* entropy, int deterministic, void* stream);
-/* The same with the legal set given as bitmap rows (kz_step_rollout): bitmap [n][ldb_words] uint32.  For a 16-byte
- * aligned byte mask of the same set the two entry points return identical actions, log-probs and entropies. */
+/* The same with the legal set given as bitmap rows (kz_step_rollout): bitmap [n][ldb_words] uint32; the pad bits
+ * 13,527-13,535 of word 422 and words 423.. are ignored.  For a 16-byte aligned byte mask of the same set the two entry
+ * points return identical actions, log-probs and entropies. */
 int kz_sample_bitmap(const void* logits, int logits_bf16, int64_t ld, const uint32_t* bitmap, int64_t ldb_words,
                      int n, uint64_t seed, uint64_t offset, const uint64_t* offset_dev, void* actions,
                      int actions_i64, float* logp, float* entropy, int deterministic, void* stream);
@@ -285,7 +287,9 @@ int kz_gae_exact(const float* rewards, const float* values, const uint8_t* dones
  * (SURVEY 8f-1): masked softmax, log-prob of the taken action and entropy (Categorical(probs) clamp semantics),
  * forward and backward.  logits [n][ld] fp32/bf16; mask rows are mask[mask_rows[i]] when mask_rows != NULL (lets
  * a minibatch index the rollout's mask storage without gathering it); saved4 [n][4] fp32 scratch handed from
- * forward to backward; dlogits [n][ldg] in the logits dtype (pad columns beyond 13,527 are not written). */
+ * forward to backward; dlogits [n][ldg] in the logits dtype (pad columns beyond 13,527 are not written).  Rows whose
+ * softmax is NaN (no legal action, every legal logit -inf, a legal logit NaN or +inf) take the uniform distribution,
+ * as kz_sample_masked does, with a zero gradient and no bias contribution. */
 int kz_eval_masked_fwd(const void* logits, int logits_bf16, int64_t ld, const uint8_t* mask, int64_t ldm,
                        const int64_t* mask_rows, const int64_t* actions, int n, float* logp, float* entropy,
                        float* saved4, void* stream);
@@ -303,7 +307,8 @@ int kz_eval_masked_bwd_bias(const void* logits, int logits_bf16, int64_t ld, con
                             const float* dentropy, const float* saved4, void* dlogits, int64_t ldg, int64_t* dbias_q44,
                             void* stream);
 /* Bitmap forms of the evaluation pair: legal sets as rows bitmap[bitmap_rows[i]] (or bitmap[i]) of kz_step_rollout's
- * output; dbias_q44 optional (NULL: no bias gradient).  Results identical to the byte-mask forms on the same sets. */
+ * output, pad bits ignored as in kz_sample_bitmap; dbias_q44 optional (NULL: no bias gradient).  Results identical to
+ * the byte-mask forms on the same sets. */
 int kz_eval_bitmap_fwd(const void* logits, int logits_bf16, int64_t ld, const uint32_t* bitmap, int64_t ldb_words,
                        const int64_t* bitmap_rows, const int64_t* actions, int n, float* logp, float* entropy,
                        float* saved4, void* stream);

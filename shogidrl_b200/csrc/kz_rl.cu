@@ -82,10 +82,12 @@ struct BitmapWindows {
     nw = (KZ_NUM_ACTIONS + 15) >> 4;
   }
   __device__ __forceinline__ int first(int w) const { return w << 4; }
+  // window nw - 1 = bits 13,520-13,535 of word 422: only its low 7 bits are actions, the 9 pad bits read as 0
   __device__ __forceinline__ uint32_t load(int w) const {
     if (w >= nw) return 0u;
     const uint32_t x = __ldg(row + (w >> 1));
-    return (w & 1) ? (x >> 16) : (x & 0xFFFFu);
+    const uint32_t v = (w & 1) ? (x >> 16) : (x & 0xFFFFu);
+    return w == nw - 1 ? v & ((1u << (KZ_NUM_ACTIONS - 16 * (nw - 1))) - 1u) : v;
   }
   static __device__ __forceinline__ uint32_t bits16(uint32_t v) { return v; }
   __device__ __forceinline__ bool legal(long long a) const { return (row[a >> 5] >> (a & 31)) & 1u; }
@@ -173,8 +175,11 @@ __global__ void __launch_bounds__(256, 4) kz_sample_kernel(const void* logits, i
   LegalList ll{s_list[threadIdx.x >> 5], 0, false};
   const int A = KZ_NUM_ACTIONS;
 
-  // pass 1: online max / sum of exp over this lane's share of the legal entries; per-lane argmax (lowest index on ties)
-  float m = -INFINITY, s = 0.f;
+  // pass 1: online max / sum of exp over this lane's share of the legal entries; per-lane argmax (lowest index on ties).
+  // m starts at -FLT_MAX, not -inf: a -inf logit then adds exp(-inf) = 0 (from m = -inf it would add
+  // exp(-inf - -inf) = NaN), and every finite logit takes the same steps as from -inf.  A NaN logit makes s NaN, which
+  // every later update keeps; a +inf logit makes m = +inf.  Both make the reference's softmax row NaN.
+  float m = -FLT_MAX, s = 0.f;
   int amax = 0x7fffffff;
   each_legal_of_row(W, lane, ll, [&](int i) {
     const float x = ld_logit(lrow, i, bf16);
@@ -186,16 +191,16 @@ __global__ void __launch_bounds__(256, 4) kz_sample_kernel(const void* logits, i
   for (int o = 16; o; o >>= 1) M = fmaxf(M, __shfl_xor_sync(FULL, M, o));
   long long act = -1;
   float lp = 0.f, ent = 0.f;
-  if (!(M > -INFINITY)) {
-    // no legal entry (or all legal logits are -inf): softmax is NaN -> uniform over all actions
-    // (base_actor_critic.py:93-101)
+  if (!(M < INFINITY) || __any_sync(FULL, isnan(s)) || !__any_sync(FULL, s > 0.f)) {
+    // a legal +inf or NaN logit, all legal logits -inf, or no legal entry: the softmax row is NaN -> uniform over all
+    // actions (base_actor_critic.py:93-101)
     const float p = 1.0f / (float)A;
     if (deterministic) act = 0;
     else act = (long long)(((unsigned long long)hash_u32(seed, offset + row) * (unsigned long long)A) >> 32);
     lp = logf(p);
     ent = -logf(p);
   } else {
-    const float mys = (m > -INFINITY) ? s * expf(m - M) : 0.f;  // this lane's sum rescaled to the row max
+    const float mys = s * expf(m - M);  // this lane's sum rescaled to the row max (0 for a lane without a finite entry)
     float tot = mys;
 #pragma unroll
     for (int o = 16; o; o >>= 1) tot += __shfl_xor_sync(FULL, tot, o);
@@ -323,8 +328,7 @@ __global__ void __launch_bounds__(256) kz_heuristic_kernel(const uint8_t* __rest
 #pragma unroll 9
   for (int r = 0; r < HEUR_ROUNDS; r++) {
     const int A = 32 * r + lane;
-    uint32_t v = A < HEUR_WINDOWS ? legal16(W, A) : 0u;
-    if (A == HEUR_WINDOWS - 1) v &= (1u << (KZ_NUM_ACTIONS - 16 * (HEUR_WINDOWS - 1))) - 1u;  // bitmap pad bits
+    const uint32_t v = A < HEUR_WINDOWS ? legal16(W, A) : 0u;  // (BitmapWindows drops the bitmap's pad bits)
     uint32_t t0, t1;
     heur_classify(v, A, enemy, pawns, t0, t1);
     c0 += __popc(t0); c1 += __popc(t1); c2 += __popc(v & ~(t0 | t1));
@@ -442,7 +446,8 @@ __global__ void kz_gae_warpscan_kernel(const float* __restrict__ rewards, const 
 // entropy with torch.distributions.Categorical(probs)'s clamp(p, eps, 1 - eps), one warp per row, and the
 // matching backward.  Replaces ~30 elementwise ATen passes over [B, 13527] by two reads (forward) and one
 // read + one write (backward).  Forward saves per row: max M, normaliser Z, S = sum_i g_i p_i with
-// g_i = dH/dp_i; rows without a legal action fall back to the uniform distribution with zero gradient.
+// g_i = dH/dp_i; rows whose softmax is NaN (no legal action, all legal logits -inf, a legal NaN or +inf logit) fall
+// back to the uniform distribution with zero gradient.
 __device__ __forceinline__ float ent_g(float p, float eps) {  // dH/dp for H = -sum p log(clamp(p))
   if (p < eps) return -logf(eps);
   if (p > 1.0f - eps) return -logf(1.0f - eps);
@@ -462,7 +467,7 @@ __global__ void __launch_bounds__(256, 4) kz_eval_fwd_kernel(const void* logits,
   LegalList ll{s_list[threadIdx.x >> 5], 0, false};
   const int A = KZ_NUM_ACTIONS;
   const float eps = FLT_EPSILON;
-  float m = -INFINITY, s = 0.f;
+  float m = -FLT_MAX, s = 0.f;  // non-finite logits as in kz_sample_kernel's pass 1
   each_legal_of_row(W, lane, ll, [&](int i) {
     const float x = ld_logit(lrow, i, bf16);
     if (x > m) { s = s * expf(m - x) + 1.f; m = x; }
@@ -472,12 +477,14 @@ __global__ void __launch_bounds__(256, 4) kz_eval_fwd_kernel(const void* logits,
 #pragma unroll
   for (int o = 16; o; o >>= 1) M = fmaxf(M, __shfl_xor_sync(FULL, M, o));
   float lp, ent, Z = 0.f, S = 0.f;
-  if (!(M > -INFINITY)) {  // NaN softmax -> uniform (base_actor_critic.py:166-174); constant, so no gradient
+  if (!(M < INFINITY) || __any_sync(FULL, isnan(s)) || !__any_sync(FULL, s > 0.f)) {
+    // NaN softmax (a legal +inf or NaN logit, all legal logits -inf, no legal entry) -> uniform
+    // (base_actor_critic.py:166-174); constant, so no gradient
     lp = logf(1.0f / (float)A);
     ent = -lp;
     M = INFINITY;  // marks the row for the backward pass
   } else {
-    float z = (m > -INFINITY) ? s * expf(m - M) : 0.f;
+    float z = s * expf(m - M);
 #pragma unroll
     for (int o = 16; o; o >>= 1) z += __shfl_xor_sync(FULL, z, o);
     Z = z;

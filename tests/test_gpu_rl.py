@@ -348,28 +348,42 @@ def test_fused_ppo_loss_matches_torch(n):
         assert torch.allclose(a, t.grad, rtol=1e-5, atol=1e-9), float((a - t.grad).abs().max())
 
 
-@pytest.mark.parametrize("weight_decay,max_norm", [(0.0, 0.5), (0.01, 0.5), (0.0, 1e9)])
-def test_fused_clip_adam_matches_torch(weight_decay, max_norm):
+_ADAM_SHAPES = [(1353, 129), (16, 46, 3, 3), (4096,), (7,), (1,), (3, 4099), (32, 24, 3, 3)]
+# 40 non-empty tensors = three launch groups of 16 / 16 / 8 (numel around the 4,096-element per-CTA chunk), plus a
+# zero-element tensor (left out of the groups) and, last, a parameter that gets no gradient
+_ADAM_GROUPS = [(4095,), (4096,), (4097,), (0,)] + [(37 * k + 1,) for k in range(30)] + \
+    [(64, 65), (4095,), (4097,), (3, 4096), (5, 7), (1,), (4096, 2)]
+
+
+@pytest.mark.parametrize("weight_decay,max_norm,shapes,no_grad", [
+    pytest.param(0.0, 0.5, _ADAM_SHAPES, False, id="0.0-0.5"),
+    pytest.param(0.01, 0.5, _ADAM_SHAPES, False, id="0.01-0.5"),
+    pytest.param(0.0, 1e9, _ADAM_SHAPES, False, id="0.0-1000000000.0"),
+    pytest.param(0.01, 0.5, _ADAM_GROUPS, True, id="three_groups"),
+])
+def test_fused_clip_adam_matches_torch(weight_decay, max_norm, shapes, no_grad):
     """kz_adam_clip_step against torch.nn.utils.clip_grad_norm_ + torch.optim.Adam(capturable) (ppo_agent.py:405-413)
-    over several steps on tensors of ragged sizes (vector body, scalar tails, a 1-element tensor): parameters,
-    both moments, the step counters and the reported gradient norm.  fp32 tolerance 1e-5 relative."""
+    over several steps on tensors of ragged sizes (vector body, scalar tails, a 1-element tensor; or several launch
+    groups with an empty tensor and one without a gradient): parameters, both moments, the step counters and the
+    reported gradient norm.  fp32 tolerance 1e-5 relative."""
     from shogidrl_b200 import rl
     dev = torch.device("cuda:0")
     g = torch.Generator(device="cpu").manual_seed(5)
-    shapes = [(1353, 129), (16, 46, 3, 3), (4096,), (7,), (1,), (3, 4099), (32, 24, 3, 3)]
+    shapes = shapes + [(300,)] if no_grad else shapes
     base = [torch.randn(s, generator=g) for s in shapes]
     pa = [torch.nn.Parameter(b.clone().to(dev)) for b in base]
     pb = [torch.nn.Parameter(b.clone().to(dev)) for b in base]
     # the last tensor lives in channels_last memory (the ResNet tower's convolution weights) and gets default-layout
     # gradients: the fused tail pairs elements by their logical index, not by their position in the storage
-    pa[-1].data = pa[-1].data.contiguous(memory_format=torch.channels_last)
-    assert not pa[-1].is_contiguous()
+    if len(shapes[-1]) == 4:
+        pa[-1].data = pa[-1].data.contiguous(memory_format=torch.channels_last)
+        assert not pa[-1].is_contiguous()
     kw = dict(lr=3e-4, weight_decay=weight_decay, capturable=True)
     oa, ob = torch.optim.Adam(pa, **kw), torch.optim.Adam(pb, **kw)
     assert rl.adam_clip_applicable(oa)
     for it in range(6):
         grads = [torch.randn(s, generator=g) * (10.0 if it % 2 else 0.01) for s in shapes]  # clipped and unclipped steps
-        for p, q, gr in zip(pa, pb, grads):
+        for p, q, gr in zip(pa[:len(pa) - no_grad], pb, grads):
             p.grad = gr.clone().to(dev)
             q.grad = gr.clone().to(dev)
         gn_a = rl.adam_clip_step(oa, max_norm)
@@ -378,6 +392,9 @@ def test_fused_clip_adam_matches_torch(weight_decay, max_norm):
         assert torch.allclose(gn_a, gn_b, rtol=1e-5), (float(gn_a), float(gn_b))
         for p, q in zip(pa, pb):
             assert torch.allclose(p, q, rtol=1e-5, atol=1e-7), (it, tuple(p.shape), float((p - q).abs().max()))
+            if p.grad is None:
+                assert len(oa.state[p]) == len(ob.state[q]) == 0 and torch.equal(p, q)
+                continue
             sa, sb = oa.state[p], ob.state[q]
             assert float(sa["step"]) == float(sb["step"]) == it + 1
             assert torch.allclose(sa["exp_avg"], sb["exp_avg"], rtol=1e-5, atol=1e-9)
