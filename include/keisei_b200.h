@@ -221,6 +221,16 @@ int kz_expand(const void* state, int n, int hist_cap, int counter_slot, const in
               int actions_i64, int m, float* obs, int64_t obs_stride, uint32_t* bitmap, int64_t bitmap_stride_words,
               uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner, int32_t* ep_len,
               int32_t* legal_count, uint8_t* err, void* child_state, int child_hist_cap, void* stream);
+/* Legal moves that give check: out row g = the legal-bitmap row g (input, kz_legal_bitmap's row of the current position)
+ * ANDed with "after this move the side that did not move is in check" (is_in_check, shogi_rules_logic.py:36-67, with the
+ * reference's "a missing king counts as in check": with the enemy king missing every legal move checks).  Reads the
+ * board, side to move and status from the state.  The row is exact whenever the side NOT to move is not already in check,
+ * which holds for every position reached by play; a loaded position in which it is gets ALL its legal moves (a superset:
+ * callers that decide mates by kz_expand stay exact).  Pad bits 13527..13535 and words 423.. of each out row are zero.  A
+ * finished game (status != 0) gets an empty row and count 0.  count (int32 [n], popcount of each out row) may be NULL.
+ * Strides in 32-bit words, >= KZ_BITMAP_WORDS_MIN; bitmap and out 16-byte aligned; out must not overlap bitmap. */
+int kz_check_bitmap(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words, uint32_t* out,
+                    int64_t out_stride_words, int32_t* count, void* stream);
 
 /* Thin conveniences over kz_refresh. */
 int kz_legal_mask(void* state, int n, int hist_cap, uint8_t* mask, int64_t mask_stride,

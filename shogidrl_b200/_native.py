@@ -18,6 +18,8 @@ OBS_FLOATS = 46 * 81
 MASK_PAD_STRIDE = 13536
 BITMAP_WORDS = 448
 REASONS = {0: None, 1: "Tsumi", 2: "stalemate", 3: "Max moves reached", 4: "Sennichite"}
+TSUMI = 1  # KZ_TSUMI
+ERR_KING_CAPTURE = 4  # KZ_ERR_KING_CAPTURE
 
 EXPORTS = [
     "kz_abi_version", "kz_last_cuda_error", "kz_build_info", "kz_init_tables", "kz_state_layout", "kz_reset", "kz_load_positions",
@@ -27,7 +29,7 @@ EXPORTS = [
     "kz_step_rollout", "kz_legal_bitmap", "kz_bitmap_expand", "kz_sample_bitmap",
     "kz_eval_bitmap_fwd", "kz_eval_bitmap_bwd", "kz_step_range", "kz_cobs_conv_fwd", "kz_cobs_conv_wgrad_ctas",
     "kz_cobs_conv_wgrad", "kz_heuristic_actions", "kz_pool_records", "kz_step_pool", "kz_reset_pool", "kz_legal_list",
-    "kz_expand",
+    "kz_expand", "kz_check_bitmap",
 ]
 COBS_WORDS = 40
 POOL_RECORD_WORDS = 512
@@ -81,6 +83,7 @@ def lib() -> C.CDLL:
     L.kz_reset_pool.argtypes = [vp, i32, i32, vp, i32, vp, i32, vp, u64, u32, vp, vp]
     L.kz_legal_list.argtypes = [vp, i64, i32, vp, vp, vp, i32, vp]
     L.kz_expand.argtypes = [vp, i32, i32, i32, vp, vp, i32, i32, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]
+    L.kz_check_bitmap.argtypes = [vp, i32, i32, vp, i64, vp, i64, vp, vp]
     L.kz_legal_mask.argtypes = [vp, i32, i32, vp, i64, vp, vp]
     L.kz_observe.argtypes = [vp, i32, i32, vp, i64, vp]
     L.kz_errors.argtypes = [vp, i32, i32, vp, i32, vp]

@@ -1424,6 +1424,156 @@ __global__ void __launch_bounds__(256) kz_legal_list_kernel(const uint32_t* __re
 }
 
 // ------------------------------------------------------------------------------------------------
+// Legal moves that give check (kz_check_bitmap), one warp per game, games in a grid-stride loop.  Built per game from the
+// enemy king's square KE at the current occupancy:
+//   check squares cs[t]: the squares from which a piece of the mover's type t attacks KE -- the targets from KE of the
+//     ENEMY's piece of type t (reverse step pattern; sliders up to and including the first blocker), one lane per type;
+//   discovered-check lines: lane d walks ray d from KE; an own first piece followed by an own slider that attacks KE along
+//     that ray makes the first piece a candidate, and seg[d] is the squares strictly between KE and the slider.
+// A board move from -> to checks if `to` is in the check squares of the piece's type after the move (promoted type for the
+// odd bits), or if from is a candidate and to leaves seg[d]; a drop of type t on `to` checks if `to` is in cs[t].  The
+// check squares are taken at the occupancy before the move; the only square that changes and could lie between `to`
+// and KE is `from`, and then the piece moves along that line away from KE, so it already attacked KE from `from` (no
+// promotion adds a slide direction) -- the enemy was in check, which is the out-of-contract case below.
+// Row = legal row AND that set.  Finished game: empty row.  Enemy king missing, or already attacked (loaded positions
+// only): the whole legal row.
+struct CheckScratch {
+  uint32_t cs[14][3];  // check squares per piece type of the mover (bitboards)
+  uint32_t seg[8][3];  // discovered-check line d: squares strictly between KE and the own slider
+  uint8_t board[96];
+  uint8_t disc[96];    // direction of the line a discovered-check candidate blocks, 0xFF none
+  uint8_t dchk[96];    // bit t: a drop of type t on this square gives check
+};
+
+__device__ __forceinline__ uint32_t bits17(const uint32_t (&b)[3], int lo) {  // bits lo .. lo + 16 of a bitboard (lo <= 64)
+  const int wd = lo >> 5;
+  const uint32_t a = wd == 0 ? b[0] : (wd == 1 ? b[1] : b[2]);
+  const uint32_t c = wd == 0 ? b[1] : (wd == 1 ? b[2] : 0u);
+  return __funnelshift_r(a, c, lo & 31) & 0x1FFFFu;
+}
+
+__global__ void __launch_bounds__(256) kz_check_bitmap_kernel(const uint8_t* __restrict__ boards,
+                                                              const uint8_t* __restrict__ meta, int n,
+                                                              const uint32_t* __restrict__ bitmap, long long ldb,
+                                                              uint32_t* __restrict__ out, long long ldo, int32_t* count) {
+  __shared__ CheckScratch s_chk[8];
+  for (int i = threadIdx.x; i < 81 * 8 * 3; i += blockDim.x) s_ray[i] = g_ray[i];
+  for (int i = threadIdx.x; i < NCLS * 81 * 3; i += blockDim.x) s_step[i] = g_step[i];
+  __syncthreads();
+  const Tables T{};
+  const int lane = threadIdx.x & 31;
+  CheckScratch& S = s_chk[threadIdx.x >> 5];
+  const uint32_t tab = code_info(lane);
+  for (int g = blockIdx.x * 8 + (threadIdx.x >> 5); g < n; g += gridDim.x * 8) {  // warp-uniform
+    __syncwarp();
+    if (lane < 24) reinterpret_cast<uint32_t*>(S.board)[lane] = reinterpret_cast<const uint32_t*>(boards + (size_t)g * 96)[lane];
+    const int me = meta[(size_t)g * 32 + 14], status = meta[(size_t)g * 32 + 15];
+    __syncwarp();
+    int c[3];
+    uint32_t o[3], ek[3];
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+      c[j] = lane + 32 * j < 81 ? S.board[lane + 32 * j] : 0;
+      o[j] = __ballot_sync(FULL, c[j] != 0);
+      ek[j] = __ballot_sync(FULL, c[j] == 8 + 14 * (1 - me));
+      S.disc[lane + 32 * j] = 0xFF;
+    }
+    __syncwarp();
+    const BB occ{o[0], o[1], o[2]};
+    const int KE = (ek[0] | ek[1] | ek[2]) ? bb_lsb(BB{ek[0], ek[1], ek[2]}) : -1;  // find_king: first in row-major order
+    int mode = status != 0 ? 0 : (KE < 0 ? 1 : 2);  // 0 empty row, 1 every legal move, 2 checking moves
+    if (mode == 2) {
+      {  // check squares: lane t < 14 = the targets from KE of the enemy's piece of type t
+        const uint32_t inf = __shfl_sync(FULL, tab, lane < 14 ? 1 + lane + 14 * (1 - me) : 0);
+        if (lane < 14) {
+          BB t = ld_step(T, (inf >> 16) & 15, KE);
+          uint32_t sl = (inf >> 8) & 0xFF;
+          while (sl) {
+            const int d = __ffs(sl) - 1;
+            sl &= sl - 1;
+            t = t | slide_ray(T, KE, d, occ);
+          }
+          S.cs[lane][0] = t.w0; S.cs[lane][1] = t.w1; S.cs[lane][2] = t.w2;
+        }
+      }
+      {  // discovered-check candidates on the eight rays from KE
+        const int d = lane & 7, od = (d + 4) & 7;
+        const BB ray = ld_ray(T, KE, d);
+        const BB bl = ray & occ;
+        const bool pos = dir_positive(d);
+        int b1 = -1, b2 = -1;
+        if (bb_any(bl)) {
+          b1 = pos ? bb_lsb(bl) : bb_msb(bl);
+          const BB bl2 = bb_andn(bl, bb_bit(b1));
+          if (bb_any(bl2)) b2 = pos ? bb_lsb(bl2) : bb_msb(bl2);
+        }
+        const int code1 = b1 >= 0 ? S.board[b1] : 0, code2 = b2 >= 0 ? S.board[b2] : 0;
+        const uint32_t inf2 = __shfl_sync(FULL, tab, code2);
+        if (lane < 8 && code1 && code_color(code1) == me && code2 && code_color(code2) == me && ((inf2 >> (8 + od)) & 1)) {
+          const BB seg = pos ? (ray & bb_below(b2)) : bb_andn(ray, bb_upto(b2));
+          S.disc[b1] = (uint8_t)d;
+          S.seg[d][0] = seg.w0; S.seg[d][1] = seg.w1; S.seg[d][2] = seg.w2;
+        }
+      }
+      __syncwarp();
+      bool attacks = false;  // an own piece already attacks KE: the side not to move is in check
+#pragma unroll
+      for (int j = 0; j < 3; j++) {
+        const int sq = lane + 32 * j;
+        if (sq < 81 && c[j] && code_color(c[j]) == me) attacks |= (S.cs[code_type(c[j])][j] >> lane) & 1;
+        if (sq < 96) {
+          uint32_t v = 0;
+#pragma unroll
+          for (int t = 0; t < 7; t++) v |= (sq < 81 ? (S.cs[t][j] >> lane) & 1 : 0u) << t;
+          S.dchk[sq] = (uint8_t)v;
+        }
+      }
+      if (__any_sync(FULL, attacks)) mode = 1;
+      __syncwarp();
+    }
+    const uint32_t* src = bitmap + (size_t)g * ldb;
+    uint32_t* dst = out + (size_t)g * ldo;
+    int cnt = 0;
+    for (int wi = lane; wi < KZ_BITMAP_WORDS_MIN; wi += 32) {
+      uint32_t v = mode ? __ldg(src + wi) : 0u;
+      if (wi == KZ_BITMAP_WORDS_MIN - 1) v &= (1u << (KZ_NUM_ACTIONS - 32 * (KZ_BITMAP_WORDS_MIN - 1))) - 1u;
+      if (mode == 2 && v) {
+        uint32_t chk;
+        if (wi < 405) {  // board moves: source square wi / 5, targets to' = lo .. lo + 15 (to = to' + (to' >= from))
+          const int from = wi / 5, lo = 16 * (wi - 5 * from);
+          const int t = code_type(S.board[from]);
+          const int tp = (t <= 3 || t == 5 || t == 6) ? t + promo_delta(t) : t;  // odd bits exist only for promotable types
+          const uint32_t below = lowmask32(from - lo);
+          auto compact = [&](uint32_t x) { return ((x & below) | ((x >> 1) & ~below)) & 0xFFFFu; };
+          chk = spread16(compact(bits17(S.cs[t], lo))) | (spread16(compact(bits17(S.cs[tp], lo))) << 1);
+          const int dd = S.disc[from];
+          if (dd != 0xFF) chk |= spread16(~compact(bits17(S.seg[dd], lo)) & 0xFFFFu) * 3u;
+        } else {  // drops: word 405 + q holds drop-stream bits [32q, 32q + 32) (as gen_moves packs them)
+          const int q = wi - 405;
+          const int to0 = (32 * q * 293) >> 11;  // floor(32q / 7)
+          int p = 7 * to0 - 32 * q;             // <= 0
+          chk = 0;
+#pragma unroll
+          for (int i = 0; i < 6; i++) {
+            const int to = to0 + i;
+            const uint32_t dv = to < 81 ? S.dchk[to] : 0;
+            if (p >= 0) { if (p < 32) chk |= dv << p; }
+            else chk |= dv >> (-p);
+            p += 7;
+          }
+        }
+        v &= chk;
+      }
+      dst[wi] = v;
+      cnt += __popc(v);
+    }
+    for (long long wi = KZ_BITMAP_WORDS_MIN + lane; wi < ldo; wi += 32) dst[wi] = 0u;
+    cnt = (int)__reduce_add_sync(FULL, (unsigned)cnt);
+    if (count && lane == 0) count[g] = cnt;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 __global__ void kz_reset_kernel(uint8_t* boards, uint8_t* meta, uint4* rep, int rep_slots, int n,
                                 const uint8_t* env_mask, int max_moves) {
   const int g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -2048,6 +2198,26 @@ int kz_expand(const void* state, int n, int hist_cap, int counter_slot, const in
     P.child_rep_slots = C.rep_slots;
   }
   return launch_kernel(P, sched, counter_slot, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int kz_check_bitmap(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words, uint32_t* out,
+                    int64_t out_stride_words, int32_t* count, void* stream) {
+  if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535 || !bitmap || !out || bitmap_stride_words < KZ_BITMAP_WORDS_MIN ||
+      out_stride_words < KZ_BITMAP_WORDS_MIN || ((uintptr_t)state & 255) || ((uintptr_t)bitmap & 15) || ((uintptr_t)out & 15) ||
+      ((uintptr_t)count & 3))
+    return KZ_E_ARG;
+  const uintptr_t b0 = (uintptr_t)bitmap, b1 = b0 + (uintptr_t)n * (uintptr_t)bitmap_stride_words * 4u;
+  const uintptr_t o0 = (uintptr_t)out, o1 = o0 + (uintptr_t)n * (uintptr_t)out_stride_words * 4u;
+  if (o0 < b1 && b0 < o1) return KZ_E_ARG;  // out overlaps bitmap
+  if (!host_ready()) return KZ_E_NOT_INIT;
+  const Layout L = layout(n, hist_cap);
+  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
+  int grid = sm_count() * 8;  // 8 CTAs of 8 warps per SM (24 KB of static shared memory each)
+  if (grid > (n + 7) / 8) grid = (n + 7) / 8;
+  kz_check_bitmap_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      base + L.off_boards, base + L.off_meta, n, bitmap, bitmap_stride_words, out, out_stride_words, count);
+  CK(cudaGetLastError());
+  return KZ_OK;
 }
 
 }  // extern "C"

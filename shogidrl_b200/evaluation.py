@@ -16,6 +16,7 @@ from typing import Any, Dict, List, Mapping, Optional, Sequence, Tuple
 
 import torch
 
+from . import _native as nv
 from .utils.opponents import BaseOpponent, SimpleHeuristicOpponent, SimpleRandomOpponent
 from .vec_env import VecShogiEnv
 
@@ -155,6 +156,99 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
             outcomes.extend(OUTCOMES[c] for c in stats[4: 4 + stats[0]])
             start_ids.extend(stats[4 + stats[0]:])
     return EvaluationResult(done_games, agent_w, opp_w, draws, length_sum / max(1, done_games), outcomes, start_ids)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# Mate in one: can a player see a mate that is there?  Positions with a mate in one are harvested from random play on the
+# device (no external tsume collection needed); a player's move solves a position when its expansion ends the game by
+# Tsumi.
+
+@dataclass
+class MateInOneResult:
+    positions: int  # positions evaluated
+    with_mate: int  # positions that have a mate in one (only these count toward the rate)
+    solved: int  # positions whose move by the player mates
+    solved_flags: List[bool] = field(default_factory=list)  # per position: the player's move mates
+    mate_flags: List[bool] = field(default_factory=list)  # per position: a mate in one exists
+
+    @property
+    def solve_rate(self) -> float:
+        return self.solved / max(1, self.with_mate)
+
+
+def harvest_mate_in_one(num_positions: int, *, seed: int = 0, num_envs: int = 1024, max_moves_per_game: int = 500,
+                        device="cuda", max_steps: Optional[int] = None) -> List[str]:
+    """SFENs of ``num_positions`` positions that have a mate in one, collected from uniform-random self-play on the
+    device: after every step, the positions of the envs whose ``mate_in_one().count >= 1`` are kept, in env order, until
+    there are enough.  Deterministic for a seed.  Stops after ``max_steps`` steps (default 100 x max_moves_per_game) with
+    what it has."""
+    if num_positions < 0 or num_envs < 1:
+        raise ValueError(f"num_positions = {num_positions}, num_envs = {num_envs}: need num_positions >= 0 and num_envs >= 1")
+    env = VecShogiEnv(num_envs, max_moves_per_game=max_moves_per_game, device=device, seed=seed, auto_reset=True)
+    env.refresh(random_actions=True)
+    acts = [env.next_actions.clone(), torch.empty_like(env.next_actions)]
+    out: List[str] = []
+    limit = max_steps if max_steps is not None else 100 * max_moves_per_game
+    for i in range(limit):
+        if len(out) >= num_positions:
+            break
+        env.step(acts[i % 2], next_out=acts[(i + 1) % 2], random_actions=True)
+        ids = torch.nonzero(env.mate_in_one()["count"] > 0).flatten().tolist()
+        if ids:
+            out.extend(env.to_sfen(ids[: num_positions - len(out)]))
+    return out
+
+
+def mate_batches(num_positions: int, num_envs: int) -> List[Tuple[int, int, int]]:
+    """Host batching of evaluate_mate_in_one: -> [(first, count, n)] with n = min(num_envs, num_positions) envs per batch;
+    batch b evaluates positions [first, first + count) and pads its last n - count envs (the last batch only) with
+    copies of its first position, whose results are dropped."""
+    if num_envs < 1:
+        raise ValueError(f"num_envs = {num_envs}: need num_envs >= 1")
+    n = min(num_envs, num_positions)
+    return [(f, min(n, num_positions - f), n) for f in range(0, num_positions, n)] if n > 0 else []
+
+
+def evaluate_mate_in_one(player, positions: Sequence[str], *, num_envs: int = 1024, device="cuda", seed: int = 0,
+                         deterministic: bool = True) -> MateInOneResult:
+    """Mate-in-one score of ``player`` on ``positions`` (SFEN strings, e.g. from harvest_mate_in_one): the player is an
+    agent (``select_actions(obs, mask)``), ``"random"`` or ``"heuristic"``, as in evaluate_vs_opponent.  The positions are
+    loaded in batches of ``num_envs`` (``load_sfens``, the last batch padded), the player picks one move per position, and
+    the move solves the position when ``expand`` ends the game by Tsumi without capturing a king.  Positions without a
+    mate in one (``mate_in_one``) do not count toward the rate.  The random player's move on position i is the engine's
+    fused uniform-random legal action keyed (seed, i, step 0); the heuristic player's draw is keyed the same way
+    (with its own salt, as ``heuristic_actions``)."""
+    kind = _player_kind(player)
+    positions = [str(s) for s in positions]
+    batches = mate_batches(len(positions), num_envs)
+    solved_flags: List[bool] = []
+    mate_flags: List[bool] = []
+    if not batches:
+        return MateInOneResult(0, 0, 0)
+    n = batches[0][2]
+    # max_moves 65535: a harvested position keeps its move number, which must not end the game at load; history is not
+    # needed (a mate does not depend on it), so one repetition slot per game suffices
+    env = VecShogiEnv(n, max_moves_per_game=65535, device=device, seed=seed, auto_reset=False, hist_cap=1)
+    ids = torch.arange(n, dtype=torch.int32, device=env.device)
+    for first, count, _ in batches:
+        batch = positions[first:first + count]
+        env.env_offset = first  # position i draws from the random stream of index i
+        env.load_sfens(batch + [batch[0]] * (n - count))
+        if kind == "random":
+            env.refresh(random_actions=True)
+            actions = env.next_actions.clone()
+        elif kind == "heuristic":
+            actions = env.heuristic_actions()
+        else:
+            actions = player.select_actions(env.obs, env.mask, is_training=not deterministic)[0]
+            actions = actions.to(device=env.device, dtype=torch.int64).contiguous()
+        out = env.expand(ids, actions)
+        solved = (out["reason"] == nv.TSUMI) & ((out["err"] & nv.ERR_KING_CAPTURE) == 0)
+        has = env.mate_in_one()["count"] > 0
+        flags = torch.stack([solved, has]).cpu().tolist()
+        solved_flags.extend(bool(x) for x in flags[0][:count])
+        mate_flags.extend(bool(x) for x in flags[1][:count])
+    return MateInOneResult(len(positions), sum(mate_flags), sum(solved_flags), solved_flags, mate_flags)
 
 
 # ---------------------------------------------------------------------------------------------------------------

@@ -393,6 +393,67 @@ class VecShogiEnv:
                                    self._sp()), "kz_expand")
         return out
 
+    def check_bitmap(self, bitmap: torch.Tensor, out: Optional[torch.Tensor] = None):
+        """The legal moves of every env's CURRENT position that give check (kz_check_bitmap): ``bitmap`` holds the legal
+        rows (int32 [n, 448], as ``legal_bitmap`` writes them) -> (out rows of the checking moves, count int32 [n]).
+        ``out`` (default: new rows) must not overlap ``bitmap``.  Exact for positions in which the side not to move is
+        not in check (every position reached by play); a loaded position in which it is gets all its legal moves.
+        Finished games get an empty row."""
+        bp, bs = self._bitmap_args(bitmap)
+        if out is None:
+            out = torch.empty((self.n, nv.BITMAP_WORDS), dtype=torch.int32, device=self.device)
+        op, os_ = self._bitmap_args(out)
+        count = torch.empty(self.n, dtype=torch.int32, device=self.device)
+        nv.check(self._L.kz_check_bitmap(self.state.data_ptr(), self.n, self.hist_cap, bp, bs, op, os_, count.data_ptr(),
+                                         self._sp()), "kz_check_bitmap")
+        return out, count
+
+    def checking_actions(self):
+        """Every legal move that gives check, of every env's CURRENT position, in ``legal_actions``' CSR form: ->
+        (offsets int64 [n+1], parent int32 [M], actions int64 [M]).  kz_legal_bitmap, kz_check_bitmap, then kz_legal_list
+        on the check rows; one host read (of M)."""
+        d, sp = self.device, self._sp()
+        bitmap = torch.empty((self.n, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
+        count = torch.empty(self.n, dtype=torch.int32, device=d)
+        nv.check(self._L.kz_legal_bitmap(self.state.data_ptr(), self.n, self.hist_cap, None, 0, bitmap.data_ptr(),
+                                         nv.BITMAP_WORDS, None, count.data_ptr(), sp), "kz_legal_bitmap")
+        rows, count = self.check_bitmap(bitmap)
+        offsets = torch.zeros(self.n + 1, dtype=torch.int64, device=d)
+        offsets[1:] = torch.cumsum(count, 0, dtype=torch.int64)
+        m = int(offsets[-1])
+        parent = torch.empty(m, dtype=torch.int32, device=d)
+        actions = torch.empty(m, dtype=torch.int64, device=d)
+        if m > 0:  # empty tensors have no storage to hand to kz_legal_list
+            nv.check(self._L.kz_legal_list(rows.data_ptr(), nv.BITMAP_WORDS, self.n, offsets.data_ptr(), parent.data_ptr(),
+                                           actions.data_ptr(), 1, sp), "kz_legal_list")
+        return offsets, parent, actions
+
+    def mate_in_one(self) -> Dict[str, torch.Tensor]:
+        """Mates in one of every env's CURRENT position: -> {"action": int64 [n] the lowest-index mating move (-1: none),
+        "count": int32 [n] the number of mating moves}.  A mate must give check, so only ``checking_actions`` are
+        expanded (``expand``); a move mates when its expansion ends the game by Tsumi without capturing a king (capturing
+        a king is outside the engine's contract, as in ``step``).  No env moves."""
+        _, parent, actions = self.checking_actions()
+        d = self.device
+        count = torch.zeros(self.n, dtype=torch.int32, device=d)
+        action = torch.full((self.n,), -1, dtype=torch.int64, device=d)
+        if parent.numel() == 0:
+            return {"action": action, "count": count}
+        m = int(parent.numel())
+        reason = torch.empty(m, dtype=torch.uint8, device=d)
+        err = torch.empty(m, dtype=torch.uint8, device=d)
+        # kz_expand directly rather than expand(): the parents come from kz_legal_list and need no host-side check
+        nv.check(self._L.kz_expand(self.state.data_ptr(), self.n, self.hist_cap, 0, parent.data_ptr(), actions.data_ptr(), 1,
+                                   m, None, 0, None, 0, None, None, None, reason.data_ptr(), None, None, None,
+                                   err.data_ptr(), None, 0, self._sp()), "kz_expand")
+        mate = (reason == nv.TSUMI) & ((err & nv.ERR_KING_CAPTURE) == 0)
+        p = parent.long()
+        count.index_add_(0, p, mate.to(torch.int32))
+        first = torch.full((self.n,), nv.NUM_ACTIONS, dtype=torch.int64, device=d)
+        first.scatter_reduce_(0, p, torch.where(mate, actions, nv.NUM_ACTIONS), "amin")
+        action = torch.where(count > 0, first, action)
+        return {"action": action, "count": count}
+
     # The heuristic opponent draws from the env's random stream keyed by seed ^ HEURISTIC_SALT, so its pick is independent
     # of the fused uniform-random action (next_actions, keyed by the seed itself) drawn for the same step and env.
     HEURISTIC_SALT = 0x48657572697374  # "Heurist"
