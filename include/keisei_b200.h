@@ -280,6 +280,36 @@ int kz_heuristic_actions(const void* state, int n, int hist_cap, const uint8_t* 
                          const uint32_t* bitmap, int64_t bitmap_stride_words, void* actions, int actions_i64, uint8_t* tier,
                          int32_t* tier_count, uint64_t seed, uint32_t rng_step, uint32_t env_offset, void* stream);
 
+/* ---- one-ply look-ahead opponent.  Piece values by type (P L N S G B R K +P +L +N +S +B +R): 1 3 4 5 6 8 10 0 6 6 6 6 10 12.
+ * The GAIN of a move for the side making it: a board move onto a piece X of the other colour gains v(X) + v(unpromoted X)
+ * (X leaves the opponent's board and enters the mover's hand), a promoting move of a piece of type T adds
+ * v(promoted T) - v(T), and a drop gains 0.
+ * kz_capture_gain: for each of the n games of `state` (board, side to move and status read from it), gain[g] (int32) = the
+ * largest gain over the legal moves of bitmap row g (kz_legal_bitmap's or kz_expand's row of the current position; stride
+ * in words >= KZ_BITMAP_WORDS_MIN, 4-byte aligned; pad bits 13527.. and words 423.. are ignored), and count[g] (int32,
+ * optional) = the number of those moves that reach it.  A finished game (status != 0) and a row without moves get 0 and 0.
+ * Rows are addressed in 64 bits.  state 256-byte aligned.  Needs no tables. */
+int kz_capture_gain(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words, int32_t* gain,
+                    int32_t* count, void* stream);
+/* kz_lookahead_select: the look-ahead opponent's move for each of the n games of `state`.  Game g's items are
+ * [offsets[g], offsets[g+1]) of the m items (offsets int64 [n+1]; each value is clamped to [0, m] and a range whose end is
+ * below its start is empty, so no offsets value makes the kernel read outside the m items); they are game g's moves in
+ * ascending action order, as kz_legal_list writes them (actions int64 if actions_i64 else int32), with for each item i:
+ *   done / reason / err (u8): kz_expand's outputs for the move on game g (its history included),
+ *   reply_gain (int32): R of the successor C, kz_capture_gain of C's row (0 if C is finished or has no legal move),
+ *   reply_mates (int32): the number of legal replies in C that end the game by Tsumi without KZ_ERR_KING_CAPTURE.
+ * The SCORE of item i, by the first rule that applies: 1,000,000 if the move ends the game by Tsumi without
+ * KZ_ERR_KING_CAPTURE; gain if it ends the game in any other way; -1,000,000 if reply_mates > 0; gain - reply_gain
+ * otherwise (gain decoded from game g's board and the action: from*160 + 2*to' + promote for board moves, >= 12960 drops).
+ * The pick is the k-th of the items with the maximum score in item order, k = mulhi(rand32(seed, env_offset + g, rng_step),
+ * ties): kz_heuristic_actions' convention.  actions_out (int64 if out_i64 else int32) gets the pick, score (int32,
+ * optional) the maximum score and ties (int32, optional) the number of items reaching it; a finished game (status != 0)
+ * or one without items gets -1, 0 and 0.  With m == 0 the per-item pointers may be NULL.  Needs no tables. */
+int kz_lookahead_select(const void* state, int n, int hist_cap, const int64_t* offsets, int64_t m, const void* actions,
+                        int actions_i64, const uint8_t* done, const uint8_t* reason, const uint8_t* err,
+                        const int32_t* reply_gain, const int32_t* reply_mates, uint64_t seed, uint32_t rng_step,
+                        uint32_t env_offset, void* actions_out, int out_i64, int32_t* score, int32_t* ties, void* stream);
+
 /* ExperienceBuffer.compute_advantages_and_returns (experience_buffer.py:99-145) over a [T][N]
  * layout, one reverse scan per env column (N = 1 is the reference's flat buffer):
  *   delta = (r + (gamma * nv) * m) - V ;  gae = delta + (gamma_lambda * m) * gae   (no FMA)

@@ -29,7 +29,7 @@ EXPORTS = [
     "kz_step_rollout", "kz_legal_bitmap", "kz_bitmap_expand", "kz_sample_bitmap",
     "kz_eval_bitmap_fwd", "kz_eval_bitmap_bwd", "kz_step_range", "kz_cobs_conv_fwd", "kz_cobs_conv_wgrad_ctas",
     "kz_cobs_conv_wgrad", "kz_heuristic_actions", "kz_pool_records", "kz_step_pool", "kz_reset_pool", "kz_legal_list",
-    "kz_expand", "kz_check_bitmap",
+    "kz_expand", "kz_check_bitmap", "kz_capture_gain", "kz_lookahead_select",
 ]
 COBS_WORDS = 40
 POOL_RECORD_WORDS = 512
@@ -84,6 +84,8 @@ def lib() -> C.CDLL:
     L.kz_legal_list.argtypes = [vp, i64, i32, vp, vp, vp, i32, vp]
     L.kz_expand.argtypes = [vp, i32, i32, i32, vp, vp, i32, i32, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]
     L.kz_check_bitmap.argtypes = [vp, i32, i32, vp, i64, vp, i64, vp, vp]
+    L.kz_capture_gain.argtypes = [vp, i32, i32, vp, i64, vp, vp, vp]
+    L.kz_lookahead_select.argtypes = [vp, i32, i32, vp, i64, vp, i32, vp, vp, vp, vp, vp, u64, u32, u32, vp, i32, vp, vp, vp]
     L.kz_legal_mask.argtypes = [vp, i32, i32, vp, i64, vp, vp]
     L.kz_observe.argtypes = [vp, i32, i32, vp, i64, vp]
     L.kz_errors.argtypes = [vp, i32, i32, vp, i32, vp]

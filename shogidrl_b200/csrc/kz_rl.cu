@@ -3,6 +3,7 @@
 //                      (keisei/core/base_actor_critic.py:64-116; torch.distributions.Categorical(probs=...))
 //   kz_gae           : reverse-time GAE over a [T][N] rollout (keisei/core/experience_buffer.py:99-145)
 //   kz_heuristic_actions : the scripted SimpleHeuristicOpponent's move for every game (keisei/utils/opponents.py)
+//   kz_capture_gain / kz_lookahead_select : the one-ply look-ahead opponent's best reply gain and pick
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <float.h>
@@ -378,6 +379,157 @@ __global__ void __launch_bounds__(256) kz_heuristic_kernel(const uint8_t* __rest
   }
 }
 
+// ---- One-ply look-ahead opponent (kz_capture_gain, kz_lookahead_select), one warp per game ----
+// Piece values by type P L N S G B R K +P +L +N +S +B +R: 1 3 4 5 6 8 10 0 6 6 6 6 10 12.  A capture gains the captured
+// piece's value plus the value of its unpromoted type (it leaves the opponent's board and enters the mover's hand
+// unpromoted); a promotion gains the promoted type's value minus the piece's own.
+__constant__ int8_t c_cap_value[28] = {  // by board code 1..28 (index code - 1), either colour
+    2, 6, 8, 10, 12, 16, 20, 0, 7, 9, 10, 11, 18, 22, 2, 6, 8, 10, 12, 16, 20, 0, 7, 9, 10, 11, 18, 22};
+__constant__ int8_t c_promo_bonus[14] = {5, 3, 2, 1, 0, 2, 2, 0, 0, 0, 0, 0, 0, 0};  // by piece type
+
+#define LOOKAHEAD_MATE 1000000
+
+// (best, count) of the gains seen so far: count c moves of gain x
+__device__ __forceinline__ void gain_acc(int& best, int& cnt, int x, int c) {
+  if (c == 0) return;
+  if (x > best) { best = x; cnt = c; }
+  else if (x == best) cnt += c;
+}
+
+// R of each game: the largest gain over the legal moves of its bitmap row, and how many moves reach it.  Every gain is
+// >= 0, so (0, 0) is also the answer for a row without moves.  Board-move window A < 810 has one source square: its
+// quiet moves gain the source piece's promotion bonus on odd (promoting) bits and 0 on even ones; its capture bits (from
+// enemy occupancy: the heuristic's capture tier) each add the captured piece's value.  Drop windows gain 0.
+__global__ void __launch_bounds__(256) kz_capture_gain_kernel(const uint8_t* __restrict__ boards,
+                                                              const uint8_t* __restrict__ meta, int n,
+                                                              const uint32_t* __restrict__ legal, long long ldw,
+                                                              int32_t* __restrict__ gain_out, int32_t* __restrict__ count_out) {
+  const int lane = threadIdx.x & 31;
+  const int g = blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (g >= n) return;
+  const uint8_t* b = boards + (size_t)g * 96;
+  const int side = meta[(size_t)g * 32 + 14], status = meta[(size_t)g * 32 + 15];
+  int best = 0, cnt = 0;
+  if (status == 0) {
+    uint32_t e[3];
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+      const int s = lane + 32 * j;
+      const int c = s < 81 ? b[s] : 0;
+      e[j] = __ballot_sync(FULL, c != 0 && code_color(c) != side);
+    }
+    const BB enemy{e[0], e[1], e[2]}, none{0u, 0u, 0u};
+    const BitmapWindows W(legal + (long long)g * ldw);  // 64-bit row address: M x 448 words passes 2^31
+    for (int r = 0; r < HEUR_ROUNDS; r++) {
+      const int A = 32 * r + lane;
+      const uint32_t v = A < HEUR_WINDOWS ? W.load(A) : 0u;  // (pad bits and words 423.. are never read)
+      if (!v) continue;
+      if (A >= 810) { gain_acc(best, cnt, 0, __popc(v)); continue; }
+      const int from = A / 10;
+      uint32_t cap, pawn;
+      heur_classify(v, A, enemy, none, cap, pawn);  // the heuristic's capture tier
+      const int src = b[from];
+      const int pb = (src >= 1 && src <= 28) ? c_promo_bonus[code_type(src)] : 0;
+      gain_acc(best, cnt, 0, __popc(v & ~cap & 0x5555u));
+      gain_acc(best, cnt, pb, __popc(v & ~cap & 0xAAAAu));
+      for (uint32_t z = cap; z; z &= z - 1) {
+        const int j = __ffs(z) - 1;
+        const int tp = 8 * (A - 10 * from) + (j >> 1);
+        const int to = tp + (tp >= from);
+        gain_acc(best, cnt, c_cap_value[b[to] - 1] + ((j & 1) ? pb : 0), 1);
+      }
+    }
+    const int M = __reduce_max_sync(FULL, best);
+    cnt = (int)__reduce_add_sync(FULL, (unsigned)(best == M ? cnt : 0));
+    best = M;
+  }
+  if (lane == 0) {
+    gain_out[g] = best;
+    if (count_out) count_out[g] = cnt;
+  }
+}
+
+// gain of action a for `side` on board b; 0 for drops and for anything that is not a board move
+__device__ __forceinline__ int move_gain(const uint8_t* b, int side, long long a) {
+  if (a < 0 || a >= 12960) return 0;
+  const int pair = (int)(a >> 1), from = pair / 80, tp = pair - 80 * from, to = tp + (tp >= from);
+  const int dst = b[to], src = b[from];
+  int x = (dst >= 1 && dst <= 28 && code_color(dst) != side) ? c_cap_value[dst - 1] : 0;
+  if ((a & 1) && src >= 1 && src <= 28) x += c_promo_bonus[code_type(src)];
+  return x;
+}
+
+struct LookaheadItems {
+  const void* actions;
+  int actions_i64;
+  const uint8_t* done;
+  const uint8_t* reason;
+  const uint8_t* err;
+  const int32_t* reply_gain;
+  const int32_t* reply_mates;
+  __device__ __forceinline__ long long action(long long i) const {
+    return actions_i64 ? reinterpret_cast<const long long*>(actions)[i] : (long long)reinterpret_cast<const int*>(actions)[i];
+  }
+  // the look-ahead score of item i, the first rule that applies
+  __device__ __forceinline__ int score(const uint8_t* b, int side, long long i) const {
+    const int x = move_gain(b, side, action(i));
+    if (done[i]) return (reason[i] == KZ_TSUMI && !(err[i] & KZ_ERR_KING_CAPTURE)) ? LOOKAHEAD_MATE : x;
+    if (reply_mates[i] > 0) return -LOOKAHEAD_MATE;
+    return x - reply_gain[i];
+  }
+};
+
+// Game g's items [offsets[g], offsets[g+1]) (clamped to [0, m]; a range that is not monotone is empty): the maximum
+// score, the number of items reaching it, and the k-th of those in item order, k = mulhi(rand32(seed, env_offset + g,
+// rng_step), ties).  Items are in ascending action order, so item order is action order.
+__global__ void __launch_bounds__(256) kz_lookahead_select_kernel(const uint8_t* __restrict__ boards,
+                                                                  const uint8_t* __restrict__ meta, int n,
+                                                                  const long long* __restrict__ offsets, long long m,
+                                                                  const LookaheadItems it, unsigned long long seed,
+                                                                  uint32_t rng_step, uint32_t env_offset, void* actions_out,
+                                                                  int out_i64, int32_t* score_out, int32_t* ties_out) {
+  const int lane = threadIdx.x & 31;
+  const int g = blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (g >= n) return;
+  const uint8_t* b = boards + (size_t)g * 96;
+  const int side = meta[(size_t)g * 32 + 14], status = meta[(size_t)g * 32 + 15];
+  long long lo = offsets[g], hi = offsets[g + 1];
+  lo = lo < 0 ? 0 : (lo > m ? m : lo);
+  hi = hi < 0 ? 0 : (hi > m ? m : hi);
+  if (hi < lo || status != 0) hi = lo;
+  int best = -2147483647 - 1, cnt = 0;
+  for (long long i = lo + lane; i < hi; i += 32) {
+    const int s = it.score(b, side, i);
+    if (s > best) { best = s; cnt = 1; }
+    else if (s == best) cnt++;
+  }
+  const int M = __reduce_max_sync(FULL, best);
+  const int ties = (int)__reduce_add_sync(FULL, (unsigned)(best == M ? cnt : 0));
+  long long pick = -1;
+  if (ties > 0) {
+    int k = (int)(((unsigned long long)rand32(seed, (unsigned long long)env_offset + (unsigned long long)g, rng_step) *
+                   (unsigned long long)ties) >> 32);
+    for (long long base = lo; base < hi; base += 32) {
+      const long long i = base + lane;
+      const bool t = i < hi && it.score(b, side, i) == M;
+      const uint32_t bal = __ballot_sync(FULL, t);
+      const int c = __popc(bal);
+      if (k < c) {  // warp-uniform
+        const uint32_t own = __ballot_sync(FULL, t && __popc(bal & lowmask32(lane)) == k);
+        pick = it.action(base + __ffs(own) - 1);
+        break;
+      }
+      k -= c;
+    }
+  }
+  if (lane == 0) {
+    if (out_i64) reinterpret_cast<long long*>(actions_out)[g] = pick;
+    else reinterpret_cast<int*>(actions_out)[g] = (int)pick;
+    if (score_out) score_out[g] = ties > 0 ? M : 0;
+    if (ties_out) ties_out[g] = ties;
+  }
+}
+
 // GAE, exact variant: one thread per env column, sequential over time in the reference's op order with
 // every operation rounded separately (__fmul_rn/__fadd_rn are never contracted into FMAs).  Loads are
 // coalesced across envs.  Used when N offers enough parallelism.
@@ -682,6 +834,41 @@ int kz_heuristic_actions(const void* state, int n, int hist_cap, const uint8_t* 
     kz_heuristic_kernel<MaskWindows><<<(n + 7) / 8, 256, 0, st>>>(base + offs[0], base + offs[1], n, mask, mask_stride,
                                                                    actions, actions_i64, tier, tier_count, seed, rng_step,
                                                                    env_offset);
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? KZ_OK : fail(e);
+}
+
+int kz_capture_gain(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words, int32_t* gain,
+                    int32_t* count, void* stream) {
+  int64_t offs[3], total = 0;
+  if (!state || !bitmap || !gain || kz_state_layout(n, hist_cap, offs, &total) != KZ_OK) return KZ_E_ARG;
+  if (bitmap_stride_words < KZ_BITMAP_WORDS_MIN || ((uintptr_t)state & 255) || ((uintptr_t)bitmap & 3) ||
+      ((uintptr_t)gain & 3) || ((uintptr_t)count & 3))
+    return KZ_E_ARG;
+  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
+  kz_capture_gain_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      base + offs[0], base + offs[1], n, bitmap, bitmap_stride_words, gain, count);
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? KZ_OK : fail(e);
+}
+
+int kz_lookahead_select(const void* state, int n, int hist_cap, const int64_t* offsets, int64_t m, const void* actions,
+                        int actions_i64, const uint8_t* done, const uint8_t* reason, const uint8_t* err,
+                        const int32_t* reply_gain, const int32_t* reply_mates, uint64_t seed, uint32_t rng_step,
+                        uint32_t env_offset, void* actions_out, int out_i64, int32_t* score, int32_t* ties, void* stream) {
+  int64_t offs[3], total = 0;
+  if (!state || !offsets || !actions_out || m < 0 || kz_state_layout(n, hist_cap, offs, &total) != KZ_OK) return KZ_E_ARG;
+  if (((uintptr_t)state & 255) || ((uintptr_t)offsets & 7) || ((uintptr_t)actions_out & (out_i64 ? 7 : 3)) ||
+      ((uintptr_t)score & 3) || ((uintptr_t)ties & 3))
+    return KZ_E_ARG;
+  if (m > 0 && (!actions || !done || !reason || !err || !reply_gain || !reply_mates ||
+                ((uintptr_t)actions & (actions_i64 ? 7 : 3)) || ((uintptr_t)reply_gain & 3) || ((uintptr_t)reply_mates & 3)))
+    return KZ_E_ARG;
+  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
+  const LookaheadItems it{actions, actions_i64, done, reason, err, reply_gain, reply_mates};
+  kz_lookahead_select_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      base + offs[0], base + offs[1], n, reinterpret_cast<const long long*>(offsets), m, it, seed, rng_step, env_offset,
+      actions_out, out_i64, score, ties);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? KZ_OK : fail(e);
 }

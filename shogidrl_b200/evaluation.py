@@ -6,7 +6,9 @@ once on a VecShogiEnv: one player moves for one colour, the other for the other;
 counting until ``num_games`` have been completed.  A player is an agent-like object (``select_actions(obs, mask)``) or
 one of the reference's scripted opponents (keisei/utils/opponents.py), played on the device: ``"random"`` /
 ``SimpleRandomOpponent`` (the engine's fused uniform-random legal action) or ``"heuristic"`` /
-``SimpleHeuristicOpponent`` (``VecShogiEnv.heuristic_actions``, one launch per step)."""
+``SimpleHeuristicOpponent`` (``VecShogiEnv.heuristic_actions``, one launch per step) -- and the one-ply look-ahead
+player ``"lookahead"`` (``VecShogiEnv.lookahead_actions``: mates, material and the opponent's best reply for every
+legal move), which has no scalar counterpart in the reference."""
 from __future__ import annotations
 
 import json
@@ -39,14 +41,17 @@ class EvaluationResult:
 
 
 def _player_kind(player) -> str:
-    """"random", "heuristic" or "agent" for a player of evaluate_vs_opponent (None = the uniform-random player)."""
+    """"random", "heuristic", "lookahead" or "agent" for a player of evaluate_vs_opponent (None = the uniform-random
+    player)."""
     if player is None or isinstance(player, SimpleRandomOpponent) or (isinstance(player, str) and player == "random"):
         return "random"
     if isinstance(player, SimpleHeuristicOpponent) or (isinstance(player, str) and player == "heuristic"):
         return "heuristic"
+    if isinstance(player, str) and player == "lookahead":
+        return "lookahead"
     if isinstance(player, (str, BaseOpponent)):
-        raise ValueError(f"unknown scripted player {player!r}: expected 'random', 'heuristic', SimpleRandomOpponent, "
-                         "SimpleHeuristicOpponent or an agent with select_actions(obs, mask)")
+        raise ValueError(f"unknown scripted player {player!r}: expected 'random', 'heuristic', 'lookahead', "
+                         "SimpleRandomOpponent, SimpleHeuristicOpponent or an agent with select_actions(obs, mask)")
     return "agent"
 
 
@@ -79,8 +84,9 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
                          max_steps: Optional[int] = None, start_positions: Optional[Sequence[str]] = None
                          ) -> EvaluationResult:
     """Play ``num_games`` games of ``agent`` against ``opponent`` (None = uniform-random legal moves).  Either side may
-    be an agent-like object, ``"random"``, ``"heuristic"`` or an instance of the two scripted opponent classes; results
-    are counted from ``agent``'s side.  The agent plays Black in even-numbered envs and White in odd-numbered ones.
+    be an agent-like object, ``"random"``, ``"heuristic"``, ``"lookahead"`` or an instance of the two scripted opponent
+    classes; results are counted from ``agent``'s side.  A ``"lookahead"`` player is computed each step only for the envs
+    where it is to move (``lookahead_actions(active=...)``).  The agent plays Black in even-numbered envs and White in odd-numbered ones.
     Every env has a fixed QUOTA of games (``num_games`` spread evenly over the envs): the first ``quota`` games an env finishes are counted and later ones
     are ignored, so the sample is ``num_games`` independent games exactly as the reference's sequential loop plays them
     -- counting "the first num_games completions of the batch" would over-sample short (decisive) games, because a
@@ -110,12 +116,15 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
         env.reset(refresh=False, start_pick=paired_openings(finished, pool_size))
     env.refresh(random_actions=True)
     heuristic = env.heuristic_actions() if "heuristic" in kinds else None
+    lookahead = torch.full((n,), -1, dtype=torch.int64, device=dev) if "lookahead" in kinds else None
 
     def actions_of(player, kind):
         if kind == "random":
             return env.next_actions
         if kind == "heuristic":
             return heuristic
+        if kind == "lookahead":
+            return lookahead
         return player.select_actions(env.obs, env.mask, is_training=not deterministic)[0]
 
     # side to move per env: read from plane 42 of the observation (1.0 = Black to move)
@@ -128,6 +137,9 @@ def evaluate_vs_opponent(agent, num_games: int, *, opponent=None, num_envs: int 
     while done_games < num_games and steps < limit:
         black_to_move = env.obs[:, 42, 0, 0] > 0.5
         agent_turn = black_to_move == agent_is_black
+        if lookahead is not None:  # for the envs where a look-ahead player is to move
+            env.lookahead_actions(out=lookahead, active=None if kinds[0] == kinds[1] else
+                                  (agent_turn if kinds[0] == "lookahead" else ~agent_turn))
         a_agent = actions_of(agent, kinds[0])
         a_opp = actions_of(opponent, kinds[1])
         actions = torch.where(agent_turn, a_agent, a_opp).contiguous()
@@ -212,12 +224,12 @@ def mate_batches(num_positions: int, num_envs: int) -> List[Tuple[int, int, int]
 def evaluate_mate_in_one(player, positions: Sequence[str], *, num_envs: int = 1024, device="cuda", seed: int = 0,
                          deterministic: bool = True) -> MateInOneResult:
     """Mate-in-one score of ``player`` on ``positions`` (SFEN strings, e.g. from harvest_mate_in_one): the player is an
-    agent (``select_actions(obs, mask)``), ``"random"`` or ``"heuristic"``, as in evaluate_vs_opponent.  The positions are
-    loaded in batches of ``num_envs`` (``load_sfens``, the last batch padded), the player picks one move per position, and
-    the move solves the position when ``expand`` ends the game by Tsumi without capturing a king.  Positions without a
+    agent (``select_actions(obs, mask)``), ``"random"``, ``"heuristic"`` or ``"lookahead"``, as in evaluate_vs_opponent.
+    The positions are loaded in batches of ``num_envs`` (``load_sfens``, the last batch padded), the player picks one
+    move per position, and the move solves the position when ``expand`` ends the game by Tsumi without capturing a king.  Positions without a
     mate in one (``mate_in_one``) do not count toward the rate.  The random player's move on position i is the engine's
     fused uniform-random legal action keyed (seed, i, step 0); the heuristic player's draw is keyed the same way
-    (with its own salt, as ``heuristic_actions``)."""
+    (with its own salt, as ``heuristic_actions``), and so is the look-ahead player's (``lookahead_actions``)."""
     kind = _player_kind(player)
     positions = [str(s) for s in positions]
     batches = mate_batches(len(positions), num_envs)
@@ -239,6 +251,8 @@ def evaluate_mate_in_one(player, positions: Sequence[str], *, num_envs: int = 10
             actions = env.next_actions.clone()
         elif kind == "heuristic":
             actions = env.heuristic_actions()
+        elif kind == "lookahead":
+            actions = env.lookahead_actions()
         else:
             actions = player.select_actions(env.obs, env.mask, is_training=not deterministic)[0]
             actions = actions.to(device=env.device, dtype=torch.int64).contiguous()
@@ -360,7 +374,7 @@ def tournament_standings(results: Mapping[str, EvaluationResult]) -> Dict[str, A
 def evaluate_tournament(agent, opponents: Mapping[str, Any], num_games_per_opponent: int,
                         **kwargs) -> Tuple[Dict[str, Any], Dict[str, EvaluationResult]]:
     """Round of matches against every opponent of the pool (name -> a player of evaluate_vs_opponent: an agent-like
-    object, "random" / None, "heuristic" or a scripted opponent instance), colours balanced inside each match; returns
+    object, "random" / None, "heuristic", "lookahead" or a scripted opponent instance), colours balanced inside each match; returns
     (standings, per-opponent results)."""
     results = {name: evaluate_vs_opponent(agent, num_games_per_opponent, opponent=opp, **kwargs)
                for name, opp in opponents.items()}

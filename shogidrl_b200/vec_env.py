@@ -36,6 +36,40 @@ def parse_start_positions(sfens: Sequence[str], max_moves: int):
             np.asarray([p[2] for p in packed], np.uint8), np.asarray([p[3] for p in packed], np.int32))
 
 
+def _mates_in_one(L, state: torch.Tensor, n: int, hist_cap: int, bitmap: torch.Tensor, sp):
+    """Mates in one of the n games of a state blob, from their legal rows ``bitmap`` (int32 [n, 448]): -> (the lowest
+    mating action int64 [n], -1 for none; the number of mating moves int32 [n]).  A mate must give check, so
+    kz_check_bitmap keeps the checking moves, kz_legal_list lists them and kz_expand decides them: Tsumi without
+    capturing a king.  One host read (of the number of checking moves)."""
+    d = bitmap.device
+    rows = torch.empty((n, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
+    count = torch.empty(n, dtype=torch.int32, device=d)
+    nv.check(L.kz_check_bitmap(state.data_ptr(), n, hist_cap, bitmap.data_ptr(), bitmap.stride(0), rows.data_ptr(),
+                               nv.BITMAP_WORDS, count.data_ptr(), sp), "kz_check_bitmap")
+    offsets = torch.zeros(n + 1, dtype=torch.int64, device=d)
+    offsets[1:] = torch.cumsum(count, 0, dtype=torch.int64)
+    m = int(offsets[-1])
+    mates = torch.zeros(n, dtype=torch.int32, device=d)
+    action = torch.full((n,), -1, dtype=torch.int64, device=d)
+    if m == 0:
+        return action, mates
+    parent = torch.empty(m, dtype=torch.int32, device=d)
+    actions = torch.empty(m, dtype=torch.int64, device=d)
+    nv.check(L.kz_legal_list(rows.data_ptr(), nv.BITMAP_WORDS, n, offsets.data_ptr(), parent.data_ptr(), actions.data_ptr(),
+                             1, sp), "kz_legal_list")
+    del rows
+    reason = torch.empty(m, dtype=torch.uint8, device=d)
+    err = torch.empty(m, dtype=torch.uint8, device=d)
+    nv.check(L.kz_expand(state.data_ptr(), n, hist_cap, 0, parent.data_ptr(), actions.data_ptr(), 1, m, None, 0, None, 0,
+                         None, None, None, reason.data_ptr(), None, None, None, err.data_ptr(), None, 0, sp), "kz_expand")
+    mate = (reason == nv.TSUMI) & ((err & nv.ERR_KING_CAPTURE) == 0)
+    p = parent.long()
+    mates.index_add_(0, p, mate.to(torch.int32))
+    first = torch.full((n,), nv.NUM_ACTIONS, dtype=torch.int64, device=d)
+    first.scatter_reduce_(0, p, torch.where(mate, actions, nv.NUM_ACTIONS), "amin")
+    return torch.where(mates > 0, first, action), mates
+
+
 class VecShogiEnv:
     # Pool draws are keyed by seed ^ POOL_SALT (auto-reset inside kz_step_pool) and seed ^ POOL_RESET_SALT (explicit
     # reset), so that they are independent of the fused random actions and of each other: a reset() right after an
@@ -344,16 +378,22 @@ class VecShogiEnv:
                                          self.legal_count.data_ptr(), self._sp()), "kz_legal_bitmap")
         return obs, bitmap
 
+    def _legal_rows(self):
+        """Scratch legal-bitmap rows (int32 [n, 448]) and legal counts (int32 [n]) of the CURRENT positions
+        (kz_legal_bitmap); the env's own legal_count is left as it is."""
+        bitmap = torch.empty((self.n, nv.BITMAP_WORDS), dtype=torch.int32, device=self.device)
+        count = torch.empty(self.n, dtype=torch.int32, device=self.device)
+        nv.check(self._L.kz_legal_bitmap(self.state.data_ptr(), self.n, self.hist_cap, None, 0, bitmap.data_ptr(),
+                                         nv.BITMAP_WORDS, None, count.data_ptr(), self._sp()), "kz_legal_bitmap")
+        return bitmap, count
+
     def legal_actions(self):
         """Every legal move of every env's CURRENT position as a list grouped by env (CSR): -> (offsets int64 [n+1],
         parent int32 [M], actions int64 [M]); env g's legal actions are actions[offsets[g]:offsets[g+1]] in ascending
         order, and parent[i] is the env of move i.  kz_legal_bitmap into scratch rows, then kz_legal_list; one host read
         (of M, to size the list)."""
         d, sp = self.device, self._sp()
-        bitmap = torch.empty((self.n, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
-        count = torch.empty(self.n, dtype=torch.int32, device=d)
-        nv.check(self._L.kz_legal_bitmap(self.state.data_ptr(), self.n, self.hist_cap, None, 0, bitmap.data_ptr(),
-                                         nv.BITMAP_WORDS, None, count.data_ptr(), sp), "kz_legal_bitmap")
+        bitmap, count = self._legal_rows()
         offsets = torch.zeros(self.n + 1, dtype=torch.int64, device=d)
         offsets[1:] = torch.cumsum(count, 0, dtype=torch.int64)
         m = int(offsets[-1])
@@ -413,10 +453,7 @@ class VecShogiEnv:
         (offsets int64 [n+1], parent int32 [M], actions int64 [M]).  kz_legal_bitmap, kz_check_bitmap, then kz_legal_list
         on the check rows; one host read (of M)."""
         d, sp = self.device, self._sp()
-        bitmap = torch.empty((self.n, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
-        count = torch.empty(self.n, dtype=torch.int32, device=d)
-        nv.check(self._L.kz_legal_bitmap(self.state.data_ptr(), self.n, self.hist_cap, None, 0, bitmap.data_ptr(),
-                                         nv.BITMAP_WORDS, None, count.data_ptr(), sp), "kz_legal_bitmap")
+        bitmap, _ = self._legal_rows()
         rows, count = self.check_bitmap(bitmap)
         offsets = torch.zeros(self.n + 1, dtype=torch.int64, device=d)
         offsets[1:] = torch.cumsum(count, 0, dtype=torch.int64)
@@ -430,29 +467,91 @@ class VecShogiEnv:
 
     def mate_in_one(self) -> Dict[str, torch.Tensor]:
         """Mates in one of every env's CURRENT position: -> {"action": int64 [n] the lowest-index mating move (-1: none),
-        "count": int32 [n] the number of mating moves}.  A mate must give check, so only ``checking_actions`` are
+        "count": int32 [n] the number of mating moves}.  A mate must give check, so only the checking moves are
         expanded (``expand``); a move mates when its expansion ends the game by Tsumi without capturing a king (capturing
         a king is outside the engine's contract, as in ``step``).  No env moves."""
-        _, parent, actions = self.checking_actions()
-        d = self.device
-        count = torch.zeros(self.n, dtype=torch.int32, device=d)
-        action = torch.full((self.n,), -1, dtype=torch.int64, device=d)
-        if parent.numel() == 0:
-            return {"action": action, "count": count}
-        m = int(parent.numel())
-        reason = torch.empty(m, dtype=torch.uint8, device=d)
-        err = torch.empty(m, dtype=torch.uint8, device=d)
-        # kz_expand directly rather than expand(): the parents come from kz_legal_list and need no host-side check
-        nv.check(self._L.kz_expand(self.state.data_ptr(), self.n, self.hist_cap, 0, parent.data_ptr(), actions.data_ptr(), 1,
-                                   m, None, 0, None, 0, None, None, None, reason.data_ptr(), None, None, None,
-                                   err.data_ptr(), None, 0, self._sp()), "kz_expand")
-        mate = (reason == nv.TSUMI) & ((err & nv.ERR_KING_CAPTURE) == 0)
-        p = parent.long()
-        count.index_add_(0, p, mate.to(torch.int32))
-        first = torch.full((self.n,), nv.NUM_ACTIONS, dtype=torch.int64, device=d)
-        first.scatter_reduce_(0, p, torch.where(mate, actions, nv.NUM_ACTIONS), "amin")
-        action = torch.where(count > 0, first, action)
+        bitmap, _ = self._legal_rows()
+        action, count = _mates_in_one(self._L, self.state, self.n, self.hist_cap, bitmap, self._sp())
         return {"action": action, "count": count}
+
+    # The look-ahead opponent draws from the env's random stream keyed by seed ^ LOOKAHEAD_SALT, independently of the
+    # fused uniform-random action and of the heuristic opponent's draw for the same step and env.
+    LOOKAHEAD_SALT = 0x4C6F6F6B416864  # "LookAhd"
+
+    def lookahead_actions(self, out: Optional[torch.Tensor] = None, *, active: Optional[torch.Tensor] = None,
+                          score: Optional[torch.Tensor] = None, ties: Optional[torch.Tensor] = None,
+                          max_items: int = 1 << 20) -> torch.Tensor:
+        """The one-ply look-ahead opponent's move for every env's CURRENT position.  Every legal move ``a`` is expanded
+        with the env's history (``expand``) and scored by the first rule that applies: 1,000,000 if it mates (Tsumi
+        without capturing a king); its gain if it ends the game otherwise (sennichite, stalemate, move limit); -1,000,000
+        if the opponent then has a mate in one; otherwise its gain minus the opponent's best reply gain R.  The gain of a
+        board move is the captured piece's value plus the value of its unpromoted type, plus the promotion bonus of a
+        promoting move (values P L N S G B R K +P +L +N +S +B +R = 1 3 4 5 6 8 10 0 6 6 6 6 10 12); a drop gains 0.  The
+        pick is uniform over the moves of the best score: the k-th in ascending action order, k = mulhi(rand32(seed ^
+        LOOKAHEAD_SALT, env_offset + env, step_index), ties), as ``heuristic_actions`` draws.
+
+        The replies are judged on the successors without history (as ``expand``'s children carry none): a mate does not
+        depend on it, R ignores repetition draws a reply could cause.  ``active`` (bool / uint8 [n], default all): only
+        these envs are computed, the others get -1, as do finished games and games without a legal move.  ``out`` int64 /
+        int32 [n] (default: a new int64 tensor); ``score`` and ``ties`` (int32 [n], optional) receive the best score and
+        the number of moves reaching it (0 and 0 where the action is -1).  Games are processed in chunks of whole games of
+        at most ``max_items`` legal moves (>= 1,024, so one game's moves always fit; the result does not depend on it);
+        memory is about 5 KB per item of a chunk.  No env moves and nothing of the env is written but its work counter."""
+        if int(max_items) < 1024:
+            raise ValueError(f"lookahead_actions: max_items must be at least 1024, got {max_items}")
+        L, d, sp, n = self._L, self.device, self._sp(), self.n
+        if out is None:
+            out = torch.empty(n, dtype=torch.int64, device=d)
+        op = self._vec_arg(out, "out", (torch.int64, torch.int32))
+        sc, tp = self._vec_arg(score, "score", (torch.int32,)), self._vec_arg(ties, "ties", (torch.int32,))
+        self._vec_arg(active, "active", (torch.bool, torch.uint8))
+        state = self.state.data_ptr()
+        bitmap, count = self._legal_rows()
+        listed = self.export()[2][:, 3] == 0  # finished games list nothing
+        if active is not None:
+            listed &= active[:n] != 0
+        offsets = torch.zeros(n + 1, dtype=torch.int64, device=d)
+        offsets[1:] = torch.cumsum(torch.where(listed, count, 0), 0, dtype=torch.int64)
+        offsets_h = offsets.cpu().numpy()
+        m = int(offsets_h[-1])
+        parent = torch.empty(m, dtype=torch.int32, device=d)
+        actions = torch.empty(m, dtype=torch.int64, device=d)
+        done, reason, err = (torch.empty(m, dtype=torch.uint8, device=d) for _ in range(3))
+        reply_gain, reply_mates = (torch.empty(m, dtype=torch.int32, device=d) for _ in range(2))
+        if m > 0:
+            nv.check(L.kz_legal_list(bitmap.data_ptr(), nv.BITMAP_WORDS, n, offsets.data_ptr(), parent.data_ptr(),
+                                     actions.data_ptr(), 1, sp), "kz_legal_list")
+        del bitmap
+        a = 0
+        while a < n:  # chunks of consecutive games with at most max_items items
+            b = max(int(np.searchsorted(offsets_h, offsets_h[a] + max_items, side="right")) - 1, a + 1)
+            i0, i1 = int(offsets_h[a]), int(offsets_h[b])
+            if i1 > i0:
+                self._lookahead_chunk(i0, i1, parent, actions, done, reason, err, reply_gain, reply_mates)
+            a = b
+        items = (actions, done, reason, err, reply_gain, reply_mates)
+        ptrs = [t.data_ptr() if m > 0 else None for t in items]
+        nv.check(L.kz_lookahead_select(state, n, self.hist_cap, offsets.data_ptr(), m, ptrs[0], 1, *ptrs[1:],
+                                       (self.seed ^ self.LOOKAHEAD_SALT) & 0xFFFFFFFFFFFFFFFF, self.step_index,
+                                       self.env_offset, op, int(out.dtype == torch.int64), sc, tp, sp),
+                 "kz_lookahead_select")
+        return out
+
+    def _lookahead_chunk(self, i0: int, i1: int, parent, actions, done, reason, err, reply_gain, reply_mates) -> None:
+        """Items [i0, i1) of lookahead_actions: kz_expand into a child batch with its legal rows, then R of each child
+        (kz_capture_gain) and its number of mates in one (the mate_in_one route on the child batch)."""
+        L, d, sp, m = self._L, self.device, self._sp(), i1 - i0
+        total = C.c_int64()
+        nv.check(L.kz_state_layout(m, 1, None, C.byref(total)), "kz_state_layout")
+        child = torch.empty(total.value, dtype=torch.uint8, device=d)
+        rows = torch.empty((m, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
+        nv.check(L.kz_expand(self.state.data_ptr(), self.n, self.hist_cap, 0, parent[i0:].data_ptr(),
+                             actions[i0:].data_ptr(), 1, m, None, 0, rows.data_ptr(), nv.BITMAP_WORDS, None, None,
+                             done[i0:].data_ptr(), reason[i0:].data_ptr(), None, None, None, err[i0:].data_ptr(),
+                             child.data_ptr(), 1, sp), "kz_expand")
+        nv.check(L.kz_capture_gain(child.data_ptr(), m, 1, rows.data_ptr(), nv.BITMAP_WORDS, reply_gain[i0:].data_ptr(),
+                                   None, sp), "kz_capture_gain")
+        reply_mates[i0:i1] = _mates_in_one(L, child, m, 1, rows, sp)[1]
 
     # The heuristic opponent draws from the env's random stream keyed by seed ^ HEURISTIC_SALT, so its pick is independent
     # of the fused uniform-random action (next_actions, keyed by the seed itself) drawn for the same step and env.
