@@ -68,7 +68,10 @@ int kz_init_tables(void* stream);
  * slots (124-bit Zobrist-style position key + 4-bit occurrence count, open addressing, slots =
  * power of two >= 2*hist_cap) replacing the tuple history of shogi_game.py:347-372, and a
  * trailing 256-byte scheduling word block (work counter of the launch in flight).
- * offsets3 (HOST) receives the byte offsets of the first three sections. */
+ * offsets3 (HOST) receives the byte offsets of the first three sections.
+ * THE BLOB RULE of every function below that takes (state, n, hist_cap), and of kz_expand's (child_state, m,
+ * child_hist_cap) when m > 0: state is non-null and 256-byte aligned, n >= 1 and 0 <= hist_cap <= 65535; otherwise the call returns
+ * KZ_E_ARG (never KZ_E_NOT_INIT) and launches nothing.  state must hold kz_state_layout(n, hist_cap) bytes. */
 int kz_state_layout(int n, int hist_cap, int64_t* offsets3, int64_t* total_bytes);
 
 /* ShogiGame.reset (shogi_game.py:79-130) for the envs whose env_mask byte is non-zero (all
@@ -288,7 +291,7 @@ int kz_heuristic_actions(const void* state, int n, int hist_cap, const uint8_t* 
  * largest gain over the legal moves of bitmap row g (kz_legal_bitmap's or kz_expand's row of the current position; stride
  * in words >= KZ_BITMAP_WORDS_MIN, 4-byte aligned; pad bits 13527.. and words 423.. are ignored), and count[g] (int32,
  * optional) = the number of those moves that reach it.  A finished game (status != 0) and a row without moves get 0 and 0.
- * Rows are addressed in 64 bits.  state 256-byte aligned.  Needs no tables. */
+ * Rows are addressed in 64 bits.  Needs no tables. */
 int kz_capture_gain(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words, int32_t* gain,
                     int32_t* count, void* stream);
 /* kz_lookahead_select: the look-ahead opponent's move for each of the n games of `state`.  Game g's items are

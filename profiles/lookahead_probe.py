@@ -28,6 +28,7 @@ sys.path.insert(0, os.path.join(ROOT, "profiles"))
 from mate_probe import card, timed, wall  # noqa: E402
 from shogidrl_b200 import VecShogiEnv  # noqa: E402
 from shogidrl_b200 import _native as nv  # noqa: E402
+from shogidrl_b200._batch import chunks  # noqa: E402
 from shogidrl_b200.evaluation import evaluate_vs_opponent  # noqa: E402
 
 
@@ -58,13 +59,10 @@ def at_size(n: int) -> dict:
     m = int(parent.numel())
     done, reason, err = (torch.empty(m, dtype=torch.uint8, device=d) for _ in range(3))
     gain, mates = (torch.empty(m, dtype=torch.int32, device=d) for _ in range(2))
-    off_h = offsets.cpu()
+    off_h = offsets.cpu().numpy()
     chunk = 1 << 20
-    a = 0
-    while a < n:
-        b = max(int(torch.searchsorted(off_h, off_h[a] + chunk, right=True)) - 1, a + 1)
+    for a, b in chunks(off_h, chunk):
         env._lookahead_chunk(int(off_h[a]), int(off_h[b]), parent, actions, done, reason, err, gain, mates)
-        a = b
     # the first chunk's children again, for kz_capture_gain and their checking replies
     m0 = min(m, chunk)
     total = C.c_int64()

@@ -1,9 +1,10 @@
-// kz_common.cuh -- bitboard helpers and piece tables shared by the engine kernels.
+// kz_common.cuh -- bitboard helpers and piece tables shared by the engine kernels, and the host binding of a state blob.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
+#include "../../include/keisei_b200.h"
 
 #define FULL 0xffffffffu
 #define BITMAP_WORDS 448      // ceil(13527 / 32) = 423, padded to 14 words per lane (k-th set bit selection)
@@ -126,4 +127,38 @@ __device__ __forceinline__ uint32_t code_info(int code) {
     if (cls <= CLS_BN) cls += 4;
   }
   return step | (slide << 8) | (cls << 16) | (prom << 20) | (must << 21) | (king << 23);
+}
+
+// ---- host: the state blob of n games (kz_state_layout)
+struct Layout { int64_t off_boards, off_meta, off_hist, off_sched, total; int rep_slots; };
+inline Layout layout(int n, int hist_cap) {
+  Layout L;
+  L.rep_slots = 64;  // power of two >= 2 * hist_cap keeps the load factor below 1/2
+  while (L.rep_slots < 2 * hist_cap) L.rep_slots *= 2;
+  L.off_boards = 0;
+  L.off_meta = (int64_t)n * 96;
+  L.off_hist = L.off_meta + (int64_t)n * 32;
+  L.off_hist = (L.off_hist + 255) & ~(int64_t)255;
+  L.off_sched = L.off_hist + (int64_t)n * L.rep_slots * 16;  // 256 B: the tile counter of the launch in flight
+  L.total = L.off_sched + 256;
+  return L;
+}
+
+// Sections of a bound state blob.
+struct StateBlob {
+  uint8_t* boards;  // [n][96]
+  uint8_t* meta;    // [n][32]
+  uint4* hist;      // [n][rep_slots] repetition tables
+  uint8_t* sched;   // the scheduling block
+  int rep_slots;
+};
+// Every entry point that takes (state, n, hist_cap) binds it here, before any other check that can return KZ_E_NOT_INIT:
+// KZ_E_ARG unless state is non-null and 256-byte aligned, n >= 1 and 0 <= hist_cap <= 65535.
+inline int bind_state(const void* state, int n, int hist_cap, StateBlob& B) {
+  if (!state || ((uintptr_t)state & 255) || n <= 0 || hist_cap < 0 || hist_cap > 65535) return KZ_E_ARG;
+  const Layout L = layout(n, hist_cap);
+  uint8_t* base = reinterpret_cast<uint8_t*>(const_cast<void*>(state));
+  B = StateBlob{base + L.off_boards, base + L.off_meta, reinterpret_cast<uint4*>(base + L.off_hist), base + L.off_sched,
+                L.rep_slots};
+  return KZ_OK;
 }

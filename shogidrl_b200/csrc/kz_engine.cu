@@ -1754,20 +1754,6 @@ inline int cur_device() { int d = 0; return cudaGetDevice(&d) == cudaSuccess && 
 inline bool host_ready() { const int d = cur_device(); return d >= 0 && g_ready[d]; }
 inline int sm_count() { const int d = cur_device(); return d >= 0 ? g_sm_counts[d] : 0; }
 
-struct Layout { int64_t off_boards, off_meta, off_hist, off_sched, total; int rep_slots; };
-Layout layout(int n, int hist_cap) {
-  Layout L;
-  L.rep_slots = 64;  // power of two >= 2 * hist_cap keeps the load factor below 1/2
-  while (L.rep_slots < 2 * hist_cap) L.rep_slots *= 2;
-  L.off_boards = 0;
-  L.off_meta = (int64_t)n * 96;
-  L.off_hist = L.off_meta + (int64_t)n * 32;
-  L.off_hist = (L.off_hist + 255) & ~(int64_t)255;
-  L.off_sched = L.off_hist + (int64_t)n * L.rep_slots * 16;  // 256 B: the tile counter of the launch in flight
-  L.total = L.off_sched + 256;
-  return L;
-}
-
 // The kz_step_kernel instantiations, [pool][mode]: refresh (mode 0) and expansion (mode 3) have no pool form.  launch_step
 // launches through this table and kz_init_tables sets the dynamic shared-memory limit of every entry.
 using StepKernel = void (*)(const StepParams);
@@ -1779,38 +1765,23 @@ StepKernel step_kernel(int mode, bool pool) { return mode >= 0 && mode < 4 ? kSt
 #define KZ_COMPACT_CTAS_PER_SM 2
 #endif
 
-// Pointers of the state blob's sections (n games, hist_cap) in P; KZ_E_ARG for a bad blob.
-int bind_state(void* state, int n, int hist_cap, StepParams& P, uint8_t** sched) {
-  if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535) return KZ_E_ARG;
-  if (((uintptr_t)state & 255) != 0) return KZ_E_ARG;
-  const Layout L = layout(n, hist_cap);
-  uint8_t* base = reinterpret_cast<uint8_t*>(state);
-  P.boards = base + L.off_boards;
-  P.meta = base + L.off_meta;
-  P.hist = reinterpret_cast<uint4*>(base + L.off_hist);
-  P.rep_slots = L.rep_slots;
-  P.hist_cap = hist_cap;
-  *sched = base + L.off_sched;
-  return KZ_OK;
-}
-
-int launch_kernel(StepParams P, uint8_t* sched, int slot, cudaStream_t st);
+int launch_kernel(StepParams P, const StateBlob& src, int hist_cap, int slot, cudaStream_t st);
 
 int launch_step(void* state, int n, int hist_cap, StepParams P, cudaStream_t st, int first = 0, int count = -1, int slot = 0) {
-  if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535) return KZ_E_ARG;
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK) return KZ_E_ARG;
   if (count < 0) count = n - first;
   if (first < 0 || count <= 0 || first + count > n || slot < 0 || slot >= 64) return KZ_E_ARG;
   if (!host_ready()) return KZ_E_NOT_INIT;
-  uint8_t* sched = nullptr;
-  if (bind_state(state, n, hist_cap, P, &sched) != KZ_OK) return KZ_E_ARG;
   P.n = count;
   P.g_first = first;
-  return launch_kernel(P, sched, slot, st);
+  return launch_kernel(P, B, hist_cap, slot, st);
 }
 
-// Row checks, grid, work counter (slot `slot` of the scheduling block `sched`) and the launch of kz_step_kernel<P.mode>
-// over the P.n games (or kz_expand's items) from P.g_first on.
-int launch_kernel(StepParams P, uint8_t* sched, int slot, cudaStream_t st) {
+// Row checks, grid, work counter (slot `slot` of the source blob's scheduling block) and the launch of
+// kz_step_kernel<P.mode> on the source blob `src` over the P.n games (or kz_expand's items) from P.g_first on.
+int launch_kernel(StepParams P, const StateBlob& src, int hist_cap, int slot, cudaStream_t st) {
+  P.boards = src.boards; P.meta = src.meta; P.hist = src.hist; P.rep_slots = src.rep_slots; P.hist_cap = hist_cap;
   const int count = P.n;
   if (P.obs) {
     if (((uintptr_t)P.obs & 15) || (P.obs_stride & 1) || P.obs_stride < KZ_OBS_FLOATS) return KZ_E_ARG;
@@ -1836,7 +1807,7 @@ int launch_kernel(StepParams P, uint8_t* sched, int slot, cudaStream_t st) {
   if (grid < ctas_needed && count % WARPS_PER_CTA == 0) {
     // launches on one state buffer are ordered by their data dependence, so the counter can live in it (launches over
     // disjoint game ranges that run concurrently, kz_step_range, name different counter slots)
-    P.tile_counter = reinterpret_cast<int*>(sched) + slot;
+    P.tile_counter = reinterpret_cast<int*>(src.sched) + slot;
     CK(cudaMemsetAsync(P.tile_counter, 0, sizeof(int), st));
   }
 #endif
@@ -1967,20 +1938,22 @@ int kz_init_tables(void* stream) {
   g_ready[dev] = true;
   // legal bitmap of the start position, computed once by the engine itself on a scratch game
   {
-    const Layout L = layout(1, 0);
+    int64_t total = 0;
+    kz_state_layout(1, 0, nullptr, &total);
     void* scratch = nullptr;
-    CK(cudaMalloc(&scratch, L.total + KZ_MASK_PAD_STRIDE));
-    uint8_t* sb = reinterpret_cast<uint8_t*>(scratch);
-    kz_reset_kernel<<<1, 32, 0, st>>>(sb + L.off_boards, sb + L.off_meta, nullptr, 0, 1, nullptr, 500);
+    CK(cudaMalloc(&scratch, total + KZ_MASK_PAD_STRIDE));
+    StateBlob B;
+    bind_state(scratch, 1, 0, B);
+    kz_reset_kernel<<<1, 32, 0, st>>>(B.boards, B.meta, nullptr, 0, 1, nullptr, 500);
     StepParams P{};
-    P.mask = sb + L.total;
+    P.mask = reinterpret_cast<uint8_t*>(scratch) + total;  // the mask row follows the blob
     P.mask_stride = KZ_MASK_PAD_STRIDE;
     P.mode = 0;
     int rc = launch_step(scratch, 1, 0, P, st);
     if (rc != KZ_OK) { cudaFree(scratch); return rc; }
     CK(cudaStreamSynchronize(st));
     static uint8_t hm[KZ_MASK_PAD_STRIDE];
-    CK(cudaMemcpy(hm, sb + L.total, KZ_MASK_PAD_STRIDE, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(hm, P.mask, KZ_MASK_PAD_STRIDE, cudaMemcpyDeviceToHost));
     static uint32_t bm[BITMAP_WORDS];
     memset(bm, 0, sizeof bm);
     for (int i = 0; i < KZ_NUM_ACTIONS; i++)
@@ -1992,81 +1965,72 @@ int kz_init_tables(void* stream) {
 }
 
 int kz_reset(void* state, int n, int hist_cap, const uint8_t* env_mask, int max_moves, void* stream) {
-  if (!state || n <= 0 || max_moves < 0 || max_moves > 65535) return KZ_E_ARG;
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || max_moves < 0 || max_moves > 65535) return KZ_E_ARG;
   if (!host_ready()) return KZ_E_NOT_INIT;
-  const Layout L = layout(n, hist_cap);
-  uint8_t* base = reinterpret_cast<uint8_t*>(state);
-  kz_reset_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      base + L.off_boards, base + L.off_meta, reinterpret_cast<uint4*>(base + L.off_hist), L.rep_slots, n, env_mask, max_moves);
+  kz_reset_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(B.boards, B.meta, B.hist, B.rep_slots, n,
+                                                                                  env_mask, max_moves);
   CK(cudaGetLastError());
   return KZ_OK;
 }
 
 int kz_reset_pool(void* state, int n, int hist_cap, const uint8_t* env_mask, int max_moves, const uint32_t* pool, int pool_size,
                   const int32_t* pick, uint64_t pool_seed, uint32_t env_offset, int32_t* start_ids, void* stream) {
-  if (!state || n <= 0 || max_moves < 0 || max_moves > 65535 || !pool || pool_size <= 0 || ((uintptr_t)pool & 15))
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || max_moves < 0 || max_moves > 65535 || !pool || pool_size <= 0 ||
+      ((uintptr_t)pool & 15))
     return KZ_E_ARG;
   if (!host_ready()) return KZ_E_NOT_INIT;
-  const Layout L = layout(n, hist_cap);
-  uint8_t* base = reinterpret_cast<uint8_t*>(state);
   kz_reset_pool_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      base + L.off_boards, base + L.off_meta, reinterpret_cast<uint4*>(base + L.off_hist), L.rep_slots, n, env_mask, max_moves,
-      pool, pool_size, pick, pool_seed, env_offset, start_ids);
+      B.boards, B.meta, B.hist, B.rep_slots, n, env_mask, max_moves, pool, pool_size, pick, pool_seed, env_offset, start_ids);
   CK(cudaGetLastError());
   return KZ_OK;
 }
 
 int kz_pool_records(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words,
                     const int32_t* legal_count, const uint8_t* in_check, uint32_t* records, void* stream) {
-  if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535 || !bitmap || bitmap_stride_words < BITMAP_WORDS || !legal_count ||
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || !bitmap || bitmap_stride_words < BITMAP_WORDS || !legal_count ||
       !in_check || !records || ((uintptr_t)records & 15))
     return KZ_E_ARG;
-  const Layout L = layout(n, hist_cap);
-  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
   kz_pool_records_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      base + L.off_boards, base + L.off_meta, n, bitmap, bitmap_stride_words, legal_count, in_check, records);
+      B.boards, B.meta, n, bitmap, bitmap_stride_words, legal_count, in_check, records);
   CK(cudaGetLastError());
   return KZ_OK;
 }
 
 int kz_load_positions(void* state, int n, int hist_cap, const int8_t* boards, const uint8_t* hands,
                       const uint8_t* side, const int32_t* move_count, const int32_t* max_moves, void* stream) {
-  if (!state || n <= 0 || !boards || !hands || !side || !move_count || !max_moves) return KZ_E_ARG;
-  const Layout L = layout(n, hist_cap);
-  uint8_t* base = reinterpret_cast<uint8_t*>(state);
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || !boards || !hands || !side || !move_count || !max_moves) return KZ_E_ARG;
   kz_load_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      base + L.off_boards, base + L.off_meta, reinterpret_cast<uint4*>(base + L.off_hist), L.rep_slots, n, boards, hands, side,
-      move_count, max_moves);
+      B.boards, B.meta, B.hist, B.rep_slots, n, boards, hands, side, move_count, max_moves);
   CK(cudaGetLastError());
   return KZ_OK;
 }
 
 int kz_export_positions(const void* state, int n, int hist_cap, int8_t* boards, uint8_t* hands, int32_t* meta8,
                         void* stream) {
-  if (!state || n <= 0) return KZ_E_ARG;
-  const Layout L = layout(n, hist_cap);
-  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
-  kz_export_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(base + L.off_boards, base + L.off_meta, n,
-                                                                                    boards, hands, meta8);
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK) return KZ_E_ARG;
+  kz_export_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(B.boards, B.meta, n, boards, hands, meta8);
   CK(cudaGetLastError());
   return KZ_OK;
 }
 
 int kz_piece_targets(const void* state, int n, int hist_cap, const int32_t* squares, uint32_t* targets3, void* stream) {
-  if (!state || n <= 0 || !squares || !targets3) return KZ_E_ARG;
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || !squares || !targets3) return KZ_E_ARG;
   if (!host_ready()) return KZ_E_NOT_INIT;
-  const Layout L = layout(n, hist_cap);
-  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
-  kz_targets_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(base + L.off_boards, n, squares, targets3);
+  kz_targets_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(B.boards, n, squares, targets3);
   CK(cudaGetLastError());
   return KZ_OK;
 }
 
 int kz_errors(void* state, int n, int hist_cap, int32_t* out, int clear, void* stream) {
-  if (!state || n <= 0 || !out) return KZ_E_ARG;
-  const Layout L = layout(n, hist_cap);
-  uint8_t* base = reinterpret_cast<uint8_t*>(state);
-  kz_errors_kernel<<<(n + 255) / 256, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(base + L.off_meta, n, out, clear);
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || !out) return KZ_E_ARG;
+  kz_errors_kernel<<<(n + 255) / 256, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(B.meta, n, out, clear);
   CK(cudaGetLastError());
   return KZ_OK;
 }
@@ -2172,13 +2136,14 @@ int kz_expand(const void* state, int n, int hist_cap, int counter_slot, const in
               int actions_i64, int m, float* obs, int64_t obs_stride, uint32_t* bitmap, int64_t bitmap_stride_words,
               uint32_t* cobs, float* reward, uint8_t* done, uint8_t* reason, int8_t* winner, int32_t* ep_len,
               int32_t* legal_count, uint8_t* err, void* child_state, int child_hist_cap, void* stream) {
-  if (!state || n <= 0 || !parent || !actions || m < 0 || counter_slot < 0 || counter_slot >= 64) return KZ_E_ARG;
+  StateBlob src, child;
+  if (bind_state(state, n, hist_cap, src) != KZ_OK || !parent || !actions || m < 0 || counter_slot < 0 || counter_slot >= 64)
+    return KZ_E_ARG;
   if (m == 0) return KZ_OK;
+  if (child_state && (child_state == state || bind_state(child_state, m, child_hist_cap, child) != KZ_OK)) return KZ_E_ARG;
   if (!host_ready()) return KZ_E_NOT_INIT;
-  StepParams P{};
-  uint8_t* sched = nullptr;
   // the kernel writes nothing of the source batch but its work counter (MODE 3)
-  if (bind_state(const_cast<void*>(state), n, hist_cap, P, &sched) != KZ_OK) return KZ_E_ARG;
+  StepParams P{};
   P.n = m;
   P.g_first = 0;
   P.actions = actions; P.actions_i64 = actions_i64;
@@ -2189,33 +2154,25 @@ int kz_expand(const void* state, int n, int hist_cap, int counter_slot, const in
   P.mode = 3;
   P.parent = parent; P.src_n = n; P.err_out = err;
   if (child_state) {
-    if (child_state == state || child_hist_cap < 0 || child_hist_cap > 65535 || ((uintptr_t)child_state & 255)) return KZ_E_ARG;
-    const Layout C = layout(m, child_hist_cap);
-    uint8_t* cb = reinterpret_cast<uint8_t*>(child_state);
-    P.child_boards = cb + C.off_boards;
-    P.child_meta = cb + C.off_meta;
-    P.child_hist = reinterpret_cast<uint4*>(cb + C.off_hist);
-    P.child_rep_slots = C.rep_slots;
+    P.child_boards = child.boards; P.child_meta = child.meta; P.child_hist = child.hist; P.child_rep_slots = child.rep_slots;
   }
-  return launch_kernel(P, sched, counter_slot, reinterpret_cast<cudaStream_t>(stream));
+  return launch_kernel(P, src, hist_cap, counter_slot, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int kz_check_bitmap(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words, uint32_t* out,
                     int64_t out_stride_words, int32_t* count, void* stream) {
-  if (!state || n <= 0 || hist_cap < 0 || hist_cap > 65535 || !bitmap || !out || bitmap_stride_words < KZ_BITMAP_WORDS_MIN ||
-      out_stride_words < KZ_BITMAP_WORDS_MIN || ((uintptr_t)state & 255) || ((uintptr_t)bitmap & 15) || ((uintptr_t)out & 15) ||
-      ((uintptr_t)count & 3))
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || !bitmap || !out || bitmap_stride_words < KZ_BITMAP_WORDS_MIN ||
+      out_stride_words < KZ_BITMAP_WORDS_MIN || ((uintptr_t)bitmap & 15) || ((uintptr_t)out & 15) || ((uintptr_t)count & 3))
     return KZ_E_ARG;
   const uintptr_t b0 = (uintptr_t)bitmap, b1 = b0 + (uintptr_t)n * (uintptr_t)bitmap_stride_words * 4u;
   const uintptr_t o0 = (uintptr_t)out, o1 = o0 + (uintptr_t)n * (uintptr_t)out_stride_words * 4u;
   if (o0 < b1 && b0 < o1) return KZ_E_ARG;  // out overlaps bitmap
   if (!host_ready()) return KZ_E_NOT_INIT;
-  const Layout L = layout(n, hist_cap);
-  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
   int grid = sm_count() * 8;  // 8 CTAs of 8 warps per SM (24 KB of static shared memory each)
   if (grid > (n + 7) / 8) grid = (n + 7) / 8;
   kz_check_bitmap_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      base + L.off_boards, base + L.off_meta, n, bitmap, bitmap_stride_words, out, out_stride_words, count);
+      B.boards, B.meta, n, bitmap, bitmap_stride_words, out, out_stride_words, count);
   CK(cudaGetLastError());
   return KZ_OK;
 }

@@ -818,20 +818,18 @@ int kz_sample_bitmap(const void* logits, int logits_bf16, int64_t ld, const uint
 int kz_heuristic_actions(const void* state, int n, int hist_cap, const uint8_t* mask, int64_t mask_stride,
                          const uint32_t* bitmap, int64_t bitmap_stride_words, void* actions, int actions_i64, uint8_t* tier,
                          int32_t* tier_count, uint64_t seed, uint32_t rng_step, uint32_t env_offset, void* stream) {
-  int64_t offs[3], total = 0;
-  if (!state || !actions || (mask == nullptr) == (bitmap == nullptr) || kz_state_layout(n, hist_cap, offs, &total) != KZ_OK)
-    return KZ_E_ARG;
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || !actions || (mask == nullptr) == (bitmap == nullptr)) return KZ_E_ARG;
   if (mask && mask_stride < KZ_NUM_ACTIONS) return KZ_E_ARG;
   if (bitmap && (bitmap_stride_words < KZ_BITMAP_WORDS_MIN || ((uintptr_t)bitmap & 3))) return KZ_E_ARG;
   if (((uintptr_t)actions & (actions_i64 ? 7 : 3)) || ((uintptr_t)tier_count & 3)) return KZ_E_ARG;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
   if (bitmap)
-    kz_heuristic_kernel<BitmapWindows><<<(n + 7) / 8, 256, 0, st>>>(base + offs[0], base + offs[1], n, bitmap,
+    kz_heuristic_kernel<BitmapWindows><<<(n + 7) / 8, 256, 0, st>>>(B.boards, B.meta, n, bitmap,
                                                                      bitmap_stride_words * 4, actions, actions_i64, tier,
                                                                      tier_count, seed, rng_step, env_offset);
   else
-    kz_heuristic_kernel<MaskWindows><<<(n + 7) / 8, 256, 0, st>>>(base + offs[0], base + offs[1], n, mask, mask_stride,
+    kz_heuristic_kernel<MaskWindows><<<(n + 7) / 8, 256, 0, st>>>(B.boards, B.meta, n, mask, mask_stride,
                                                                    actions, actions_i64, tier, tier_count, seed, rng_step,
                                                                    env_offset);
   cudaError_t e = cudaGetLastError();
@@ -840,14 +838,12 @@ int kz_heuristic_actions(const void* state, int n, int hist_cap, const uint8_t* 
 
 int kz_capture_gain(const void* state, int n, int hist_cap, const uint32_t* bitmap, int64_t bitmap_stride_words, int32_t* gain,
                     int32_t* count, void* stream) {
-  int64_t offs[3], total = 0;
-  if (!state || !bitmap || !gain || kz_state_layout(n, hist_cap, offs, &total) != KZ_OK) return KZ_E_ARG;
-  if (bitmap_stride_words < KZ_BITMAP_WORDS_MIN || ((uintptr_t)state & 255) || ((uintptr_t)bitmap & 3) ||
-      ((uintptr_t)gain & 3) || ((uintptr_t)count & 3))
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || !bitmap || !gain || bitmap_stride_words < KZ_BITMAP_WORDS_MIN ||
+      ((uintptr_t)bitmap & 3) || ((uintptr_t)gain & 3) || ((uintptr_t)count & 3))
     return KZ_E_ARG;
-  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
   kz_capture_gain_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      base + offs[0], base + offs[1], n, bitmap, bitmap_stride_words, gain, count);
+      B.boards, B.meta, n, bitmap, bitmap_stride_words, gain, count);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? KZ_OK : fail(e);
 }
@@ -856,18 +852,16 @@ int kz_lookahead_select(const void* state, int n, int hist_cap, const int64_t* o
                         int actions_i64, const uint8_t* done, const uint8_t* reason, const uint8_t* err,
                         const int32_t* reply_gain, const int32_t* reply_mates, uint64_t seed, uint32_t rng_step,
                         uint32_t env_offset, void* actions_out, int out_i64, int32_t* score, int32_t* ties, void* stream) {
-  int64_t offs[3], total = 0;
-  if (!state || !offsets || !actions_out || m < 0 || kz_state_layout(n, hist_cap, offs, &total) != KZ_OK) return KZ_E_ARG;
-  if (((uintptr_t)state & 255) || ((uintptr_t)offsets & 7) || ((uintptr_t)actions_out & (out_i64 ? 7 : 3)) ||
-      ((uintptr_t)score & 3) || ((uintptr_t)ties & 3))
+  StateBlob B;
+  if (bind_state(state, n, hist_cap, B) != KZ_OK || !offsets || !actions_out || m < 0 || ((uintptr_t)offsets & 7) ||
+      ((uintptr_t)actions_out & (out_i64 ? 7 : 3)) || ((uintptr_t)score & 3) || ((uintptr_t)ties & 3))
     return KZ_E_ARG;
   if (m > 0 && (!actions || !done || !reason || !err || !reply_gain || !reply_mates ||
                 ((uintptr_t)actions & (actions_i64 ? 7 : 3)) || ((uintptr_t)reply_gain & 3) || ((uintptr_t)reply_mates & 3)))
     return KZ_E_ARG;
-  const uint8_t* base = reinterpret_cast<const uint8_t*>(state);
   const LookaheadItems it{actions, actions_i64, done, reason, err, reply_gain, reply_mates};
   kz_lookahead_select_kernel<<<(n + 7) / 8, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      base + offs[0], base + offs[1], n, reinterpret_cast<const long long*>(offsets), m, it, seed, rng_step, env_offset,
+      B.boards, B.meta, n, reinterpret_cast<const long long*>(offsets), m, it, seed, rng_step, env_offset,
       actions_out, out_i64, score, ties);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? KZ_OK : fail(e);

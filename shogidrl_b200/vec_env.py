@@ -5,13 +5,13 @@ Batched counterpart of ``keisei.shogi.ShogiGame`` + the reset-on-done handling o
 GPU; observations and masks are written by the kernel straight into caller-provided rollout storage."""
 from __future__ import annotations
 
-import ctypes as C
 from typing import Dict, Optional, Sequence
 
 import numpy as np
 import torch
 
 from . import _native as nv
+from ._batch import GameBatch, chunks, list_moves
 
 
 def parse_start_positions(sfens: Sequence[str], max_moves: int):
@@ -36,40 +36,6 @@ def parse_start_positions(sfens: Sequence[str], max_moves: int):
             np.asarray([p[2] for p in packed], np.uint8), np.asarray([p[3] for p in packed], np.int32))
 
 
-def _mates_in_one(L, state: torch.Tensor, n: int, hist_cap: int, bitmap: torch.Tensor, sp):
-    """Mates in one of the n games of a state blob, from their legal rows ``bitmap`` (int32 [n, 448]): -> (the lowest
-    mating action int64 [n], -1 for none; the number of mating moves int32 [n]).  A mate must give check, so
-    kz_check_bitmap keeps the checking moves, kz_legal_list lists them and kz_expand decides them: Tsumi without
-    capturing a king.  One host read (of the number of checking moves)."""
-    d = bitmap.device
-    rows = torch.empty((n, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
-    count = torch.empty(n, dtype=torch.int32, device=d)
-    nv.check(L.kz_check_bitmap(state.data_ptr(), n, hist_cap, bitmap.data_ptr(), bitmap.stride(0), rows.data_ptr(),
-                               nv.BITMAP_WORDS, count.data_ptr(), sp), "kz_check_bitmap")
-    offsets = torch.zeros(n + 1, dtype=torch.int64, device=d)
-    offsets[1:] = torch.cumsum(count, 0, dtype=torch.int64)
-    m = int(offsets[-1])
-    mates = torch.zeros(n, dtype=torch.int32, device=d)
-    action = torch.full((n,), -1, dtype=torch.int64, device=d)
-    if m == 0:
-        return action, mates
-    parent = torch.empty(m, dtype=torch.int32, device=d)
-    actions = torch.empty(m, dtype=torch.int64, device=d)
-    nv.check(L.kz_legal_list(rows.data_ptr(), nv.BITMAP_WORDS, n, offsets.data_ptr(), parent.data_ptr(), actions.data_ptr(),
-                             1, sp), "kz_legal_list")
-    del rows
-    reason = torch.empty(m, dtype=torch.uint8, device=d)
-    err = torch.empty(m, dtype=torch.uint8, device=d)
-    nv.check(L.kz_expand(state.data_ptr(), n, hist_cap, 0, parent.data_ptr(), actions.data_ptr(), 1, m, None, 0, None, 0,
-                         None, None, None, reason.data_ptr(), None, None, None, err.data_ptr(), None, 0, sp), "kz_expand")
-    mate = (reason == nv.TSUMI) & ((err & nv.ERR_KING_CAPTURE) == 0)
-    p = parent.long()
-    mates.index_add_(0, p, mate.to(torch.int32))
-    first = torch.full((n,), nv.NUM_ACTIONS, dtype=torch.int64, device=d)
-    first.scatter_reduce_(0, p, torch.where(mate, actions, nv.NUM_ACTIONS), "amin")
-    return torch.where(mates > 0, first, action), mates
-
-
 class VecShogiEnv:
     # Pool draws are keyed by seed ^ POOL_SALT (auto-reset inside kz_step_pool) and seed ^ POOL_RESET_SALT (explicit
     # reset), so that they are independent of the fused random actions and of each other: a reset() right after an
@@ -89,11 +55,9 @@ class VecShogiEnv:
         self.auto_reset = bool(auto_reset)
         self._L = nv.lib()
         nv.init_tables(self.device)
-        offs = (C.c_int64 * 3)()
-        total = C.c_int64()
-        nv.check(self._L.kz_state_layout(self.n, self.hist_cap, offs, C.byref(total)), "kz_state_layout")
-        self.state = torch.zeros(total.value, dtype=torch.uint8, device=self.device)
-        self.state_bytes = total.value
+        self._batch = GameBatch(self.n, self.hist_cap, self.device)
+        self.state = self._batch.state.zero_()
+        self.state_bytes = self.state.numel()
         # persistent per-step outputs
         d = self.device
         self.obs = torch.zeros((self.n, 46, 9, 9), dtype=torch.float32, device=d)
@@ -203,27 +167,18 @@ class VecShogiEnv:
     def _build_pool(self, parsed) -> torch.Tensor:
         """Pool records (int32 [P, POOL_RECORD_WORDS]) of parsed positions: kz_load_positions + kz_refresh
         (termination, in-check) + kz_legal_bitmap on a scratch batch of the P positions, then kz_pool_records."""
-        boards, hands, sides, mcs = parsed
-        P, d, sp = len(sides), self.device, self._sp()
-        offs, total = (C.c_int64 * 3)(), C.c_int64()
-        nv.check(self._L.kz_state_layout(P, 0, offs, C.byref(total)), "kz_state_layout")
-        state = torch.zeros(total.value, dtype=torch.uint8, device=d)
-        dev = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt).to(d).contiguous()  # noqa: E731
-        b, h, s, mc = dev(boards, torch.int8), dev(hands, torch.uint8), dev(sides, torch.uint8), dev(mcs, torch.int32)
-        mm = torch.full((P,), self.max_moves, dtype=torch.int32, device=d)
-        nv.check(self._L.kz_load_positions(state.data_ptr(), P, 0, b.data_ptr(), h.data_ptr(), s.data_ptr(), mc.data_ptr(),
-                                           mm.data_ptr(), sp), "kz_load_positions")
-        count = torch.zeros(P, dtype=torch.int32, device=d)
+        P, d, sp = len(parsed[2]), self.device, self._sp()
+        batch = GameBatch(P, 0, d).load(*parsed, self.max_moves)
         check = torch.zeros(P, dtype=torch.uint8, device=d)
-        nv.check(self._L.kz_refresh(state.data_ptr(), P, 0, None, 0, None, 0, count.data_ptr(), None, 1, 0, 0, 0, 1,
-                                    check.data_ptr(), sp), "kz_refresh")
-        bitmap = torch.zeros((P, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
-        nv.check(self._L.kz_legal_bitmap(state.data_ptr(), P, 0, None, 0, bitmap.data_ptr(), nv.BITMAP_WORDS, None,
-                                         count.data_ptr(), sp), "kz_legal_bitmap")
+        nv.check(self._L.kz_refresh(*batch.blob_args, None, 0, None, 0, None, None, 1, 0, 0, 0, 1, check.data_ptr(), sp),
+                 "kz_refresh")
+        bitmap, count = batch.legal_rows()
+        b = torch.empty((P, 81), dtype=torch.int8, device=d)
         meta = torch.empty((P, 8), dtype=torch.int32, device=d)
-        nv.check(self._L.kz_export_positions(state.data_ptr(), P, 0, None, None, meta.data_ptr(), sp), "kz_export_positions")
+        nv.check(self._L.kz_export_positions(*batch.blob_args, b.data_ptr(), None, meta.data_ptr(), sp),
+                 "kz_export_positions")
         # a legal board move onto the square of the opponent's king (kz_step flags that as KZ_ERR_KING_CAPTURE)
-        side = s.long()
+        side = meta[:, 0].long()
         ksq = torch.where(b == (8 + 14 * (1 - side))[:, None], torch.arange(81, device=d), 81).amin(1)  # 81: no king
         frm = torch.arange(81, device=d)[None, :]
         to = ksq[:, None].clamp(max=80)
@@ -238,7 +193,7 @@ class VecShogiEnv:
             if bool(kc[i]):
                 raise ValueError(f"start position {i} lets the side to move capture the opponent's king")
         records = torch.empty((P, nv.POOL_RECORD_WORDS), dtype=torch.int32, device=d)
-        nv.check(self._L.kz_pool_records(state.data_ptr(), P, 0, bitmap.data_ptr(), nv.BITMAP_WORDS, count.data_ptr(),
+        nv.check(self._L.kz_pool_records(*batch.blob_args, bitmap.data_ptr(), nv.BITMAP_WORDS, count.data_ptr(),
                                          check.data_ptr(), records.data_ptr(), sp), "kz_pool_records")
         return records
 
@@ -252,13 +207,11 @@ class VecShogiEnv:
             mp = env_mask.data_ptr()
         pk = self._pick_arg(start_pick, in_step=False)
         if self.pool is not None:
-            nv.check(self._L.kz_reset_pool(self.state.data_ptr(), self.n, self.hist_cap, mp, self.max_moves,
-                                           self.pool.data_ptr(), self.pool.shape[0], pk,
-                                           (self.seed ^ self.POOL_RESET_SALT) & 0xFFFFFFFFFFFFFFFF, self.env_offset,
-                                           self.start_ids.data_ptr(), self._sp()), "kz_reset_pool")
+            nv.check(self._L.kz_reset_pool(*self._batch.blob_args, mp, self.max_moves, self.pool.data_ptr(),
+                                           self.pool.shape[0], pk, (self.seed ^ self.POOL_RESET_SALT) & 0xFFFFFFFFFFFFFFFF,
+                                           self.env_offset, self.start_ids.data_ptr(), self._sp()), "kz_reset_pool")
         else:
-            nv.check(self._L.kz_reset(self.state.data_ptr(), self.n, self.hist_cap, mp, self.max_moves, self._sp()),
-                     "kz_reset")
+            nv.check(self._L.kz_reset(*self._batch.blob_args, mp, self.max_moves, self._sp()), "kz_reset")
             if self._ids_in_use:
                 if env_mask is None:
                     self.start_ids.fill_(-1)
@@ -279,8 +232,7 @@ class VecShogiEnv:
         mask = self.mask if mask is None else mask
         op, os_ = self._obs_args(obs)
         mp, ms = self._mask_args(mask)
-        nv.check(self._L.kz_refresh(self.state.data_ptr(), self.n, self.hist_cap, op, os_, mp, ms,
-                                    self.legal_count.data_ptr(),
+        nv.check(self._L.kz_refresh(*self._batch.blob_args, op, os_, mp, ms, self.legal_count.data_ptr(),
                                     (self.next_actions if next_out is None else next_out).data_ptr() if random_actions else None,
                                     1, self.seed, self.step_index, self.env_offset, int(eval_termination),
                                     nv.ptr(in_check), self._sp()),
@@ -348,9 +300,8 @@ class VecShogiEnv:
         else:
             fn, name = self._L.kz_step_range, "kz_step_range"
             args += (int(self.auto_reset),)
-        state = self.state.data_ptr()
         if self.step_streams == 1:  # no events: rollout steps are captured into a CUDA graph
-            nv.check(fn(state, self.n, self.hist_cap, 0, self.n, 0, *args, self._sp()), name)
+            nv.check(fn(*self._batch.blob_args, 0, self.n, 0, *args, self._sp()), name)
         else:
             cur = torch.cuda.current_stream(self.device)
             per = self.n // self.step_streams
@@ -358,7 +309,7 @@ class VecShogiEnv:
             fork.record(cur)
             for i, st in enumerate(self._side_streams):
                 st.wait_event(fork)
-                nv.check(fn(state, self.n, self.hist_cap, i * per, per, i, *args, st.cuda_stream), name)
+                nv.check(fn(*self._batch.blob_args, i * per, per, i, *args, st.cuda_stream), name)
                 join = torch.cuda.Event()
                 join.record(st)
                 cur.wait_event(join)
@@ -374,46 +325,28 @@ class VecShogiEnv:
         (kz_legal_bitmap)."""
         bp, bs = self._bitmap_args(bitmap)
         op, os_ = self._obs_args(obs)
-        nv.check(self._L.kz_legal_bitmap(self.state.data_ptr(), self.n, self.hist_cap, op, os_, bp, bs, self._cobs_arg(cobs),
+        nv.check(self._L.kz_legal_bitmap(*self._batch.blob_args, op, os_, bp, bs, self._cobs_arg(cobs),
                                          self.legal_count.data_ptr(), self._sp()), "kz_legal_bitmap")
         return obs, bitmap
-
-    def _legal_rows(self):
-        """Scratch legal-bitmap rows (int32 [n, 448]) and legal counts (int32 [n]) of the CURRENT positions
-        (kz_legal_bitmap); the env's own legal_count is left as it is."""
-        bitmap = torch.empty((self.n, nv.BITMAP_WORDS), dtype=torch.int32, device=self.device)
-        count = torch.empty(self.n, dtype=torch.int32, device=self.device)
-        nv.check(self._L.kz_legal_bitmap(self.state.data_ptr(), self.n, self.hist_cap, None, 0, bitmap.data_ptr(),
-                                         nv.BITMAP_WORDS, None, count.data_ptr(), self._sp()), "kz_legal_bitmap")
-        return bitmap, count
 
     def legal_actions(self):
         """Every legal move of every env's CURRENT position as a list grouped by env (CSR): -> (offsets int64 [n+1],
         parent int32 [M], actions int64 [M]); env g's legal actions are actions[offsets[g]:offsets[g+1]] in ascending
-        order, and parent[i] is the env of move i.  kz_legal_bitmap into scratch rows, then kz_legal_list; one host read
+        order, and parent[i] is the env of move i.  kz_legal_bitmap into scratch rows, then list_moves; one host read
         (of M, to size the list)."""
-        d, sp = self.device, self._sp()
-        bitmap, count = self._legal_rows()
-        offsets = torch.zeros(self.n + 1, dtype=torch.int64, device=d)
-        offsets[1:] = torch.cumsum(count, 0, dtype=torch.int64)
-        m = int(offsets[-1])
-        parent = torch.empty(m, dtype=torch.int32, device=d)
-        actions = torch.empty(m, dtype=torch.int64, device=d)
-        nv.check(self._L.kz_legal_list(bitmap.data_ptr(), nv.BITMAP_WORDS, self.n, offsets.data_ptr(), parent.data_ptr(),
-                                       actions.data_ptr(), 1, sp), "kz_legal_list")
-        return offsets, parent, actions
+        return list_moves(*self._batch.legal_rows())
 
     def expand(self, parent: torch.Tensor, actions: torch.Tensor, *, obs: Optional[torch.Tensor] = None,
                bitmap: Optional[torch.Tensor] = None, cobs: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         """What would happen if env ``parent[i]`` played ``actions[i]``, for M items at once, without moving any env
-        (kz_expand): -> dict of per-item tensors reward, done, reason, winner, ep_len, legal_count and err (error bits),
+        (GameBatch.expand): -> dict of per-item tensors reward, done, reason, winner, ep_len, legal_count and err (error bits),
         each exactly what ``step`` (without auto-reset) would report for that one move on a copy of the env, its
         repetition history included.  ``parent`` int32 [M] (each in [0, n)), ``actions`` int64 / int32 [M]; ``obs``
         (fp32 [M, 46, 9, 9]), ``bitmap`` (int32 [M, 448]) and ``cobs`` (int32 [M, 40]) optionally receive the successors'
         rows as ``step_rollout`` writes them.  Items of one env should be adjacent (as ``legal_actions`` lists them)."""
         m = int(parent.numel())
-        pp = self._vec_arg(parent, "parent", (torch.int32,), m)
-        ap = self._vec_arg(actions, "actions", (torch.int64, torch.int32), m)
+        self._vec_arg(parent, "parent", (torch.int32,), m)
+        self._vec_arg(actions, "actions", (torch.int64, torch.int32), m)
         nv.require(int(actions.numel()) == m, "parent and actions must have the same length")
         d = self.device
         out = {"reward": torch.zeros(m, dtype=torch.float32, device=d), "done": torch.zeros(m, dtype=torch.uint8, device=d),
@@ -424,54 +357,36 @@ class VecShogiEnv:
             return out
         if bool(((parent < 0) | (parent >= self.n)).any()):
             raise ValueError(f"parent: every entry must name an env in [0, {self.n})")
-        op, os_ = self._obs_args(obs, m)
-        bp, bs = (None, 0) if bitmap is None else self._bitmap_args(bitmap, m)
-        nv.check(self._L.kz_expand(self.state.data_ptr(), self.n, self.hist_cap, 0, pp, ap, int(actions.dtype == torch.int64),
-                                   m, op, os_, bp, bs, self._cobs_arg(cobs, m), out["reward"].data_ptr(),
-                                   out["done"].data_ptr(), out["reason"].data_ptr(), out["winner"].data_ptr(),
-                                   out["ep_len"].data_ptr(), out["legal_count"].data_ptr(), out["err"].data_ptr(), None, 0,
-                                   self._sp()), "kz_expand")
+        self._obs_args(obs, m)
+        if bitmap is not None:
+            self._bitmap_args(bitmap, m)
+        self._cobs_arg(cobs, m)
+        self._batch.expand(parent, actions, obs=obs, rows=bitmap, cobs=cobs, **out)
         return out
 
     def check_bitmap(self, bitmap: torch.Tensor, out: Optional[torch.Tensor] = None):
-        """The legal moves of every env's CURRENT position that give check (kz_check_bitmap): ``bitmap`` holds the legal
+        """The legal moves of every env's CURRENT position that give check (GameBatch.check_rows): ``bitmap`` holds the legal
         rows (int32 [n, 448], as ``legal_bitmap`` writes them) -> (out rows of the checking moves, count int32 [n]).
         ``out`` (default: new rows) must not overlap ``bitmap``.  Exact for positions in which the side not to move is
         not in check (every position reached by play); a loaded position in which it is gets all its legal moves.
         Finished games get an empty row."""
-        bp, bs = self._bitmap_args(bitmap)
-        if out is None:
-            out = torch.empty((self.n, nv.BITMAP_WORDS), dtype=torch.int32, device=self.device)
-        op, os_ = self._bitmap_args(out)
-        count = torch.empty(self.n, dtype=torch.int32, device=self.device)
-        nv.check(self._L.kz_check_bitmap(self.state.data_ptr(), self.n, self.hist_cap, bp, bs, op, os_, count.data_ptr(),
-                                         self._sp()), "kz_check_bitmap")
-        return out, count
+        self._bitmap_args(bitmap)
+        if out is not None:
+            self._bitmap_args(out)
+        return self._batch.check_rows(bitmap, out)
 
     def checking_actions(self):
         """Every legal move that gives check, of every env's CURRENT position, in ``legal_actions``' CSR form: ->
-        (offsets int64 [n+1], parent int32 [M], actions int64 [M]).  kz_legal_bitmap, kz_check_bitmap, then kz_legal_list
-        on the check rows; one host read (of M)."""
-        d, sp = self.device, self._sp()
-        bitmap, _ = self._legal_rows()
-        rows, count = self.check_bitmap(bitmap)
-        offsets = torch.zeros(self.n + 1, dtype=torch.int64, device=d)
-        offsets[1:] = torch.cumsum(count, 0, dtype=torch.int64)
-        m = int(offsets[-1])
-        parent = torch.empty(m, dtype=torch.int32, device=d)
-        actions = torch.empty(m, dtype=torch.int64, device=d)
-        if m > 0:  # empty tensors have no storage to hand to kz_legal_list
-            nv.check(self._L.kz_legal_list(rows.data_ptr(), nv.BITMAP_WORDS, self.n, offsets.data_ptr(), parent.data_ptr(),
-                                           actions.data_ptr(), 1, sp), "kz_legal_list")
-        return offsets, parent, actions
+        (offsets int64 [n+1], parent int32 [M], actions int64 [M]).  Legal rows, their checking rows, then list_moves on
+        the check rows; one host read (of M)."""
+        return list_moves(*self._batch.check_rows(self._batch.legal_rows()[0]))
 
     def mate_in_one(self) -> Dict[str, torch.Tensor]:
         """Mates in one of every env's CURRENT position: -> {"action": int64 [n] the lowest-index mating move (-1: none),
         "count": int32 [n] the number of mating moves}.  A mate must give check, so only the checking moves are
         expanded (``expand``); a move mates when its expansion ends the game by Tsumi without capturing a king (capturing
         a king is outside the engine's contract, as in ``step``).  No env moves."""
-        bitmap, _ = self._legal_rows()
-        action, count = _mates_in_one(self._L, self.state, self.n, self.hist_cap, bitmap, self._sp())
+        action, count = self._batch.mates_in_one(self._batch.legal_rows()[0])
         return {"action": action, "count": count}
 
     # The look-ahead opponent draws from the env's random stream keyed by seed ^ LOOKAHEAD_SALT, independently of the
@@ -499,59 +414,41 @@ class VecShogiEnv:
         memory is about 5 KB per item of a chunk.  No env moves and nothing of the env is written but its work counter."""
         if int(max_items) < 1024:
             raise ValueError(f"lookahead_actions: max_items must be at least 1024, got {max_items}")
-        L, d, sp, n = self._L, self.device, self._sp(), self.n
+        d, n = self.device, self.n
         if out is None:
             out = torch.empty(n, dtype=torch.int64, device=d)
         op = self._vec_arg(out, "out", (torch.int64, torch.int32))
         sc, tp = self._vec_arg(score, "score", (torch.int32,)), self._vec_arg(ties, "ties", (torch.int32,))
         self._vec_arg(active, "active", (torch.bool, torch.uint8))
-        state = self.state.data_ptr()
-        bitmap, count = self._legal_rows()
+        rows, count = self._batch.legal_rows()
         listed = self.export()[2][:, 3] == 0  # finished games list nothing
         if active is not None:
             listed &= active[:n] != 0
-        offsets = torch.zeros(n + 1, dtype=torch.int64, device=d)
-        offsets[1:] = torch.cumsum(torch.where(listed, count, 0), 0, dtype=torch.int64)
-        offsets_h = offsets.cpu().numpy()
+        offsets, parent, actions, offsets_h = list_moves(rows, torch.where(listed, count, 0), host_offsets=True)
+        del rows
         m = int(offsets_h[-1])
-        parent = torch.empty(m, dtype=torch.int32, device=d)
-        actions = torch.empty(m, dtype=torch.int64, device=d)
         done, reason, err = (torch.empty(m, dtype=torch.uint8, device=d) for _ in range(3))
         reply_gain, reply_mates = (torch.empty(m, dtype=torch.int32, device=d) for _ in range(2))
-        if m > 0:
-            nv.check(L.kz_legal_list(bitmap.data_ptr(), nv.BITMAP_WORDS, n, offsets.data_ptr(), parent.data_ptr(),
-                                     actions.data_ptr(), 1, sp), "kz_legal_list")
-        del bitmap
-        a = 0
-        while a < n:  # chunks of consecutive games with at most max_items items
-            b = max(int(np.searchsorted(offsets_h, offsets_h[a] + max_items, side="right")) - 1, a + 1)
-            i0, i1 = int(offsets_h[a]), int(offsets_h[b])
-            if i1 > i0:
-                self._lookahead_chunk(i0, i1, parent, actions, done, reason, err, reply_gain, reply_mates)
-            a = b
+        for a, b in chunks(offsets_h, max_items):
+            self._lookahead_chunk(int(offsets_h[a]), int(offsets_h[b]), parent, actions, done, reason, err, reply_gain,
+                                  reply_mates)
         items = (actions, done, reason, err, reply_gain, reply_mates)
         ptrs = [t.data_ptr() if m > 0 else None for t in items]
-        nv.check(L.kz_lookahead_select(state, n, self.hist_cap, offsets.data_ptr(), m, ptrs[0], 1, *ptrs[1:],
-                                       (self.seed ^ self.LOOKAHEAD_SALT) & 0xFFFFFFFFFFFFFFFF, self.step_index,
-                                       self.env_offset, op, int(out.dtype == torch.int64), sc, tp, sp),
+        nv.check(self._L.kz_lookahead_select(*self._batch.blob_args, offsets.data_ptr(), m, ptrs[0], 1, *ptrs[1:],
+                                             (self.seed ^ self.LOOKAHEAD_SALT) & 0xFFFFFFFFFFFFFFFF, self.step_index,
+                                             self.env_offset, op, int(out.dtype == torch.int64), sc, tp, self._sp()),
                  "kz_lookahead_select")
         return out
 
     def _lookahead_chunk(self, i0: int, i1: int, parent, actions, done, reason, err, reply_gain, reply_mates) -> None:
-        """Items [i0, i1) of lookahead_actions: kz_expand into a child batch with its legal rows, then R of each child
-        (kz_capture_gain) and its number of mates in one (the mate_in_one route on the child batch)."""
-        L, d, sp, m = self._L, self.device, self._sp(), i1 - i0
-        total = C.c_int64()
-        nv.check(L.kz_state_layout(m, 1, None, C.byref(total)), "kz_state_layout")
-        child = torch.empty(total.value, dtype=torch.uint8, device=d)
-        rows = torch.empty((m, nv.BITMAP_WORDS), dtype=torch.int32, device=d)
-        nv.check(L.kz_expand(self.state.data_ptr(), self.n, self.hist_cap, 0, parent[i0:].data_ptr(),
-                             actions[i0:].data_ptr(), 1, m, None, 0, rows.data_ptr(), nv.BITMAP_WORDS, None, None,
-                             done[i0:].data_ptr(), reason[i0:].data_ptr(), None, None, None, err[i0:].data_ptr(),
-                             child.data_ptr(), 1, sp), "kz_expand")
-        nv.check(L.kz_capture_gain(child.data_ptr(), m, 1, rows.data_ptr(), nv.BITMAP_WORDS, reply_gain[i0:].data_ptr(),
-                                   None, sp), "kz_capture_gain")
-        reply_mates[i0:i1] = _mates_in_one(L, child, m, 1, rows, sp)[1]
+        """Items [i0, i1) of lookahead_actions: expansion into a child batch with its legal rows, then R of each child
+        (capture_gain) and its number of mates in one (mates_in_one on the child batch)."""
+        s = slice(i0, i1)
+        rows = torch.empty((i1 - i0, nv.BITMAP_WORDS), dtype=torch.int32, device=self.device)
+        child = self._batch.expand(parent[s], actions[s], rows=rows, done=done[s], reason=reason[s], err=err[s],
+                                   child_hist_cap=1)
+        child.capture_gain(rows, reply_gain[s])
+        reply_mates[s] = child.mates_in_one(rows)[1]
 
     # The heuristic opponent draws from the env's random stream keyed by seed ^ HEURISTIC_SALT, so its pick is independent
     # of the fused uniform-random action (next_actions, keyed by the seed itself) drawn for the same step and env.
@@ -577,9 +474,8 @@ class VecShogiEnv:
             out = torch.empty(self.n, dtype=torch.int64, device=self.device)
         op = self._vec_arg(out, "out", (torch.int64, torch.int32))
         tp, cp = self._vec_arg(tier, "tier", (torch.uint8,)), self._vec_arg(tier_count, "tier_count", (torch.int32,))
-        nv.check(self._L.kz_heuristic_actions(self.state.data_ptr(), self.n, self.hist_cap, mp, ms, bp, bs, op,
-                                              int(out.dtype == torch.int64), tp, cp,
-                                              (self.seed ^ self.HEURISTIC_SALT) & 0xFFFFFFFFFFFFFFFF, self.step_index,
+        nv.check(self._L.kz_heuristic_actions(*self._batch.blob_args, mp, ms, bp, bs, op, int(out.dtype == torch.int64), tp,
+                                              cp, (self.seed ^ self.HEURISTIC_SALT) & 0xFFFFFFFFFFFFFFFF, self.step_index,
                                               self.env_offset, self._sp()), "kz_heuristic_actions")
         return out
 
@@ -602,17 +498,9 @@ class VecShogiEnv:
 
     def load_positions(self, boards, hands, side, move_count, max_moves=None, eval_termination: bool = True):
         """ShogiGame.from_sfen for every env from already-parsed arrays (numpy or torch)."""
-        d = self.device
-        b = torch.as_tensor(np.ascontiguousarray(boards), dtype=torch.int8).to(d).contiguous()
-        h = torch.as_tensor(np.ascontiguousarray(hands), dtype=torch.uint8).to(d).contiguous()
-        s = torch.as_tensor(np.ascontiguousarray(side), dtype=torch.uint8).to(d).contiguous()
-        mc = torch.as_tensor(np.ascontiguousarray(move_count), dtype=torch.int32).to(d).contiguous()
         if max_moves is None:
             max_moves = np.full(self.n, self.max_moves, np.int32)
-        mm = torch.as_tensor(np.ascontiguousarray(max_moves), dtype=torch.int32).to(d).contiguous()
-        nv.require(b.shape == (self.n, 81) and h.shape == (self.n, 14), "b.shape == (self.n, 81) and h.shape == (self.n, 14)")
-        nv.check(self._L.kz_load_positions(self.state.data_ptr(), self.n, self.hist_cap, b.data_ptr(), h.data_ptr(),
-                                           s.data_ptr(), mc.data_ptr(), mm.data_ptr(), self._sp()), "kz_load_positions")
+        self._batch.load(boards, hands, side, move_count, max_moves)
         self.refresh(eval_termination=eval_termination)
         return self.obs, self.mask
 
@@ -623,8 +511,8 @@ class VecShogiEnv:
         b = torch.empty((self.n, 81), dtype=torch.int8, device=d)
         h = torch.empty((self.n, 14), dtype=torch.uint8, device=d)
         m = torch.empty((self.n, 8), dtype=torch.int32, device=d)
-        nv.check(self._L.kz_export_positions(self.state.data_ptr(), self.n, self.hist_cap, b.data_ptr(), h.data_ptr(),
-                                             m.data_ptr(), self._sp()), "kz_export_positions")
+        nv.check(self._L.kz_export_positions(*self._batch.blob_args, b.data_ptr(), h.data_ptr(), m.data_ptr(), self._sp()),
+                 "kz_export_positions")
         return b, h, m
 
     def to_games(self, env_ids=None):
@@ -650,14 +538,13 @@ class VecShogiEnv:
 
     def errors(self, clear: bool = False) -> torch.Tensor:
         out = torch.empty(self.n, dtype=torch.int32, device=self.device)
-        nv.check(self._L.kz_errors(self.state.data_ptr(), self.n, self.hist_cap, out.data_ptr(), int(clear), self._sp()),
-                 "kz_errors")
+        nv.check(self._L.kz_errors(*self._batch.blob_args, out.data_ptr(), int(clear), self._sp()), "kz_errors")
         return out
 
     def piece_targets(self, squares) -> torch.Tensor:
         """Pseudo-legal target sets (81-bit, 3 x uint32 per env) of the pieces on ``squares`` [n]."""
         sq = torch.as_tensor(np.ascontiguousarray(squares), dtype=torch.int32).to(self.device).contiguous()
         out = torch.zeros((self.n, 3), dtype=torch.int32, device=self.device)
-        nv.check(self._L.kz_piece_targets(self.state.data_ptr(), self.n, self.hist_cap, sq.data_ptr(), out.data_ptr(),
-                                          self._sp()), "kz_piece_targets")
+        nv.check(self._L.kz_piece_targets(*self._batch.blob_args, sq.data_ptr(), out.data_ptr(), self._sp()),
+                 "kz_piece_targets")
         return out

@@ -119,3 +119,49 @@ def test_invalid_arguments_are_rejected_before_any_device_work():
     assert L.kz_cobs_conv_fwd(z, z, z, z, 16, 4, 1, z, z) == -1
     assert L.kz_cobs_conv_wgrad(z, z, z, z, 1, 16, 4, z, 1, z, z, z) == -1
     assert L.kz_obs_conv_wgrad_ctas(0) <= 0 or L.kz_obs_conv_wgrad_ctas(1) >= 1
+
+
+def test_every_state_entry_point_refuses_an_out_of_contract_blob():
+    """Every entry point that takes (state, n, hist_cap) returns KZ_E_ARG (-1) for a state misaligned by 16 bytes, a
+    hist_cap of -1 or 65536 and n = 0, with every other argument well formed.  The addresses are fake and never
+    dereferenced: with a GPU, an entry point that missed the check would launch on them, so the test needs a machine
+    without one (there the well-formed call reaches the tables check, -3, or the launch, -2)."""
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("fake device addresses: only without a GPU")
+    L = nv.lib()
+    z, p = None, 1 << 20
+    q = lambda k: p + (k << 16)  # noqa: E731  (aligned, never dereferenced)
+    outs = (q(3), q(4), q(5), q(6), q(7), q(8))
+    calls = {
+        "kz_reset": lambda s, n, h: L.kz_reset(s, n, h, z, 500, z),
+        "kz_reset_pool": lambda s, n, h: L.kz_reset_pool(s, n, h, z, 500, q(1), 2, z, 0, 0, z, z),
+        "kz_pool_records": lambda s, n, h: L.kz_pool_records(s, n, h, q(1), 448, q(2), q(3), q(4), z),
+        "kz_load_positions": lambda s, n, h: L.kz_load_positions(s, n, h, q(1), q(2), q(3), q(4), q(5), z),
+        "kz_export_positions": lambda s, n, h: L.kz_export_positions(s, n, h, q(1), q(2), q(3), z),
+        "kz_piece_targets": lambda s, n, h: L.kz_piece_targets(s, n, h, q(1), q(2), z),
+        "kz_errors": lambda s, n, h: L.kz_errors(s, n, h, q(1), 0, z),
+        "kz_refresh": lambda s, n, h: L.kz_refresh(s, n, h, z, 0, z, 0, q(1), z, 1, 0, 0, 0, 0, z, z),
+        "kz_legal_mask": lambda s, n, h: L.kz_legal_mask(s, n, h, q(1), 13536, q(2), z),
+        "kz_observe": lambda s, n, h: L.kz_observe(s, n, h, q(1), 3726, z),
+        "kz_legal_bitmap": lambda s, n, h: L.kz_legal_bitmap(s, n, h, z, 0, q(1), 448, z, q(2), z),
+        "kz_step": lambda s, n, h: L.kz_step(s, n, h, q(1), 1, z, 0, q(2), 13536, *outs, z, 0, 0, 0, 1, z),
+        "kz_step_rollout": lambda s, n, h: L.kz_step_rollout(s, n, h, q(1), 1, z, 0, q(2), 448, z, *outs, z, 0, 0, 0, 1, z),
+        "kz_step_range": lambda s, n, h: L.kz_step_range(s, n, h, 0, 2, 0, q(1), 1, z, 0, z, 0, q(2), 448, z,
+                                                         *outs, z, 0, 0, 0, 1, z),
+        "kz_step_pool": lambda s, n, h: L.kz_step_pool(s, n, h, 0, 2, 0, q(1), 1, z, 0, z, 0, q(2), 448, z,
+                                                       *outs, z, 0, 0, 0, q(9), 2, z, 0, z, z),
+        "kz_expand": lambda s, n, h: L.kz_expand(s, n, h, 0, q(1), q(2), 1, 4, z, 0, z, 0, z, *outs, q(9), z, 0, z),
+        "kz_expand child": lambda s, n, h: L.kz_expand(q(10), 4, 500, 0, q(1), q(2), 1, n, z, 0, z, 0, z, *outs, q(9), s, h,
+                                                       z),
+        "kz_check_bitmap": lambda s, n, h: L.kz_check_bitmap(s, n, h, q(1), 448, q(2), 448, z, z),
+        "kz_heuristic_actions": lambda s, n, h: L.kz_heuristic_actions(s, n, h, z, 0, q(1), 448, q(2), 1, z, z, 0, 0, 0, z),
+        "kz_capture_gain": lambda s, n, h: L.kz_capture_gain(s, n, h, q(1), 448, q(2), z, z),
+        "kz_lookahead_select": lambda s, n, h: L.kz_lookahead_select(s, n, h, q(1), 8, q(2), 1, q(2), q(2), q(2), q(2), q(2),
+                                                                     0, 0, 0, q(3), 1, z, z, z),
+    }
+    for name, call in calls.items():
+        assert call(p, 4, 500) in (-2, -3), name  # the other arguments are well formed
+        bad = [(p + 16, 4, 500), (p, 4, -1), (p, 4, 65536)] + ([(p, 0, 500)] if name != "kz_expand child" else [])
+        for s, n, h in bad:  # (the child batch has m games: m = 0 launches nothing and checks no child)
+            assert call(s, n, h) == -1, (name, s - p, n, h)

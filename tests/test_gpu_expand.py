@@ -275,6 +275,18 @@ def test_legal_actions_and_short_offsets(golden_dir):
         assert (seg[k:] == -7).all() and (segp[k:] == -7).all(), g
 
 
+def test_listings_of_a_batch_without_legal_moves_are_empty():
+    """legal_actions and checking_actions when every game is mated or stalemated: zero offsets and empty lists."""
+    from shogidrl_b200 import VecShogiEnv
+    env = VecShogiEnv(2, max_moves_per_game=500, device=DEV, auto_reset=False)
+    env.load_sfens(["4k4/4G4/4P4/9/9/9/9/9/4K4 w - 1", "8k/9/6NG1/9/9/9/9/9/4K4 w - 1"])  # mated, stalemated
+    assert env.export()[2][:, 3].tolist() == [1, 2] and env.legal_count.tolist() == [0, 0]
+    for what, (offsets, parent, actions) in (("legal", env.legal_actions()), ("checking", env.checking_actions())):
+        assert offsets.tolist() == [0, 0, 0], what
+        assert parent.shape == (0,) and parent.dtype == torch.int32, what
+        assert actions.shape == (0,) and actions.dtype == torch.int64, what
+
+
 HIRATE = [30, 900, 25470, 719731, 19861490]
 
 

@@ -61,3 +61,19 @@ def test_perft_argument_checks():
         perft("not a position", 1)
     assert perft(depth=0) == [1]
     assert perft(["4k4/9/9/9/9/9/9/9/4K4 b - 1"] * 2, 0, divide=True) == [{}, {}]
+
+
+def test_chunks_of_whole_games():
+    """The chunking perft and the look-ahead opponent share: consecutive games of at most max_items items, a game above
+    the limit alone, and no chunk without items."""
+    from shogidrl_b200._batch import chunks
+
+    def off(counts):
+        return np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    assert chunks(off([]), 4) == []
+    assert chunks(off([0, 0, 0]), 4) == []  # empty games only
+    assert chunks(off([0, 2, 0, 2, 0]), 4) == [(0, 5)]  # an exact fit, with the empty games around it
+    assert chunks(off([2, 2, 2, 2, 0]), 4) == [(0, 2), (2, 5)]
+    assert chunks(off([2, 3, 4]), 4) == [(0, 1), (1, 2), (2, 3)]
+    assert chunks(off([1, 9, 1]), 4) == [(0, 1), (1, 2), (2, 3)]  # a game above the limit is a chunk of its own
+    assert chunks(off([0, 9]), 4) == [(1, 2)]  # an empty game before a large one is a chunk without items
