@@ -362,7 +362,9 @@ int kz_eval_bitmap_bwd(const void* logits, int logits_bf16, int64_t ld, const ui
 
 /* PPO clipped-surrogate loss of one minibatch and its gradients in closed form (keisei/core/ppo_agent.py:332-372;
  * value clipping off): out6 = {loss, policy loss, value loss, entropy loss (= -mean entropy), mean(old_logp -
- * new_logp), clip fraction}; d_* = d loss / d input, multiplied by grad_scale.  All fp32 [n]. */
+ * new_logp), clip fraction}; d_* = d loss / d input, multiplied by grad_scale.  All fp32 [n].  NaN follows torch: clamp
+ * and min propagate it, and where min's arguments are NaN the whole gradient goes through the unclipped ratio
+ * (torch.minimum's backward), so a NaN new_logp, old_logp or advantage gives a NaN loss and a NaN d_logp. */
 int kz_ppo_loss(const float* new_logp, const float* entropy, const float* new_value, const float* old_logp,
                 const float* advantages, const float* returns, int n, float clip_epsilon, float value_coef,
                 float entropy_coef, float grad_scale, float* out6, float* d_logp, float* d_entropy, float* d_value,
@@ -376,6 +378,7 @@ int kz_ppo_loss(const float* new_logp, const float* entropy, const float* new_va
  * ppo_agent.py:300-309 done in place.
  * kz_obs_conv_wgrad: dweight [16][46][3][3] / dbias [16] (fp32, overwritten) from dout [n][16][9][9] (bf16 or fp32);
  * y_bf16 = the saved forward output when the forward applied ReLU (its backward is fused), else NULL.
+ * NaN as in torch: the ReLU keeps a NaN output, and the backward zeroes dout where y <= 0 only (a NaN y passes it).
  * workspace: ctas * 16 * 432 floats with ctas = kz_obs_conv_wgrad_ctas(n); deterministic (no atomics). */
 int kz_obs_conv_fwd(const float* obs, const int64_t* obs_rows, const float* weight, const float* bias, int cout, int n,
                     int relu, void* out_bf16, void* stream);
@@ -396,7 +399,8 @@ int kz_cobs_conv_wgrad(const uint32_t* cobs, const int64_t* cobs_rows, const voi
 
 /* ---- tail of a PPO minibatch update: torch.nn.utils.clip_grad_norm_(parameters, max_norm) followed by
  * torch.optim.Adam.step() (keisei/core/ppo_agent.py:405-413, optimizer built at :66-80), fused: one read of every
- * gradient for the global L2 norm, then one pass that applies the clip coefficient min(1, max_norm / (norm + 1e-6)),
+ * gradient for the global L2 norm, then one pass that applies the clip coefficient min(1, max_norm / (norm + 1e-6))
+ * (NaN when the norm is NaN, as torch.clamp gives it: one NaN gradient element then makes every parameter NaN),
  * optional L2 weight decay (g += wd * p) and the Adam update with bias correction on fp32 tensors, in place.
  *   params / grads / exp_avg / exp_avg_sq / steps: HOST arrays of `count` DEVICE pointers (fp32 tensors of numel[i]
  *   elements; steps[i] = that parameter's step counter as a device fp32 scalar, ALREADY incremented for this step,

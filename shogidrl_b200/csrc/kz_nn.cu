@@ -161,7 +161,7 @@ __global__ void __launch_bounds__(128) kz_obs_conv_fwd_kernel(const float* __res
         for (int e = 0; e < 4; e++) {
           const int c = col + (e & 1), oo = o + (e >> 1) * 8;
           float v = acc[j][e];
-          if (relu) v = fmaxf(v, 0.f);
+          if (relu) v = v != v ? v : fmaxf(v, 0.f);  // torch.relu keeps NaN
           if (c < 81) ys[oo * 81 + c] = __float2bfloat16(v);
         }
       }
@@ -205,7 +205,7 @@ __global__ void __launch_bounds__(288) kz_obs_conv_wgrad_kernel(const float* __r
         const size_t g = (size_t)b * COUT * 81 + i;
         float v = dout_bf16 ? __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(dout)[g])
                             : reinterpret_cast<const float*>(dout)[g];
-        if (y && !(__bfloat162float(y[g]) > 0.f)) v = 0.f;
+        if (y && __bfloat162float(y[g]) <= 0.f) v = 0.f;  // torch's threshold_backward: a NaN output passes dy
         dreg[k] = v;
       }
     }
@@ -370,7 +370,7 @@ __global__ void __launch_bounds__(128) kz_cobs_conv_fwd_kernel(const uint32_t* _
       }
       if (act) {
 #pragma unroll
-        for (int o = 0; o < COUT; o++) ys[warp][o * 81 + xy] = __float2bfloat16(relu ? fmaxf(acc[o], 0.f) : acc[o]);
+        for (int o = 0; o < COUT; o++) ys[warp][o * 81 + xy] = __float2bfloat16(relu && acc[o] == acc[o] ? fmaxf(acc[o], 0.f) : acc[o]);
       }
     }
     __syncwarp();

@@ -12,6 +12,7 @@
 // Deterministic (no atomics).  The clipped gradients are not written back: nobody reads them after the step.
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <vector>
 #include "../../include/keisei_b200.h"
 
 int kz_cuda_fail(cudaError_t e);  // kz_engine.cu: records the message for kz_last_cuda_error
@@ -79,7 +80,8 @@ __global__ void __launch_bounds__(THREADS) kz_sumsq_kernel(const Group G, float*
 }
 
 // out2[0] = total L2 norm of all gradients, out2[1] = clip coefficient min(1, max_norm / (norm + 1e-6))
-// (torch.nn.utils.clip_grad_norm_: clip_coef = max_norm / (total_norm + 1e-6), clamped to 1).
+// (torch.nn.utils.clip_grad_norm_: clip_coef = max_norm / (total_norm + 1e-6), clamped to 1).  A NaN norm gives a NaN
+// coefficient, as torch.clamp does (fminf would give 1: an unclipped step on every finite gradient).
 __global__ void __launch_bounds__(1024) kz_norm_kernel(const float* __restrict__ partials, int count, float max_norm,
                                                        float* __restrict__ out2) {
   __shared__ float red[32];
@@ -96,7 +98,8 @@ __global__ void __launch_bounds__(1024) kz_norm_kernel(const float* __restrict__
     if (threadIdx.x == 0) {
       const float norm = sqrtf(v);
       out2[0] = norm;
-      out2[1] = fminf(1.0f, max_norm / (norm + 1e-6f));
+      const float coef = max_norm / (norm + 1e-6f);
+      out2[1] = coef > 1.0f ? 1.0f : coef;
     }
   }
 }
@@ -181,11 +184,10 @@ int kz_adam_clip_step(int count, void* const* params, const void* const* grads, 
   const Hyper H{(float)lr, (float)beta1, (float)beta2, (float)eps, (float)weight_decay, (float)(1.0 - beta1),
                 (float)(1.0 - beta2)};
   // pass 1 builds the launch groups and runs the partial sums; pass 2 (after the norm) runs Adam on the same groups
-  Group groups[64];
-  int ngroups = 0, partial0 = 0;
+  std::vector<Group> groups;
+  int partial0 = 0;
   for (int i0 = 0; i0 < count;) {
-    if (ngroups == 64) return KZ_E_ARG;  // > 1024 tensors
-    Group& G = groups[ngroups];
+    Group G;
     G.count = 0;
     G.partial0 = partial0;
     G.blk0[0] = 0;
@@ -205,15 +207,13 @@ int kz_adam_clip_step(int count, void* const* params, const void* const* grads, 
     }
     if (G.count > 0) {
       partial0 += G.blk0[G.count];
-      ngroups++;
+      groups.push_back(G);
     }
   }
-  if (ngroups == 0) return KZ_E_ARG;
-  for (int k = 0; k < ngroups; k++)
-    kz_sumsq_kernel<<<groups[k].blk0[groups[k].count], THREADS, 0, st>>>(groups[k], workspace);
+  if (groups.empty()) return KZ_E_ARG;
+  for (const Group& G : groups) kz_sumsq_kernel<<<G.blk0[G.count], THREADS, 0, st>>>(G, workspace);
   kz_norm_kernel<<<1, 1024, 0, st>>>(workspace, partial0, (float)max_norm, norm_out2);
-  for (int k = 0; k < ngroups; k++)
-    kz_adam_kernel<<<groups[k].blk0[groups[k].count], THREADS, 0, st>>>(groups[k], H, norm_out2);
+  for (const Group& G : groups) kz_adam_kernel<<<G.blk0[G.count], THREADS, 0, st>>>(G, H, norm_out2);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? KZ_OK : fail(e);
 }

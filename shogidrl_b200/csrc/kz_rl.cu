@@ -735,17 +735,19 @@ __global__ void __launch_bounds__(1024) kz_ppo_loss_kernel(const float* __restri
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
     const float lp = new_lp[i], olp = old_lp[i], a = adv[i];
     const float ratio = expf(lp - olp);
-    const float clamped = fminf(fmaxf(ratio, 1.0f - clip_eps), 1.0f + clip_eps);
+    // torch.clamp and torch.min propagate NaN (fminf / fmaxf would drop it); s2 is NaN only when s1 is
+    const float clamped = ratio < 1.0f - clip_eps ? 1.0f - clip_eps : (ratio > 1.0f + clip_eps ? 1.0f + clip_eps : ratio);
     const float s1 = ratio * a, s2 = clamped * a;
-    acc[0] -= fminf(s1, s2);
+    acc[0] -= s1 > s2 ? s2 : s1;
     const float dv = new_v[i] - ret[i];
     acc[1] += dv * dv;
     acc[2] -= ent[i];
     acc[3] += olp - lp;
     acc[4] += fabsf(ratio - 1.0f) > clip_eps ? 1.f : 0.f;
     // d min(s1, s2) / d ratio: a through s1 when s1 <= s2 (ties: half through each, and s2 passes it on inside the
-    // range, where the tie happens); through s2 only inside the clip range, i.e. never when s2 is the strict minimum
-    const float g_ratio = (s1 <= s2) ? a : 0.f;
+    // range, where the tie happens); through s2 only inside the clip range, i.e. never when s2 is the strict minimum.
+    // A NaN s1 takes the whole gradient, as torch.minimum's backward gives it (neither side is the larger).
+    const float g_ratio = s1 > s2 ? 0.f : a;
     d_lp[i] = -inv_n * g_ratio * ratio * grad_scale;
     d_ent[i] = -inv_n * entropy_coef * grad_scale;
     d_v[i] = 2.0f * inv_n * dv * value_coef * grad_scale;

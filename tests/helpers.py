@@ -55,3 +55,36 @@ def random_endgames(n, seed):
             continue
         boards.append(b); hands.append(h); sides.append(side)
     return np.stack(boards), np.stack(hands), np.asarray(sides, np.uint8), np.zeros(n, np.int32)
+
+
+def obs_from_cobs(cobs):
+    """int32 [n, 40] compact observations -> fp32 [n, 46, 9, 9] (what they summarise), in plain torch."""
+    import torch
+    n = cobs.shape[0]
+    by = cobs.view(torch.uint8).reshape(n, 160)
+    planes = by[:, :81].long()
+    obs = torch.zeros((n, 46, 81), dtype=torch.float32, device=cobs.device)
+    has = planes < 28
+    idx = torch.nonzero(has)
+    obs[idx[:, 0], planes[has], idx[:, 1]] = 1.0
+    pv = cobs[:, 21:39].contiguous().view(torch.float32)
+    obs[:, 28:46, :] = pv[:, :, None]
+    return obs.reshape(n, 46, 9, 9)
+
+
+def rollout_positions(n=2048, T=40):
+    """(obs fp32 [(T + 1) n, 46, 9, 9], cobs int32 [(T + 1) n, 40]) of n random self-play games over T + 1 plies on cuda:0,
+    written by kz_step_rollout (games restart as they finish)."""
+    import torch
+    from shogidrl_b200 import VecShogiEnv
+    dev = torch.device("cuda:0")
+    env = VecShogiEnv(n, max_moves_per_game=60, device=dev, seed=17)
+    obs = torch.zeros((T + 1, n, 46, 9, 9), dtype=torch.float32, device=dev)
+    bm = torch.zeros((T + 1, n, 448), dtype=torch.int32, device=dev)
+    cobs = torch.full((T + 1, n, 40), -7, dtype=torch.int32, device=dev)
+    acts = [torch.zeros(n, dtype=torch.int64, device=dev) for _ in range(2)]
+    env.refresh(random_actions=True, next_out=acts[0])
+    env.legal_bitmap(bm[0], obs=obs[0], cobs=cobs[0])
+    for t in range(T):
+        env.step_rollout(acts[t & 1], obs[t + 1], bm[t + 1], random_actions=True, next_out=acts[(t + 1) & 1], cobs=cobs[t + 1])
+    return obs.reshape(-1, 46, 9, 9), cobs.reshape(-1, 40)

@@ -513,40 +513,12 @@ def test_policy_head_bias_gradient_is_deterministic_and_matches_column_sums():
 
 # ------------------------------------------------------------------------------------------------
 # compact observations (kz_step_rollout's cobs output) and the input layer that reads them (kz_cobs_conv_*)
-def _obs_from_cobs(cobs):
-    """int32 [n, 40] compact observations -> fp32 [n, 46, 9, 9] (what they summarise), in plain torch."""
-    n = cobs.shape[0]
-    by = cobs.view(torch.uint8).reshape(n, 160)
-    planes = by[:, :81].long()
-    obs = torch.zeros((n, 46, 81), dtype=torch.float32, device=cobs.device)
-    has = planes < 28
-    idx = torch.nonzero(has)
-    obs[idx[:, 0], planes[has], idx[:, 1]] = 1.0
-    pv = cobs[:, 21:39].contiguous().view(torch.float32)
-    obs[:, 28:46, :] = pv[:, :, None]
-    return obs.reshape(n, 46, 9, 9)
-
-
-def _rollout_positions(n=2048, T=40):
-    from shogidrl_b200 import VecShogiEnv
-    dev = torch.device("cuda:0")
-    env = VecShogiEnv(n, max_moves_per_game=60, device=dev, seed=17)
-    obs = torch.zeros((T + 1, n, 46, 9, 9), dtype=torch.float32, device=dev)
-    bm = torch.zeros((T + 1, n, 448), dtype=torch.int32, device=dev)
-    cobs = torch.full((T + 1, n, 40), -7, dtype=torch.int32, device=dev)
-    acts = [torch.zeros(n, dtype=torch.int64, device=dev) for _ in range(2)]
-    env.refresh(random_actions=True, next_out=acts[0])
-    env.legal_bitmap(bm[0], obs=obs[0], cobs=cobs[0])
-    for t in range(T):
-        env.step_rollout(acts[t & 1], obs[t + 1], bm[t + 1], random_actions=True, next_out=acts[(t + 1) & 1], cobs=cobs[t + 1])
-    return obs.reshape(-1, 46, 9, 9), cobs.reshape(-1, 40)
-
-
 def test_compact_observation_is_the_observation():
     """The 160-byte compact observation the engine writes beside every observation row decodes to exactly that row
     (piece-plane index per square, rotated for White to move, + the 18 constant-plane values), across resets."""
-    obs, cobs = _rollout_positions()
-    assert torch.equal(_obs_from_cobs(cobs), obs)
+    from tests.helpers import obs_from_cobs, rollout_positions
+    obs, cobs = rollout_positions()
+    assert torch.equal(obs_from_cobs(cobs), obs)
     assert bool((cobs.view(torch.uint8).reshape(-1, 160)[:, 81:84] == 0xFF).all())  # pad bytes of the square table
     side_black = obs[:, 42, 0, 0] == 1.0
     assert bool(side_black.any()) and bool((~side_black).any())  # both perspectives occur
@@ -559,7 +531,8 @@ def test_input_layer_from_compact_observations(relu):
     fp32 rows of the same positions and against torch's conv2d on bf16-rounded operands; rows gathered in place."""
     from shogidrl_b200 import nn_ops
     dev = torch.device("cuda:0")
-    obs, cobs = _rollout_positions(1024, 30)
+    from tests.helpers import rollout_positions
+    obs, cobs = rollout_positions(1024, 30)
     g = torch.Generator(device="cpu").manual_seed(4)
     w = (torch.randn(16, 46, 3, 3, generator=g) * 0.05).to(dev).requires_grad_(True)
     b = (torch.randn(16, generator=g) * 0.1).to(dev).requires_grad_(True)
